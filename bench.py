@@ -15,7 +15,14 @@ H2D of the frame and D2H of the reconstruction + bpp inside the timed region), `
 live per-launch CUDA-event timing of an instrumented eager pass of a steady-state chain frame), `cpu_baseline` (oracle on
 the host cores: ONE true 1920x1024 P-frame plus the 384x640 sample of round 1), `gpu_eager_baseline` (the same PyTorch
 restatement run eagerly on this B200: fp32, TF32 convolutions, autocast fp16), `config5` (multi-frame fusion + in-loop
-filter alone), `products_per_mac`, `gpu_launches`, `clocks`, `stats` (bpp / PSNR of the coded frames).
+filter alone), `products_per_mac`, `gpu_launches`, `clocks`, `stats` (bpp / PSNR of the coded frames).  The per-kernel
+tables of the instrumented frame (`kernels`, `memory_bound_kernels`) go to stderr as a JSON line of their own, so that the
+result line stays short.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step as DIR/<name>.npy (rank 0; float32): the
+reconstruction and both bpp of the last P-frame, or for --workload train the five outputs of the training forward and the
+loss.  Inputs and weights are generated from fixed seeds, so two builds run with the same arguments can be compared output
+for output.
 """
 import argparse
 import json
@@ -35,6 +42,20 @@ H, W, GOP = 1024, 1920, 12
 MACS_PER_PX = 3832051  # SURVEY.md 8(d): MAC per full-resolution pixel of one P-frame
 ENABLE_AMP = True   # the reference's shipped evaluation config (reference cfg/predict.yaml: `enable_amp: True`; tools/predict.py:64-65,146)
 CPU_SAMPLE = (384, 640)  # 1/8 of the 1920x1024 pixels (secondary CPU sample; the primary one is a full frame)
+DUMP_BYTES = 60 * 2 ** 20   # --dump-outputs: data of all files together (64 MB with room for the .npy headers)
+
+
+def dump_outputs(path, arrays):
+    """Writes path/<name>.npy for each tensor of `arrays` in float32 (float64 stays float64).  Should they exceed DUMP_BYTES
+    together, every array keeps every n-th element of its flattened form, the same n for all."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().cpu() for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == torch.float64 else v.float() for k, v in arrays.items()}
+    step = -(-sum(v.numel() * v.element_size() for v in arrays.values()) // DUMP_BYTES)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), (v.reshape(-1)[::step] if step > 1 else v).numpy())
 
 
 def _peaks():
@@ -91,7 +112,7 @@ def cpu_oracle_rate(steps, warmup, full=True):
     Primary sample: `steps` TRUE 1920x1024 P-frames (the workload's own first GOP, frame pair 1) after `warmup` warm-up
     frames at 384x640 (a full-size warm-up would double the minutes for nothing: the first call costs < 1 % of a 35-90 s
     frame).  Secondary: one 384x640 frame (1/8 of the pixels, the round-1 extrapolation base) and BASELINE config 1
-    (256x256).  Returns a dict."""
+    (256x256).  Returns a dict; with `full`, "outputs" holds what the last true-size frame returned."""
     import torch
     from oracle.stats import build_oracle
     from tdvc_b200 import synth
@@ -118,10 +139,11 @@ def cpu_oracle_rate(steps, warmup, full=True):
             ts = []
             for _ in range(steps):
                 t0 = time.perf_counter()
-                orc(x, refs, False)
+                recon, bpp_res, bpp_mv = orc(x, refs, False)
                 ts.append(time.perf_counter() - t0)
             out["full_s"] = sum(ts) / len(ts)
             out["full_steps"] = steps
+            out["outputs"] = {"recon": recon, "bpp_res": bpp_res, "bpp_mv": bpp_mv}
     return out
 
 
@@ -143,12 +165,14 @@ def _cpu_record(r):
 
 def run_reference(args):
     """Reference arm: the reference's CPU implementation of the path (the oracle port) on the host cores, TRUE 1920x1024
-    frames: min(K, 2) timed steps so that the run ends within a few minutes (35-90 s per frame)."""
+    frames: K timed steps (35-90 s each)."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 2))
+    steps = args.steps
     r = cpu_oracle_rate(steps, 1, full=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["outputs"])
     rec = _cpu_record(r)
     line = {"impl": "reference", "metric": "1920x1024 P-frames/sec", "value": rec["value"], "unit": "P-frames/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": 1, "ms_per_step": 1000.0 / rec["value"], "higher_is_better": True, "scaling": "weak",
@@ -256,12 +280,13 @@ def gpu_eager_training_baseline(dev, batch=8, size=256, iters=3):
     return out
 
 
-def training_leg(dev, world, steps, warmup, batch=8, size=256, graph=False, amp=None):
+def training_leg(dev, world, steps, warmup, batch=8, size=256, graph=False, amp=None, outputs=None):
     """BASELINE config 4: one training step of reference tools/train.py:125-159 (enable_amp False branch) - forward, rd_loss
     (2048 * MSE + bpp_res + bpp_mv), backward, clip_grad_norm_(2), Adam step, aux_loss backward, aux Adam step - on a
     Vimeo-shaped synthetic batch: `batch` samples of 256x256 with 4 references each PER GPU (the reference splits a global
     batch over DataParallel replicas; one process per GPU with DistributedDataParallel here, NCCL gradient all-reduce).
-    CUDA-event timed, max over ranks."""
+    CUDA-event timed, max over ranks.  `outputs` (a dict) receives the forward's outputs and the loss of the last timed step,
+    on the host."""
     import torch
     import torch.distributed as dist
     from tdvc_b200 import synth
@@ -303,6 +328,9 @@ def training_leg(dev, world, steps, warmup, batch=8, size=256, graph=False, amp=
         opt.step()
         aux_opt.step()
         losses.append(loss.detach())
+        if outputs is not None:   # (in a captured step these are the graph's output tensors, which every replay rewrites)
+            outputs.update({k: v.detach() for k, v in zip(("recon", "bpp_res", "bpp_mv", "mv_aux_loss", "res_aux_loss"), out)},
+                           loss=loss.detach())
 
     torch.cuda.reset_peak_memory_stats(dev)
     mem0 = torch.cuda.memory_allocated(dev)     # what earlier legs of the same process still hold (graphs, caches) is not this leg's
@@ -334,6 +362,8 @@ def training_leg(dev, world, steps, warmup, batch=8, size=256, graph=False, amp=
         run()
     e1.record()
     torch.cuda.synchronize()
+    if outputs is not None:
+        outputs.update({k: v.cpu() for k, v in outputs.items()})
     ms = torch.tensor([e0.elapsed_time(e1) / steps], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -368,7 +398,10 @@ def main():
     ap.add_argument("--train-graph", action="store_true", help="--workload train: capture the whole step in a CUDA graph and replay it (a measurement of the GPU-bound step: replays reuse the captured noise seed and weight scalings)")
     ap.add_argument("--height", type=int, default=H)
     ap.add_argument("--width", type=int, default=W)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -391,7 +424,11 @@ def main():
         import datetime
         dist.init_process_group("nccl", device_id=dev, timeout=datetime.timedelta(seconds=180))   # a hang must fail fast
     if args.workload == "train":
-        rec = training_leg(dev, world, max(1, min(args.steps, 8)), max(args.warmup, 3), graph=args.train_graph and world == 1, amp=False if args.train_exact else None)
+        outs = {} if args.dump_outputs else None
+        rec = training_leg(dev, world, args.steps, max(args.warmup, 3), graph=args.train_graph and world == 1,
+                           amp=False if args.train_exact else None, outputs=outs)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, outs)
         if rank == 0 and world == 1 and not args.no_eager_baseline:
             torch.cuda.empty_cache()
             rec["gpu_eager_baseline"] = gpu_eager_training_baseline(dev)
@@ -441,7 +478,7 @@ def main():
             gi += 1
 
     def run_chain(src, n_warm, n_timed, host_io):
-        """Codes n_warm + n_timed P-frames as GOP chains; returns (ms, stats[7], launches)."""
+        """Codes n_warm + n_timed P-frames as GOP chains; returns (ms, stats[7], launches, outputs of the last frame)."""
         stats = torch.zeros(7, device=dev, dtype=torch.float64)
         sse = torch.zeros(1, device=dev, dtype=torch.float64)
         it = frame_stream(src)
@@ -489,19 +526,22 @@ def main():
         if world > 1:
             dist.barrier()
         ms = ev0.elapsed_time(ev1)
-        return ms, stats, launches
+        return ms, stats, launches, {"recon": recon, "bpp_res": bpp_res, "bpp_mv": bpp_mv}
 
     sampler = ClockSampler(local)
-    ms, stats, launches = run_chain(dev_gops, Wm_total, K, host_io=False)
+    ms, stats, launches, last = run_chain(dev_gops, Wm_total, K, host_io=False)
     clocks = sampler.stop()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
+    del last
     sampler = ClockSampler(local)
     sampler.start = lambda: None  # clocks are sampled on the device-resident leg only
-    ms_e2e, _, _ = run_chain(host_gops, Wm_total, K, host_io=True)
+    ms_e2e, _, _, _ = run_chain(host_gops, Wm_total, K, host_io=True)
     # secondary: the same resident chain with every convolution at fp32-class accuracy (enabled_amp=False semantics)
     ms_exact = None
     if net._precision(ENABLE_AMP) != "exact" and world == 1:   # (run_chain holds collectives: a leg is run by all ranks or none)
         net.precision = "exact"
-        ms_exact, _, _ = run_chain(dev_gops, GOP - 1, GOP - 1, host_io=False)
+        ms_exact, _, _, _ = run_chain(dev_gops, GOP - 1, GOP - 1, host_io=False)
         ms_exact /= GOP - 1
         net.precision = args.precision
 
@@ -675,9 +715,10 @@ def main():
                 "roofline": roof, "frame_tensor_tflops": frame_tflops,
                 "frame_tensor_frac_of_sustained_bf16": frame_tflops / peaks["bf16_tflops_sustained"],
                 "products_per_mac": products_per_mac, "instrumented_frame_ms": total_ms,
-                "memory_bound_kernels": mem_rows, "kernels": kernels, "config5": cfg5, "entropy_coding": coding, "training_step": train,
+                "config5": cfg5, "entropy_coding": coding, "training_step": train,
                 "gpu_eager_baseline": eager, "exact_precision_ms_per_step": ms_exact,
                 "cpu_baseline": cpu, "stats": G.summarise(stats)}
+        print(json.dumps({"memory_bound_kernels": mem_rows, "kernels": kernels}), file=sys.stderr, flush=True)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

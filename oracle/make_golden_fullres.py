@@ -3,7 +3,7 @@
 
     python -m oracle.make_golden_fullres [pair] [chain]
 
-Two fixtures, both with the conditioned weights (seed 1111) the small fixtures use:
+Two fixtures, both with the conditioned weights (seed 1111) the small fixtures use (stored as samples, see below):
 
   tests/golden/p1024x1920_s0.npz      one P-frame with four DISTINCT raw reference frames (synth.make_frame_pair,
         seed 0): full reconstruction (uint16, x 65535), both bpp, every quantised symbol of both coders (int8), the
@@ -15,6 +15,11 @@ Two fixtures, both with the conditioned weights (seed 1111) the small fixtures u
 
 Reconstruction and bpp come from the REFERENCE code; symbols / indices / stage tensors from the restatement
 oracle/model.py run on the same inputs, which is asserted bit-exact with the reference on recon and bpp for every frame.
+
+Every quantised symbol of the pair and of chain frame 1 is stored, and every z symbol of every frame, so that the tests see
+each flipped symbol.  The rest is not stored whole (each file stays below 1 MB): shrink_pair / shrink_chain keep fixed samples
+of it - every n-th element of a flattened array (`sample`), every n-th pixel position with its three channels
+(`pixel_sample`) - and the tests take the same samples of the CUDA path's tensors.
 """
 import os
 import sys
@@ -28,7 +33,49 @@ warnings.filterwarnings("ignore")
 
 H, W = 1024, 1920
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
-STAGES = ("prediction1", "prediction", "recon_feat", "input_residual", "estmv", "mv.x_hat")
+STAGES = ("prediction1", "prediction", "recon_feat")
+Y_STEP_CHAIN = 31              # symbols of chain frames 2.. (an odd step walks across channels, rows and columns)
+PIX_STEP, S4_PIX_STEP = 97, 23  # pixel positions of the full reconstruction / of its stride-4 grid (chain)
+S32_STEP, TILE_STEP = 8, 3      # stride-32 stage samples / 64x64-tile means
+
+
+def sample(a, step):
+    """Every `step`-th element of the flattened array (numpy or torch)."""
+    return a.reshape(-1)[::step]
+
+
+def pixel_sample(img, step):
+    """(1, 3, H, W) -> (3, n): every `step`-th pixel position (row-major), all three channels."""
+    return img.reshape(3, -1)[:, ::step]
+
+
+def shrink_pair(d):
+    """Full-size arrays of the pair fixture -> what tests/golden/p1024x1920_s0.npz stores."""
+    out = {k: d[k] for k in ("h", "w", "seed", "state_checksum", "input_checksum", "bpp_res", "bpp_mv", "mse", "ind")}
+    for c in ("mv", "res"):
+        for k in (c + "_y_hat", c + "_z_hat_minus_med"):
+            out[k] = d[k]
+    out["recon_q16"] = pixel_sample(d["recon_q16"], PIX_STEP)
+    for k in STAGES:
+        out["s32_" + k] = sample(d["s32_" + k], S32_STEP)
+        out["tile_" + k] = sample(d["tile_" + k], TILE_STEP)
+        out["stat_" + k] = d["stat_" + k]
+    return out
+
+
+def shrink_chain(d):
+    """Full-size arrays of the chain fixture (the frames coded so far) -> what tests/golden/chain1024x1920_s100.npz stores."""
+    out = {k: d[k] for k in ("h", "w", "seed", "n_p", "state_checksum", "input_checksum")}
+    t = 1
+    while f"f{t}_mse" in d:
+        p = f"f{t}_"
+        for k in ("bpp_res", "bpp_mv", "mse", "ind", "recon_tile", "mv_z_hat_minus_med", "res_z_hat_minus_med"):
+            out[p + k] = d[p + k]
+        for c in ("mv", "res"):
+            out[p + c + "_y_hat"] = d[p + c + "_y_hat"] if t == 1 else sample(d[p + c + "_y_hat"], Y_STEP_CHAIN)
+        out[p + "recon_s4_q16"] = pixel_sample(d[p + "recon_s4_q16"], S4_PIX_STEP)
+        t += 1
+    return out
 
 
 def _q16(x):
@@ -78,7 +125,7 @@ def make_pair(ref, orc, csum):
         d["s32_" + k] = v[:, :, ::32, ::32].contiguous().numpy()
         d["tile_" + k] = _tile_mean(v).astype(np.float32)
         d["stat_" + k] = np.array([v.double().mean().item(), v.double().abs().mean().item(), v.abs().max().item()])
-    np.savez_compressed(os.path.join(OUT, "p1024x1920_s0.npz"), **d)
+    np.savez_compressed(os.path.join(OUT, "p1024x1920_s0.npz"), **shrink_pair(d))
     print("pair written", flush=True)
 
 
@@ -102,7 +149,7 @@ def make_chain(ref, orc, csum, n_p=6, seed=100):
         d[p + "recon_tile"] = _tile_mean(recon).astype(np.float32)
         _symbols(d, taps, orc, p)
         del taps
-        np.savez_compressed(os.path.join(OUT, f"chain1024x1920_s{seed}.npz"), **d)   # rewritten after every frame
+        np.savez_compressed(os.path.join(OUT, f"chain1024x1920_s{seed}.npz"), **shrink_chain(d))   # rewritten after every frame
     print("chain written", flush=True)
 
 

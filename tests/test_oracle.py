@@ -1,6 +1,7 @@
 """CPU tests of the oracle itself (-m "not gpu"): the restatement is pinned against
- (a) the reference's own unmodified code imported from /root/reference (skipped where that tree is absent),
- (b) the committed golden fixtures made from (a) by oracle/make_golden.py,
+ (a) the reference's own unmodified code imported from TDVC_REFERENCE_ROOT (skipped where that tree is absent),
+ (b) the committed golden fixtures made from (a) by oracle/make_golden.py, and the reference's state_dict layout and loader
+     sample lists (tests/golden/reference_lists.json),
  (c) the reference's DCNv2 known-answer test (reference main/utils/dcnv2/testcuda.py:36-71).
 """
 import numpy as np
@@ -11,11 +12,15 @@ from conftest import load_golden
 from oracle import dcn_naive, ref_import
 from tdvc_b200 import synth
 
-needs_ref = pytest.mark.skipif(not ref_import.available(), reason="/root/reference not present (GPU box)")
+needs_ref = pytest.mark.skipif(not ref_import.available(),
+                               reason="needs a checkout of the reference TDVC source tree at TDVC_REFERENCE_ROOT")
 
 
-def test_state_dict_keys_and_checksum(oracle_model):
-    sd = oracle_model.state_dict()
+def test_state_dict_keys_and_checksum():
+    """On a freshly built oracle: any forward of the session's shared one (other test modules run it) has zeroed the masked
+    taps of its context models, since MaskedConv2d masks its weight in place as compressai's does."""
+    from oracle.stats import build_oracle
+    sd = build_oracle().state_dict()
     g = load_golden("p64x64_s1")
     assert abs(synth.state_checksum(sd) - float(g["state_checksum"])) < 1e-6 * float(g["state_checksum"])
     for must in ("mvCoder.g_a.0.gdn.gamma", "mvCoder.entropy_bottleneck._matrix0",
@@ -25,13 +30,18 @@ def test_state_dict_keys_and_checksum(oracle_model):
         assert must in sd, must
 
 
-@needs_ref
+def _reference_lists():
+    import json
+    import os
+    from conftest import ROOT
+    return json.load(open(os.path.join(ROOT, "tests", "golden", "reference_lists.json")))
+
+
 def test_strict_state_dict_roundtrip_with_reference(oracle_model):
-    ref = ref_import.reference_video_compressor()
-    assert list(ref.state_dict().keys()) == list(oracle_model.state_dict().keys())
-    ref.load_state_dict(oracle_model.state_dict(), strict=True)
-    for k, v in ref.state_dict().items():
-        assert v.shape == oracle_model.state_dict()[k].shape, k
+    """The reference's state_dict keys in order with their shapes (tests/golden/reference_lists.json): a checkpoint of either
+    loads strictly into the other."""
+    want = [(k, tuple(s)) for k, s in _reference_lists()["state_dict"]]
+    assert [(k, tuple(v.shape)) for k, v in oracle_model.state_dict().items()] == want
 
 
 @needs_ref
@@ -156,36 +166,52 @@ def test_msssim_oracle_vs_reference_function():
     assert abs(float(R.ms_ssim(x, x, data_range=1.0)) - 1.0) < 1e-6 and abs(float(O.ms_ssim(x, x, data_range=1.0)) - 1.0) < 1e-6
 
 
-@needs_ref
-def test_dataset_sample_lists_match_reference_code(tmp_path):
-    """tdvc_b200.data lists the same samples as the reference's own loaders, run here from /root/reference (reference
-    main/dataloader/dataset.py: `DataSet.get_vimeo` :210-247, `UVGDataSet.__init__` :16-60, `HEVCDataSet.__init__` :100-166)."""
+def _sample_list_trees(root):
+    """Empty-file trees laid out as the reference's datasets: vimeo_septuplet (<dir>/<clip>/im1..im7.png, directory names
+    chosen so that natural and plain sorting differ) and an evaluation tree (ori_img/<seq>/imNNN.png +
+    compress_img_bpg/<seq>/<qp>/imNNN_<qp>.{png,txt}).  Returns (vimeo root, evaluation root, GOP size)."""
     import os
-    from tdvc_b200 import data as D
-    ds_ref = ref_import.load_reference_dataset()
-    # --- vimeo_septuplet tree: <dir>/<clip>/im1..im7.png (directory names chosen so that natural and plain sorting differ)
-    vimeo = tmp_path / "vimeo"
+    vimeo = root / "vimeo"
     for d, clip in (("00010", "0002"), ("00002", "0010"), ("00002", "0009")):
         os.makedirs(vimeo / d / clip)
         for i in range(1, 8):
             open(vimeo / d / clip / f"im{i}.png", "wb").close()
-    want_in, want_ref = ds_ref.DataSet.get_vimeo(None, str(vimeo))
-    got_in, got_ref = D.VimeoDataset.get_vimeo(str(vimeo))
-    assert len(want_in) == 21 and got_in == want_in and got_ref == want_ref
-    # --- evaluation tree: ori_img/<seq>/imNNN.png + compress_img_bpg/<seq>/<qp>/imNNN_<qp>.{png,txt}
-    root, gop, qp = tmp_path / "eval", 3, 27
+    ev, gop, qp = root / "eval", 3, 27
     for seq, nfr in (("Seq10_416x240_50", 7), ("Seq2_416x240_30", 6), ("BQSquare_416x240_60", 9)):
-        os.makedirs(root / "ori_img" / seq)
-        os.makedirs(root / "compress_img_bpg" / seq / str(qp))
+        os.makedirs(ev / "ori_img" / seq)
+        os.makedirs(ev / "compress_img_bpg" / seq / str(qp))
         for i in range(nfr):
-            open(root / "ori_img" / seq / f"im{i + 1:03d}.png", "wb").close()
+            open(ev / "ori_img" / seq / f"im{i + 1:03d}.png", "wb").close()
         for g in range(nfr // gop):
-            stem = root / "compress_img_bpg" / seq / str(qp) / f"im{g * gop + 1:03d}_{qp}"
+            stem = ev / "compress_img_bpg" / seq / str(qp) / f"im{g * gop + 1:03d}_{qp}"
             open(str(stem) + ".png", "wb").close()
             open(str(stem) + ".txt", "w").write(f"{0.25 * (g + 1)}\n")
-    ref_uvg = ds_ref.UVGDataSet(str(root), 2048, gop, testfull=True, isTrain=False)
-    ours = D.GopDataset(str(root), 2048, gop, testfull=True)
-    assert (ours.ref, ours.refbpp, ours.input) == (ref_uvg.ref, ref_uvg.refbpp, ref_uvg.input) and len(ours) == 7
-    ref_hevc = ds_ref.HEVCDataSet(str(root), 64, gop, "D", testfull=True, isTrain=False)
-    ours = D.GopDataset(str(root), 64, gop, testfull=True, hevc_class="D")
-    assert (ours.ref, ours.refbpp, ours.input) == (ref_hevc.ref, ref_hevc.refbpp, ref_hevc.input) and len(ours) == 3
+    return vimeo, ev, gop
+
+
+def _sample_lists(root):
+    """tdvc_b200.data's sample lists for the trees of _sample_list_trees, paths relative to `root`."""
+    import os
+    from tdvc_b200 import data as D
+    vimeo, ev, gop = _sample_list_trees(root)
+
+    def rel(x):
+        return [rel(v) for v in x] if isinstance(x, (list, tuple)) else os.path.relpath(x, root) if isinstance(x, str) else x
+
+    got_in, got_ref = D.VimeoDataset.get_vimeo(str(vimeo))
+    out = {"vimeo": {"input": rel(got_in), "ref": rel(got_ref)}}
+    for name, lmbda, hevc_class in (("uvg", 2048, None), ("hevc", 64, "D")):
+        ds = D.GopDataset(str(ev), lmbda, gop, testfull=True, hevc_class=hevc_class)
+        out[name] = {"ref": rel(ds.ref), "refbpp": list(ds.refbpp), "input": rel(ds.input), "len": len(ds)}
+    return out
+
+
+def test_dataset_sample_lists_match_reference_code(tmp_path):
+    """tdvc_b200.data lists the same samples as the reference's own loaders (reference main/dataloader/dataset.py:
+    `DataSet.get_vimeo` :210-247, `UVGDataSet.__init__` :16-60, `HEVCDataSet.__init__` :100-166) return for the same trees,
+    recorded in tests/golden/reference_lists.json."""
+    want = _reference_lists()
+    got = _sample_lists(tmp_path)
+    assert len(got["vimeo"]["input"]) == 21 and got["uvg"]["len"] == 7 and got["hevc"]["len"] == 3
+    for k in ("vimeo", "uvg", "hevc"):
+        assert got[k] == want[k], k

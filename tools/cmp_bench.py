@@ -1,10 +1,16 @@
-"""Developer tool: compare the per-kernel tables of two bench.py JSON lines (A/B of a kernel change)."""
+"""Developer tool: compare the per-kernel tables of two bench.py runs (A/B of a kernel change).
+    python bench.py > a.json 2>&1; ...; python tools/cmp_bench.py a.json b.json [threshold_ms]"""
 import json
 import sys
 
 
 def load(p):
-    return json.loads(open(p).read().strip().splitlines()[-1])
+    """The result line (stdout) merged with the per-kernel tables bench.py prints on stderr."""
+    d = {}
+    for line in open(p):
+        if line.startswith("{"):
+            d.update(json.loads(line))
+    return d
 
 
 a, b = load(sys.argv[1]), load(sys.argv[2])

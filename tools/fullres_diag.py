@@ -1,4 +1,5 @@
-"""Developer tool (GPU box): the CUDA path against the two 1920x1024 fixtures, printed instead of asserted."""
+"""Developer tool (GPU): the CUDA path against the two 1920x1024 fixtures, printed instead of asserted.  Reconstructions,
+stage tensors and the symbols of chain frames 2.. are compared on the samples the fixtures store (oracle/make_golden_fullres.py)."""
 import math
 import sys
 import warnings
@@ -10,13 +11,18 @@ warnings.filterwarnings("ignore")
 sys.path.insert(0, ".")
 sys.path.insert(0, "tests")
 
+from oracle import make_golden_fullres as GF  # noqa: E402
+
 
 def flips(g, taps, net, p=""):
     out = {}
     for c, cn in (("mv", "mvCoder"), ("res", "resCoder")):
         yh = taps[f"{c}.y_hat"].cpu()
-        bad = torch.from_numpy(yh.numpy().astype(np.int16) != g[p + f"{c}_y_hat"].astype(np.int16))
         y = taps[f"{c}.y"].cpu()
+        want = g[p + f"{c}_y_hat"]
+        if want.shape != tuple(yh.shape):     # a sampled latent: flips among the stored symbols only
+            yh, y = GF.sample(yh, GF.Y_STEP_CHAIN), GF.sample(y, GF.Y_STEP_CHAIN)
+        bad = torch.from_numpy(yh.numpy().astype(np.int16) != want.astype(np.int16))
         tie = ((y - torch.floor(y)) - 0.5).abs()
         out[c] = (int(bad.sum()), bad.numel(), float(tie[bad].max()) if bad.any() else 0.0, bad)
         med = getattr(net, cn).entropy_bottleneck.quantiles[:, 0, 1].detach().view(1, -1, 1, 1).cpu()
@@ -58,18 +64,19 @@ def main():
         print("   ind equal", bool((taps["loopfilter.ind"].cpu().numpy().astype(np.int32) == g["ind"]).all()),
               "bpp rel", abs(bres.item() - float(g["bpp_res"][0])) / float(g["bpp_res"][0]), abs(bmv.item() - float(g["bpp_mv"][0])) / float(g["bpp_mv"][0]))
         want = torch.from_numpy(g["recon_q16"].astype(np.float32) / 65535.0)
-        err = (recon.cpu() - want).abs()[0].max(0).values
+        err = (GF.pixel_sample(recon.cpu(), GF.PIX_STEP) - want).abs().max(0).values
         allbad = (f["mv"][3] | f["res"][3]).any(1, keepdim=True).float()
         for r in (0, 4, 8, 12, 16):
             m = torch.nn.functional.interpolate(torch.nn.functional.max_pool2d(allbad, 2 * r + 1, 1, r), scale_factor=16, mode="nearest")[0, 0] > 0
+            m = GF.sample(m, GF.PIX_STEP)
             print(f"   recon max err outside r={r} latents of any flip: {(err[~m].max().item() if (~m).any() else 0.0):.3e} (masked {m.float().mean().item():.4f}); overall {err.max().item():.3e}")
         mse = ((recon.cpu().double() - x.double()) ** 2).mean().item()
         print("   dPSNR", 10 * math.log10(1 / mse) - 10 * math.log10(1 / float(g["mse"])))
         for k in ("prediction1", "prediction", "recon_feat"):
             v = taps[k].cpu()
             scale = float(g["stat_" + k][2])
-            d = (v[:, :, ::32, ::32] - torch.from_numpy(g["s32_" + k])).abs()
-            tm = torch.nn.functional.avg_pool2d(v.double(), 64).float()
+            d = (GF.sample(v[:, :, ::32, ::32], GF.S32_STEP) - torch.from_numpy(g["s32_" + k])).abs()
+            tm = GF.sample(torch.nn.functional.avg_pool2d(v.double(), 64).float(), GF.TILE_STEP)
             print(f"   {k}: scale {scale:.3f} sample max err {d.max().item():.3e} frac>1e-4*scale {(d > 1e-4 * scale).float().mean().item():.2e}; "
                   f"tile-mean max err {(tm - torch.from_numpy(g['tile_' + k])).abs().max().item():.3e}")
     del taps
@@ -91,7 +98,8 @@ def main():
             p = f"f{t}_"
             f = flips(g, taps, net, p)
             mse = ((recon.double() - x.double()) ** 2).mean().item()
-            d = (recon[:, :, ::4, ::4].cpu() - torch.from_numpy(g[p + "recon_s4_q16"].astype(np.float32) / 65535.0)).abs()
+            want = torch.from_numpy(g[p + "recon_s4_q16"].astype(np.float32) / 65535.0)
+            d = (GF.pixel_sample(recon[:, :, ::4, ::4].cpu(), GF.S4_PIX_STEP) - want).abs()
             tm = torch.nn.functional.avg_pool2d(recon.double(), 64).float().cpu()
             print(f"{precision} chain frame {t}: flips mv {f['mv'][:3]} res {f['res'][:3]} z {f['mv.z']} {f['res.z']} | "
                   f"ind eq {bool((taps['loopfilter.ind'].cpu().numpy().astype(np.int32) == g[p + 'ind']).all())} | bpp rel "
