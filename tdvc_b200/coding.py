@@ -16,6 +16,8 @@ What runs where:
 * `compress`: z symbols by `tdvc_eb_symbols`; the autoregressive pass over y - compressai's per-position Python loop - by
   the wavefront kernel `tdvc_ar_code` (one launch per coder, csrc/coding.cu) on the y / hyper-decoder buffers the forward
   pass left in the plan; rANS over the symbols on the host (`tdvc_rans_encode_with_indexes`), as in compressai.
+* `decode_latents`: y strings back to symbols and y_hat on the device (`tdvc_ar_decode`, csrc/ar_decode.cu), bit-identical
+  to what `tdvc_ar_code` produced when told the encoder's cluster size.
 """
 import ctypes as C
 import math
@@ -51,6 +53,14 @@ class Tables:
     def tensors(self, device):
         return (torch.from_numpy(self.cdf.copy()).to(device), torch.from_numpy(self.length.copy()).to(device),
                 torch.from_numpy(self.offset.copy()).to(device))
+
+    def on(self, device):
+        """tensors(device), built once per device (read by the device decoder)."""
+        cache = self.__dict__.setdefault("_on", {})
+        key = str(torch.device(device))
+        if key not in cache:
+            cache[key] = self.tensors(device)
+        return cache[key]
 
 
 def _pmf_to_cdf(pmf, tail, pmf_length, max_length):
@@ -211,6 +221,8 @@ def launch_coding(plan, W, cn, tables, cluster=0, stream=None):
                    w3=e4.w.data_ptr(), b3=e4.b.data_ptr(), scale_table=tables.scale_table.data_ptr(), n_scales=SCALES_LEVELS,
                    y_hat=y_hat.data_ptr(), symbols=y_sym.data_ptr(), indexes=y_idx.data_ptr(), N=N, H=hy, W=wy, C=128,
                    cluster=cluster)
+    used = C.c_int32(0)
+    p.cluster_used_host = C.addressof(used)
     L.check(lib.tdvc_ar_code(C.byref(p), ws.data_ptr(), need, st), "ar_code")
     plan.launches += 2
     host = []
@@ -221,19 +233,20 @@ def launch_coding(plan, W, cn, tables, cluster=0, stream=None):
             host.append(h)
         done = torch.cuda.Event()
         done.record(stream)
-    return {"host": host, "done": done, "tables": tables, "N": N, "shape": (hz, wz),
+    return {"host": host, "done": done, "tables": tables, "N": N, "shape": (hz, wz), "cluster": used.value,
             "dev": {"y_symbols": y_sym, "y_indexes": y_idx, "y_hat": y_hat, "z_symbols": z_sym}}
 
 
 def finish_coding(h, keep=False):
     """Host half: rANS over the symbols, one string per image (compressai codes batch items separately).
-    Returns {"strings": [y_strings, z_strings], "shape": (h, w)} (+ clones of the device tensors if keep)."""
+    Returns {"strings": [y_strings, z_strings], "shape": (h, w), "cluster": CTAs per image the y pass ran with (the
+    summation order a decoder must reproduce)} (+ clones of the device tensors if keep)."""
     h["done"].synchronize()
     hs = [t.numpy() for t in h["host"]]
     tables = h["tables"]
     y_strings = [rans_encode(hs[0][i], hs[1][i], tables.gc) for i in range(h["N"])]
     z_strings = [rans_encode(hs[2][i], hs[3][i], tables.eb) for i in range(h["N"])]
-    out = {"strings": [y_strings, z_strings], "shape": h["shape"]}
+    out = {"strings": [y_strings, z_strings], "shape": h["shape"], "cluster": h["cluster"]}
     if keep:
         out.update({k: v.clone() for k, v in h["dev"].items()})
     return out
@@ -243,21 +256,113 @@ def code_latents(plan, W, cn, tables, cluster=0, keep=False):
     return finish_coding(launch_coding(plan, W, cn, tables, cluster=cluster), keep=keep)
 
 
+def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
+    """Device decoding of the y strings of coder `cn` ("mv" | "rs"), the inverse of launch_coding's y half
+    (compressai `_decompress_ar`): `tdvc_ar_decode` runs the context model and the entropy parameters position by position
+    and decodes the rANS stream on the device.  params: the hyper-decoder output of the same images, a channels-last Act
+    (N, h, w, >= 256 channels).  cluster: the CTAs per image `tdvc_ar_code` coded the strings with (8 or 16); the
+    predictions, and so the decoded symbols, are exact only for that value.  Returns a handle for finish_decoding."""
+    lib = L.load()
+    N, hy, wy = params.N, params.H, params.W
+    dev = params.t.device
+    if cluster not in (8, 16):
+        raise RuntimeError(f"decode_latents: encoder cluster size {cluster} (8 or 16)")
+    if len(y_strings) != N:
+        raise RuntimeError(f"decode_latents: {len(y_strings)} {cn} y strings for {N} images")
+    for i, s_ in enumerate(y_strings):
+        if len(s_) < 8 or len(s_) % 4:
+            raise RuntimeError(f"decode_latents: {cn} y string of image {i} has {len(s_)} bytes (rANS strings are whole "
+                               "32-bit words, at least two)")
+    ctx, e0, e2, e4 = W[f"{cn}.ctx"], W[f"{cn}.ep0"], W[f"{cn}.ep2"], W[f"{cn}.ep4"]
+    if ctx.cin_pad != 128 or ctx.cout_pad != 256 or e0.cin_pad != 512 or e2.cin_pad < e0.cout_pad - 4 or e4.cout_pad != 256:
+        raise RuntimeError("decode_latents: unexpected entropy-parameter layer shapes")
+    gl = tables.gc.length
+    if gl.size > 64 or (gl < 2).any() or (gl > tables.gc.cdf.shape[1]).any() or int(gl.sum()) > 32768:
+        raise RuntimeError("decode_latents: the Gaussian CDF tables are not valid rows for the device decoder")
+    stream = stream or torch.cuda.current_stream(dev)
+    words = np.frombuffer(b"".join(bytes(s_) for s_ in y_strings), dtype="<i4")
+    offsets = np.cumsum([0] + [len(s_) // 4 for s_ in y_strings]).astype(np.int64)
+    cdf, length, offset = tables.gc.on(dev)
+    with torch.cuda.stream(stream):
+        words_d = torch.from_numpy(words.copy()).to(dev)
+        offsets_d = torch.from_numpy(offsets).to(dev)
+        y_hat = torch.empty((N, hy, wy, 128), device=dev)
+        y_sym = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
+        y_idx = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
+        status = torch.empty((N,), device=dev, dtype=torch.int64)
+    p = L.ArDecodeParams(params=params.ptr, params_ld=params.ld, w_ctx=ctx.w.data_ptr(), b_ctx=ctx.b.data_ptr(),
+                         w1=e0.w.data_ptr(), b1=e0.b.data_ptr(), c1=e0.cout, c1_pad=e0.cout_pad,
+                         w2=e2.w.data_ptr(), b2=e2.b.data_ptr(), c2=e2.cout, c2_pad=e2.cout_pad,
+                         w3=e4.w.data_ptr(), b3=e4.b.data_ptr(), scale_table=tables.scale_table.data_ptr(),
+                         n_scales=SCALES_LEVELS, words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
+                         cdfs=cdf.data_ptr(), cdf_stride=cdf.shape[1], cdf_lengths=length.data_ptr(),
+                         cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(tables.gc.length.sum()),
+                         y_hat=y_hat.data_ptr(), symbols=y_sym.data_ptr(), indexes=y_idx.data_ptr(),
+                         status=status.data_ptr(), N=N, H=hy, W=wy, C=128, cluster=cluster)
+    L.check(lib.tdvc_ar_decode(C.byref(p), stream.cuda_stream), "ar_decode")
+    with torch.cuda.stream(stream):
+        status_h = _pinned_like(status)
+        status_h.copy_(status, non_blocking=True)
+        done = torch.cuda.Event()
+        done.record(stream)
+    # the inputs stay referenced until the decode has run
+    return {"cn": cn, "done": done, "status": status_h, "keep": (words_d, offsets_d), "shape": (hy, wy),
+            "y_hat": y_hat, "y_symbols": y_sym, "y_indexes": y_idx}
+
+
+def _pinned_like(t):
+    return torch.empty(t.shape, dtype=t.dtype).pin_memory()
+
+
+def finish_decoding(h):
+    """Waits for a launch_decoding and turns a failed image into RuntimeError (naming the coder, the image and the
+    latent position (h, w, c) where the stream broke).  Returns {"y_hat", "y_symbols", "y_indexes"} (N, h, w, 128)."""
+    h["done"].synchronize()
+    wy = h["shape"][1]
+    for i, st in enumerate(h["status"].tolist()):
+        if st == -2:
+            raise RuntimeError(f"ar_decode: the Gaussian CDF tables of the {h['cn']} coder are not valid rows (image {i})")
+        if st != -1:
+            pix, c = divmod(int(st), 128)
+            raise RuntimeError(f"ar_decode: the {h['cn']} y string of image {i} is truncated or corrupt at latent position "
+                               f"(h={pix // wy}, w={pix % wy}, c={c})")
+    return {k: h[k] for k in ("y_hat", "y_symbols", "y_indexes")}
+
+
+def decode_latents(W, cn, tables, y_strings, params, cluster, stream=None):
+    return finish_decoding(launch_decoding(W, cn, tables, y_strings, params, cluster, stream=stream))
+
+
 # ----------------------------------------------------------------------------------------------- bitstream container
-_MAGIC = b"TDVC"
+_MAGIC = b"TDVC"       # version 1: strings and hyper-latent shapes only
+_MAGIC_V2 = b"TDV2"    # version 2: + frame size, batch, precision mode, and each coder's autoregressive cluster size
+_PRECISIONS = ("exact", "mixed")
 
 
-def pack_frame(coded):
+def pack_frame(coded, frame=None):
     """`net.last_coded` of one P-frame -> bytes.  The reference only sketches a container (dead code, reference
     tools/utils/encoder.py:61-68: per string a big-endian shape header, a length and the payload); this one follows the
-    sketch with 32-bit lengths (a 1920x1024 motion string is ~1 MB, beyond the sketch's uint16):
-    magic "TDVC" | >B n_coders | per coder: >4s name | >2I hyper-latent shape (h, w) | >B n_lists | per list: >I n_strings |
-    per string: >I length | payload."""
+    sketch with 32-bit lengths (a 1920x1024 motion string is ~1 MB, beyond the sketch's uint16).
+    frame=None (version 1): magic "TDVC" | >B n_coders | per coder: >4s name | >2I hyper-latent shape (h, w) | >B n_lists |
+    per list: >I n_strings | per string: >I length | payload.
+    frame={"size": (H, W), "N": N, "precision": "exact" | "mixed"} (version 2, what a decoder needs to reproduce the
+    encoder exactly): magic "TDV2" | >2I H, W | >B N | >B precision (0 exact, 1 mixed) | >B n_coders | per coder: >4s name |
+    >B cluster (CTAs per image of the autoregressive pass: its summation order) | then as version 1."""
     import struct
-    out = [_MAGIC, struct.pack(">B", len(coded))]
+    if frame is None:
+        out = [_MAGIC, struct.pack(">B", len(coded))]
+    else:
+        if frame.get("precision") not in _PRECISIONS:
+            raise RuntimeError(f"pack_frame: precision must be one of {_PRECISIONS}, not {frame.get('precision')!r}")
+        H, W = (int(v) for v in frame["size"])
+        out = [_MAGIC_V2, struct.pack(">2IBBB", H, W, int(frame["N"]), _PRECISIONS.index(frame["precision"]), len(coded))]
     for name, enc in coded.items():
-        out.append(struct.pack(">4s2IB", name.encode()[:4].ljust(4), int(enc["shape"][0]), int(enc["shape"][1]),
-                               len(enc["strings"])))
+        head = struct.pack(">4s", name.encode()[:4].ljust(4))
+        if frame is not None:
+            if enc.get("cluster") not in (8, 16):
+                raise RuntimeError(f"pack_frame: coder {name!r} has no cluster size (8 or 16)")
+            head += struct.pack(">B", enc["cluster"])
+        out.append(head + struct.pack(">2IB", int(enc["shape"][0]), int(enc["shape"][1]), len(enc["strings"])))
         for lst in enc["strings"]:
             out.append(struct.pack(">I", len(lst)))
             for s_ in lst:
@@ -267,31 +372,56 @@ def pack_frame(coded):
 
 
 def unpack_frame(data):
-    """Inverse of pack_frame -> {name: {"strings": [[bytes, ...], ...], "shape": (h, w)}}."""
+    """Inverse of pack_frame -> {name: {"strings": [[bytes, ...], ...], "shape": (h, w)}}; a version-2 container adds
+    "cluster" to every coder and "frame": {"size": (H, W), "N": N, "precision": "exact" | "mixed"}.  A truncated or
+    malformed container raises RuntimeError."""
     import struct
-    if data[:4] != _MAGIC:
+    if data[:4] not in (_MAGIC, _MAGIC_V2):
         raise RuntimeError("unpack_frame: not a tdvc_b200 frame container")
+    v2 = data[:4] == _MAGIC_V2
     pos = 4
-    (n,) = struct.unpack_from(">B", data, pos)
-    pos += 1
     out = {}
-    for _ in range(n):
-        name, h, w, nl = struct.unpack_from(">4s2IB", data, pos)
-        pos += struct.calcsize(">4s2IB")
-        lists = []
-        for _ in range(nl):
-            (ns,) = struct.unpack_from(">I", data, pos)
+    try:
+        if v2:
+            H, W, N, prec, n = struct.unpack_from(">2IBBB", data, pos)
+            pos += struct.calcsize(">2IBBB")
+            if prec >= len(_PRECISIONS):
+                raise RuntimeError(f"unpack_frame: unknown precision mode {prec}")
+            frame = {"size": (H, W), "N": N, "precision": _PRECISIONS[prec]}
+        else:
+            (n,) = struct.unpack_from(">B", data, pos)
+            pos += 1
+        for _ in range(n):
+            (name,) = struct.unpack_from(">4s", data, pos)
             pos += 4
-            strs = []
-            for _ in range(ns):
-                (ln,) = struct.unpack_from(">I", data, pos)
+            cluster = None
+            if v2:
+                (cluster,) = struct.unpack_from(">B", data, pos)
+                pos += 1
+                if cluster not in (8, 16):
+                    raise RuntimeError(f"unpack_frame: cluster size {cluster} (8 or 16)")
+            h, w, nl = struct.unpack_from(">2IB", data, pos)
+            pos += struct.calcsize(">2IB")
+            lists = []
+            for _ in range(nl):
+                (ns,) = struct.unpack_from(">I", data, pos)
                 pos += 4
-                if pos + ln > len(data):
-                    raise RuntimeError("unpack_frame: truncated container")
-                strs.append(bytes(data[pos:pos + ln]))
-                pos += ln
-            lists.append(strs)
-        out[name.decode().strip()] = {"strings": lists, "shape": (h, w)}
+                strs = []
+                for _ in range(ns):
+                    (ln,) = struct.unpack_from(">I", data, pos)
+                    pos += 4
+                    if pos + ln > len(data):
+                        raise RuntimeError("unpack_frame: truncated container")
+                    strs.append(bytes(data[pos:pos + ln]))
+                    pos += ln
+                lists.append(strs)
+            out[name.decode().strip()] = {"strings": lists, "shape": (h, w)}
+            if v2:
+                out[name.decode().strip()]["cluster"] = cluster
+    except (struct.error, UnicodeDecodeError) as e:
+        raise RuntimeError(f"unpack_frame: truncated or malformed container ({e})") from None
     if pos != len(data):
         raise RuntimeError("unpack_frame: trailing bytes")
+    if v2:
+        out["frame"] = frame
     return out

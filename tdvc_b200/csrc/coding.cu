@@ -16,20 +16,12 @@
 #include <stdlib.h>
 #include <string.h>
 #include <vector>
-#include "common.cuh"
+#include "ar_common.cuh"
 
 namespace cg = cooperative_groups;
 
 namespace tdvc {
 
-constexpr int AR_THREADS = 512;
-constexpr int AR_WARPS = AR_THREADS / 32;
-constexpr int AR_PT = 8;        // positions per warp task (register tile)
-constexpr int AR_PCH = 40;      // positions per chunk of a wavefront (1920x1024: 64x120 latent, <= 40 per wavefront)
-constexpr int AR_KS_MAX = 16;   // K splits per (channel group, position group): a short wavefront still keeps every warp busy
-constexpr int AR_NS_MAX = 64;   // output channels of one CTA per stage
-constexpr int AR_C = 128;       // latent channels (Cheng2020Anchor N = M = 128 in both coders)
-constexpr int AR_KC = 128;      // K chunk staged in shared memory (one tap of the context model)
 constexpr int AR_NBUF = 3;      // staging depth
 constexpr int AR_RED = AR_WARPS * AR_PT * 32;   // one (AR_PT positions x 32 channels) tile of partial sums per warp task
 constexpr size_t AR_SMEM = (size_t)(AR_NBUF * (AR_PCH * AR_KC + AR_KC * AR_NS_MAX) + AR_RED) * sizeof(float);
@@ -56,14 +48,6 @@ __device__ __forceinline__ unsigned long long ar_now() {
     }                                                               \
   } while (0)
 
-__device__ __forceinline__ void ar_slice(int total, int align, int rank, int R, int& n0, int& n1) {
-  const int q = (total + align - 1) / align;
-  n0 = align * (int)((int64_t)q * rank / R);
-  n1 = align * (int)((int64_t)q * (rank + 1) / R);
-  if (n1 > total) n1 = total;
-  if (n0 > total) n0 = total;
-}
-
 __device__ __forceinline__ void cp_async16_cg(float* smem, const float* g, int src_bytes) {
   const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(s), "l"(g), "r"(src_bytes) : "memory");
@@ -71,17 +55,6 @@ __device__ __forceinline__ void cp_async16_cg(float* smem, const float* g, int s
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-
-// One layer of the chain as a CTA sees it: its weight columns of Wt[K][ldw], as one or two runs of 16-byte quads:
-// [n0, n0 + ns) for the first three layers; for the last one (split = number of latent channels of this CTA) the scale
-// columns [n0, n0 + split) followed by the mean columns [AR_C + n0, AR_C + n0 + split), so that both parameters of a latent
-// channel land in the same CTA.  n0, split and ldw are multiples of 4 (the last quad of a layer may reach into the
-// zero-padded columns).
-struct ArW {
-  const float* Wt;
-  int ldw, K, n0, ns, split;
-  __device__ __forceinline__ int col(int n) const { return split && n >= split ? AR_C + n0 + (n - split) : n0 + n; }
-};
 
 // weight part of chunk c of a layer -> ring slot c % AR_NBUF
 __device__ __forceinline__ void ar_issue_w(const ArW& w, int c, float* sW) {
@@ -127,8 +100,7 @@ __device__ __forceinline__ int ar_stage(const ArW& w, int P, float* sA, float* s
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ns = w.ns, K = w.K;
   const int NG = (ns + 31) >> 5, PG = (P + AR_PT - 1) / AR_PT;
-  int KS = AR_WARPS / (NG * PG);
-  KS = KS < 1 ? 1 : (KS > AR_KS_MAX ? AR_KS_MAX : KS);
+  const int KS = ar_ksplits(ns, P);
   const int tasks = NG * PG * KS;          // <= AR_WARPS: NG <= 2, PG <= 5
   const bool busy = warp < tasks;
   const int ks = warp % KS, r = warp / KS;
@@ -151,10 +123,8 @@ __device__ __forceinline__ int ar_stage(const ArW& w, int P, float* sA, float* s
     ar_issue_w(w, c + 2, sW);
     cp_async_commit();
     if (busy) {
-      const int k0 = c * AR_KC;
-      const int kc = K - k0 < AR_KC ? K - k0 : AR_KC;
-      const int nq = kc >> 2;
-      const int q0 = nq * ks / KS, q1 = nq * (ks + 1) / KS;
+      int q0, q1;
+      ar_split_quads(ar_chunk_quads(K, c), ks, KS, q0, q1);
       const float* cA = sA + (c % AR_NBUF) * (AR_PCH * AR_KC);
       const float* cW = sW + (c % AR_NBUF) * (AR_KC * AR_NS_MAX) + nl;
       const float* pA = cA + p0 * AR_KC;
@@ -166,10 +136,7 @@ __device__ __forceinline__ int ar_stage(const ArW& w, int P, float* sA, float* s
 #pragma unroll
           for (int j = 0; j < AR_PT; ++j) {
             const float4 a = *reinterpret_cast<const float4*>(pA + j * AR_KC + 4 * q);
-            acc[j] = fmaf(a.x, w0, acc[j]);
-            acc[j] = fmaf(a.y, w1, acc[j]);
-            acc[j] = fmaf(a.z, w2, acc[j]);
-            acc[j] = fmaf(a.w, w3, acc[j]);
+            acc[j] = ar_fma4(acc[j], a, w0, w1, w2, w3);
           }
         }
       } else {
@@ -180,10 +147,7 @@ __device__ __forceinline__ int ar_stage(const ArW& w, int P, float* sA, float* s
           for (int j = 0; j < AR_PT; ++j) {
             if (p0 + j < P) {
               const float4 a = *reinterpret_cast<const float4*>(pA + j * AR_KC + 4 * q);
-              acc[j] = fmaf(a.x, w0, acc[j]);
-              acc[j] = fmaf(a.y, w1, acc[j]);
-              acc[j] = fmaf(a.z, w2, acc[j]);
-              acc[j] = fmaf(a.w, w3, acc[j]);
+              acc[j] = ar_fma4(acc[j], a, w0, w1, w2, w3);
             }
           }
         }
@@ -203,9 +167,7 @@ __device__ __forceinline__ int ar_stage(const ArW& w, int P, float* sA, float* s
 __device__ __forceinline__ float ar_sum(const float* red, int KS, int P, int p, int nl) {
   const int PG = (P + AR_PT - 1) / AR_PT;
   const float* r = red + ((((nl >> 5) * PG + p / AR_PT) * KS) * AR_PT + (p % AR_PT)) * 32 + (nl & 31);
-  float v = r[0];
-  for (int ks = 1; ks < KS; ++ks) v += r[ks * AR_PT * 32];
-  return v;
+  return ar_reduce(KS, [&](int ks) { return r[ks * AR_PT * 32]; });
 }
 
 // weight chunks 0 and 1 of the NEXT layer: issued before this layer's results are published, so that the loads fly during
@@ -246,7 +208,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   int n0, n1;
   ar_slice(C2, 4, rank, R, n0, n1);
   // the 12 live taps of mask 'A' are the first 12 of the 25 in raster order: weight row = tap * C + c = k
-  const ArW wA{a.w_ctx, C2, 12 * C, n0, n1 - n0, 0};
+  const ArW wA{a.w_ctx, C2, AR_TAPS * C, n0, n1 - n0, 0};
   ar_slice(a.c1, 4, rank, R, n0, n1);
   const ArW wB{a.w1, a.c1_pad, 2 * C2, n0, n1 - n0, 0};                 // (params | ctx) -> c1
   ar_slice(a.c2, 4, rank, R, n0, n1);
@@ -258,18 +220,16 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   unsigned long long t_last = d.dbg != nullptr ? ar_now() : 0ull;
   const int waves = W + 3 * (H - 1);
   for (int t = 0; t < waves; ++t) {
-    int h_lo = t - (W - 1);
-    h_lo = h_lo <= 0 ? 0 : (h_lo + 2) / 3;
-    int h_hi = t / 3;
-    if (h_hi > H - 1) h_hi = H - 1;
+    int h_lo, h_hi;
+    ar_wave_rows(t, H, W, h_lo, h_hi);
     for (int hc = h_lo; hc <= h_hi; hc += AR_PCH) {
-      const int P = (h_hi - hc + 1) < AR_PCH ? (h_hi - hc + 1) : AR_PCH;
+      const int P = ar_chunk_len(hc, h_hi);
       // ---- context model: 12 causal taps of the 5x5 window of y_hat (zero outside the latent)
       {
         auto asrc = [&](int p, int k) -> const float* {
           const int ti = k >> 7, c = k & 127;
-          const int dy = ti < 5 ? -2 : (ti < 10 ? -1 : 0);
-          const int dx = ti < 10 ? (ti - (ti < 5 ? 0 : 5)) - 2 : ti - 12;
+          int dy, dx;
+          ar_tap(ti, dy, dx);
           const int hh = hc + p + dy, ww = t - 3 * (hc + p) + dx;
           if (hh < 0 || ww < 0 || ww >= W) return nullptr;
           return yhat + ((int64_t)hh * W + ww) * C + c;
@@ -301,7 +261,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
         for (int i = threadIdx.x; i < P * wB.ns; i += AR_THREADS) {
           const int p = i / wB.ns, nl = i - p * wB.ns;
           const float v = ar_sum(red, KS, P, p, nl) + __ldg(a.b1 + wB.n0 + nl);
-          h1_s[p * a.c1_pad + wB.n0 + nl] = v > 0.f ? v : v * 0.01f;
+          h1_s[p * a.c1_pad + wB.n0 + nl] = ar_lrelu(v);
         }
       }
       AR_MARK(4);
@@ -317,7 +277,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
         for (int i = threadIdx.x; i < P * wC.ns; i += AR_THREADS) {
           const int p = i / wC.ns, nl = i - p * wC.ns;
           const float v = ar_sum(red, KS, P, p, nl) + __ldg(a.b2 + wC.n0 + nl);
-          h2_s[p * a.c2_pad + wC.n0 + nl] = v > 0.f ? v : v * 0.01f;
+          h2_s[p * a.c2_pad + wC.n0 + nl] = ar_lrelu(v);
         }
       }
       AR_MARK(7);
@@ -334,17 +294,14 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
         for (int i = threadIdx.x; i < P * nch; i += AR_THREADS) {
           const int p = i / nch, j = i - p * nch;
           const int ch = ch0 + j;
-          float scale = ar_sum(red, KS, P, p, j) + __ldg(a.b3 + ch);
+          const float scale = ar_sum(red, KS, P, p, j) + __ldg(a.b3 + ch);
           const float mean = ar_sum(red, KS, P, p, nch + j) + __ldg(a.b3 + C + ch);
           const int hh = hc + p, ww = t - 3 * hh;
           const int64_t pix = (int64_t)hh * W + ww;
           const float q = rintf(__fsub_rn(__ldg(y + pix * a.y_ld + ch), mean));
           yhat[pix * C + ch] = __fadd_rn(q, mean);
           sym[pix * C + ch] = (int32_t)q;
-          scale = fmaxf(scale, 0.11f);
-          int ix = 0;
-          for (int s = 0; s < n_cmp; ++s) ix += s_table[s] < scale ? 1 : 0;
-          idx[pix * C + ch] = ix;
+          idx[pix * C + ch] = ar_scale_index(scale, s_table, n_cmp);
         }
       }
       AR_MARK(10);
@@ -435,6 +392,7 @@ extern "C" int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t works
       e = cudaLaunchKernelEx(&cfg, ar_code_kernel, d);
     }
     if (e == cudaSuccess) {
+      if (p->cluster_used_host != nullptr) *p->cluster_used_host = R;
       if (debug) {
         unsigned long long h[16];
         cudaStreamSynchronize(st);

@@ -46,6 +46,18 @@ class ArParams(C.Structure):
                 ("w_ctx", c_fp), ("b_ctx", c_fp), ("w1", c_fp), ("b1", c_fp), ("c1", C.c_int32), ("c1_pad", C.c_int32),
                 ("w2", c_fp), ("b2", c_fp), ("c2", C.c_int32), ("c2_pad", C.c_int32), ("w3", c_fp), ("b3", c_fp),
                 ("scale_table", c_fp), ("n_scales", C.c_int32), ("y_hat", c_fp), ("symbols", c_fp), ("indexes", c_fp),
+                ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32), ("cluster", C.c_int32),
+                ("cluster_used_host", c_fp)]
+
+
+class ArDecodeParams(C.Structure):
+    _fields_ = [("params", c_fp), ("params_ld", C.c_int32),
+                ("w_ctx", c_fp), ("b_ctx", c_fp), ("w1", c_fp), ("b1", c_fp), ("c1", C.c_int32), ("c1_pad", C.c_int32),
+                ("w2", c_fp), ("b2", c_fp), ("c2", C.c_int32), ("c2_pad", C.c_int32), ("w3", c_fp), ("b3", c_fp),
+                ("scale_table", c_fp), ("n_scales", C.c_int32), ("words", c_fp), ("word_offsets", c_fp),
+                ("cdfs", c_fp), ("cdf_stride", C.c_int32), ("cdf_lengths", c_fp), ("cdf_offsets", c_fp),
+                ("n_tables", C.c_int32), ("cdf_total", C.c_int32),
+                ("y_hat", c_fp), ("symbols", c_fp), ("indexes", c_fp), ("status", c_fp),
                 ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32), ("cluster", C.c_int32)]
 
 
@@ -107,6 +119,7 @@ SIGNATURES = {
     "tdvc_eb_symbols": [vp, i32, vp, i32, i32, i32, vp, vp, vp],
     "tdvc_ar_code_workspace_bytes": [i32, i32, i32],
     "tdvc_ar_code": [C.POINTER(ArParams), vp, sz, vp],
+    "tdvc_ar_decode": [C.POINTER(ArDecodeParams), vp],
     "tdvc_rans_encode_with_indexes": [vp, vp, i64, vp, i32, vp, vp, i32, vp, i64],
     "tdvc_rans_decode_with_indexes": [vp, i64, vp, i64, vp, i32, vp, vp, i32, vp],
     "tdvc_gc_bits_backward": [vp, vp, vp, i32, vp, vp, vp, i64, i32, vp],
