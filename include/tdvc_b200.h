@@ -309,18 +309,22 @@ int tdvc_chan_dot(const float* a, const float* b_or_null, float* out, int N, int
  *   tail mass) -> n + 1 cumulative 16-bit counts; empty bins steal from the smallest bin above 1.
  * Symbols (`compress`):
  *   eb_symbols: z NHWC -> symbols round(z - median) and table indexes (= channel) in NCHW order.
+ *   TdvcArChain: the autoregressive chain of compressai's y coding, which ar_code and ar_decode must compute identically.
+ *     All pointers are DEVICE pointers.  `params`: the hyper-decoder output, NHWC rows of params_ld >= 2C floats.  Weights
+ *     in the fp32 layout of tdvc_conv2d ([tap][cin_pad][cout_pad]): w_ctx the masked 5x5 context model (C -> 2C), w1 / w2
+ *     / w3 the entropy-parameter 1x1 layers (4C -> c1 -> c2 -> 2C, LeakyReLU 0.01 between; w1 rows: hyper-decoder output
+ *     first, context second).  `scale_table`: the n_scales scales of the Gaussian tables.  Outputs, all NHWC ((h, w, c):
+ *     the order compressai codes them in): symbols round(y - mean), table indexes of max(scale, 0.11) and y_hat =
+ *     symbol + mean.
  *   ar_code: the autoregressive pass over y of compressai `_compress_ar` as wavefronts inside one launch, one thread-block
- *     cluster per image: symbols round(y - mean), table indexes of max(scale, 0.11) and y_hat = symbol + mean, all NHWC
- *     ((h, w, c): the order compressai codes them in).  Weights in the fp32 layout of tdvc_conv2d ([tap][cin_pad][cout_pad]):
- *     w_ctx the masked 5x5 context model (C -> 2C), w1 / w2 / w3 the entropy-parameter 1x1 layers (4C -> c1 -> c2 -> 2C,
- *     LeakyReLU 0.01 between; w1 rows: hyper-decoder output first, context second).  `cluster` = CTAs per image (8; 16 =
- *     non-portable size; 0 = 16 where that launches, else 8).  `cluster_used_host` (optional) receives the size
- *     launched: the summation order, and so what a decoder must reproduce, depends on it.  `workspace`: tdvc_ar_code_workspace_bytes(N, c1_pad, c2_pad) bytes.
+ *     cluster per image.  `cluster` = CTAs per image (8; 16 = non-portable size; 0 = 16 where that launches, else 8).
+ *     `cluster_used_host` (optional, HOST pointer) receives the size launched: the summation order, and so what a decoder
+ *     must reproduce, depends on it.  `workspace`: tdvc_ar_code_workspace_bytes(N, c1_pad, c2_pad) bytes.
  * Coder (HOST pointers, host code: compressai's `ans` extension runs on the CPU too): 64-bit rANS, 16-bit precision, one CDF
  *   row per table index, out-of-range symbols escape through the last bin + a 4-bit bypass code.  encode returns the stream
- *   length in bytes (< 0: error code); decode is its inverse given the same indexes.                                        */
-typedef struct TdvcArParams {
-  const float* y;        int32_t y_ld;
+ *   length in bytes (< 0: error code); decode is its inverse given the same indexes and raises on a truncated or corrupt
+ *   stream, an escape whose value does not fit in int32 included.                                                           */
+typedef struct TdvcArChain {
   const float* params;   int32_t params_ld;
   const float* w_ctx;    const float* b_ctx;
   const float* w1;       const float* b1;   int32_t c1, c1_pad;
@@ -331,37 +335,32 @@ typedef struct TdvcArParams {
   int32_t* symbols;      /* [N][H][W][C] */
   int32_t* indexes;      /* [N][H][W][C] */
   int32_t N, H, W, C;
+} TdvcArChain;
+typedef struct TdvcArParams {
+  TdvcArChain chain;
+  const float* y;        int32_t y_ld;
   int32_t cluster;
   int32_t* cluster_used_host;
 } TdvcArParams;
 /* ar_decode: the inverse of ar_code (compressai `_decompress_ar`), one thread-block cluster per image walking the latent in
  *   raster order: per position the context model over the already decoded y_hat, the three entropy-parameter layers, then
  *   the 128 symbols of the position from the rANS stream (on the device, compressai's bypass escape included), y_hat =
- *   symbol + mean.  The predictions are bit-identical to ar_code's for the same weights and params only if ar_code ran with
- *   `cluster` CTAs per image (its K splits, and so its fp32 summation order, depend on it): pass the encoder's cluster size
- *   (8 or 16; a container records it).  All pointers are DEVICE pointers.  `words` / `word_offsets`: the N y strings as
- *   32-bit little-endian words, string n = words[word_offsets[n] .. word_offsets[n + 1]).  `cdfs` [n_tables][cdf_stride],
- *   `cdf_lengths`, `cdf_offsets`: the Gaussian tables of the rANS coder; cdf_total = sum of cdf_lengths.  Outputs as ar_code
- *   (NHWC) plus `status` [N]: -1 when image n decoded, -2 when the CDF tables are not valid rows (lengths outside
+ *   symbol + mean.  The predictions are bit-identical to ar_code's for the same chain only if ar_code ran with `cluster`
+ *   CTAs per image (its K splits, and so its fp32 summation order, depend on it): pass the encoder's cluster size (8 or 16;
+ *   a container records it).  All pointers are DEVICE pointers.  `words` / `word_offsets`: the N y strings as 32-bit
+ *   little-endian words, string n = words[word_offsets[n] .. word_offsets[n + 1]).  `cdfs` [n_tables][cdf_stride],
+ *   `cdf_lengths`, `cdf_offsets`: the Gaussian tables of the rANS coder; cdf_total = sum of cdf_lengths.  Outputs those of
+ *   the chain plus `status` [N]: -1 when image n decoded, -2 when the CDF tables are not valid rows (lengths outside
  *   [2, cdf_stride] or not summing to cdf_total; nothing is decoded), else the index (h * W + w) * C + c of the first
- *   symbol that could not be decoded (truncated or corrupt stream; nothing after it is written).  A malformed stream never faults the kernel: the
- *   caller reads `status` after the stream synchronises.                                                                    */
+ *   symbol that could not be decoded (truncated or corrupt stream; nothing after it is written).  A malformed stream never
+ *   faults the kernel: the caller reads `status` after the stream synchronises.                                            */
 typedef struct TdvcArDecodeParams {
-  const float* params;   int32_t params_ld;
-  const float* w_ctx;    const float* b_ctx;
-  const float* w1;       const float* b1;   int32_t c1, c1_pad;
-  const float* w2;       const float* b2;   int32_t c2, c2_pad;
-  const float* w3;       const float* b3;
-  const float* scale_table;  int32_t n_scales;
+  TdvcArChain chain;
   const uint32_t* words;  const int64_t* word_offsets;
   const int32_t* cdfs;   int32_t cdf_stride;
   const int32_t* cdf_lengths;  const int32_t* cdf_offsets;
   int32_t n_tables, cdf_total;
-  float* y_hat;          /* [N][H][W][C] */
-  int32_t* symbols;      /* [N][H][W][C] */
-  int32_t* indexes;      /* [N][H][W][C] */
   int64_t* status;       /* [N] */
-  int32_t N, H, W, C;
   int32_t cluster;
 } TdvcArDecodeParams;
 int tdvc_pmf_to_quantized_cdf(const float* pmf, int n, int precision, int32_t* cdf);

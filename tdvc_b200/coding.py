@@ -189,6 +189,22 @@ def _pinned(plan, name, like):
     return t
 
 
+def _ar_chain(W, cn, tables, params, out, who):
+    """The autoregressive chain of coder `cn` ("mv" | "rs") as tdvc_ar_code and tdvc_ar_decode both read it: its four layers,
+    the scale table, the hyper-decoder output `params` (a channels-last Act (N, h, w, >= 256 channels)) and the outputs
+    out = (y_hat, symbols, indexes), each (N, h, w, 128)."""
+    ctx, e0, e2, e4 = W[f"{cn}.ctx"], W[f"{cn}.ep0"], W[f"{cn}.ep2"], W[f"{cn}.ep4"]
+    if ctx.cin_pad != 128 or ctx.cout_pad != 256 or e0.cin_pad != 512 or e2.cin_pad < e0.cout_pad - 4 or e4.cout_pad != 256:
+        raise RuntimeError(f"{who}: unexpected entropy-parameter layer shapes")
+    y_hat, y_sym, y_idx = out
+    return L.ArChain(params=params.ptr, params_ld=params.ld, w_ctx=ctx.w.data_ptr(), b_ctx=ctx.b.data_ptr(),
+                     w1=e0.w.data_ptr(), b1=e0.b.data_ptr(), c1=e0.cout, c1_pad=e0.cout_pad,
+                     w2=e2.w.data_ptr(), b2=e2.b.data_ptr(), c2=e2.cout, c2_pad=e2.cout_pad,
+                     w3=e4.w.data_ptr(), b3=e4.b.data_ptr(), scale_table=tables.scale_table.data_ptr(),
+                     n_scales=SCALES_LEVELS, y_hat=y_hat.data_ptr(), symbols=y_sym.data_ptr(), indexes=y_idx.data_ptr(),
+                     N=params.N, H=params.H, W=params.W, C=128)
+
+
 def launch_coding(plan, W, cn, tables, cluster=0, stream=None):
     """Device half of compressai `compress()` for coder `cn` ("mv" | "rs") on the latents the forward pass of `plan` just
     produced: symbols + table indexes of z and y, copied to pinned host memory on `stream`.  Returns a handle for
@@ -207,22 +223,14 @@ def launch_coding(plan, W, cn, tables, cluster=0, stream=None):
     L.check(lib.tdvc_eb_symbols(z.ptr, z.ld, med.data_ptr(), N, hz * wz, 128, z_sym.data_ptr(), z_idx.data_ptr(), st),
             "eb_symbols")
     # ---- y: autoregressive pass, (h, w, c) symbol order
-    ctx, e0, e2, e4 = W[f"{cn}.ctx"], W[f"{cn}.ep0"], W[f"{cn}.ep2"], W[f"{cn}.ep4"]
     y_hat = plan.raw(f"{cn}.ac.y_hat", (N, hy, wy, 128))
     y_sym = plan.raw(f"{cn}.ac.y_sym", (N, hy, wy, 128), torch.int32)
     y_idx = plan.raw(f"{cn}.ac.y_idx", (N, hy, wy, 128), torch.int32)
-    if ctx.cin_pad != 128 or ctx.cout_pad != 256 or e0.cin_pad != 512 or e2.cin_pad < e0.cout_pad - 4 or e4.cout_pad != 256:
-        raise RuntimeError("code_latents: unexpected entropy-parameter layer shapes")
-    need = lib.tdvc_ar_code_workspace_bytes(N, e0.cout_pad, e2.cout_pad)
+    chain = _ar_chain(W, cn, tables, params, (y_hat, y_sym, y_idx), "code_latents")
+    need = lib.tdvc_ar_code_workspace_bytes(N, chain.c1_pad, chain.c2_pad)
     ws = plan.raw(f"{cn}.ac.ws", ((need + 3) // 4,))
-    p = L.ArParams(y=y.ptr, y_ld=y.ld, params=params.ptr, params_ld=params.ld, w_ctx=ctx.w.data_ptr(), b_ctx=ctx.b.data_ptr(),
-                   w1=e0.w.data_ptr(), b1=e0.b.data_ptr(), c1=e0.cout, c1_pad=e0.cout_pad,
-                   w2=e2.w.data_ptr(), b2=e2.b.data_ptr(), c2=e2.cout, c2_pad=e2.cout_pad,
-                   w3=e4.w.data_ptr(), b3=e4.b.data_ptr(), scale_table=tables.scale_table.data_ptr(), n_scales=SCALES_LEVELS,
-                   y_hat=y_hat.data_ptr(), symbols=y_sym.data_ptr(), indexes=y_idx.data_ptr(), N=N, H=hy, W=wy, C=128,
-                   cluster=cluster)
     used = C.c_int32(0)
-    p.cluster_used_host = C.addressof(used)
+    p = L.ArParams(chain=chain, y=y.ptr, y_ld=y.ld, cluster=cluster, cluster_used_host=C.addressof(used))
     L.check(lib.tdvc_ar_code(C.byref(p), ws.data_ptr(), need, st), "ar_code")
     plan.launches += 2
     host = []
@@ -273,9 +281,6 @@ def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
         if len(s_) < 8 or len(s_) % 4:
             raise RuntimeError(f"decode_latents: {cn} y string of image {i} has {len(s_)} bytes (rANS strings are whole "
                                "32-bit words, at least two)")
-    ctx, e0, e2, e4 = W[f"{cn}.ctx"], W[f"{cn}.ep0"], W[f"{cn}.ep2"], W[f"{cn}.ep4"]
-    if ctx.cin_pad != 128 or ctx.cout_pad != 256 or e0.cin_pad != 512 or e2.cin_pad < e0.cout_pad - 4 or e4.cout_pad != 256:
-        raise RuntimeError("decode_latents: unexpected entropy-parameter layer shapes")
     gl = tables.gc.length
     if gl.size > 64 or (gl < 2).any() or (gl > tables.gc.cdf.shape[1]).any() or int(gl.sum()) > 32768:
         raise RuntimeError("decode_latents: the Gaussian CDF tables are not valid rows for the device decoder")
@@ -290,15 +295,11 @@ def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
         y_sym = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
         y_idx = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
         status = torch.empty((N,), device=dev, dtype=torch.int64)
-    p = L.ArDecodeParams(params=params.ptr, params_ld=params.ld, w_ctx=ctx.w.data_ptr(), b_ctx=ctx.b.data_ptr(),
-                         w1=e0.w.data_ptr(), b1=e0.b.data_ptr(), c1=e0.cout, c1_pad=e0.cout_pad,
-                         w2=e2.w.data_ptr(), b2=e2.b.data_ptr(), c2=e2.cout, c2_pad=e2.cout_pad,
-                         w3=e4.w.data_ptr(), b3=e4.b.data_ptr(), scale_table=tables.scale_table.data_ptr(),
-                         n_scales=SCALES_LEVELS, words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
+    p = L.ArDecodeParams(chain=_ar_chain(W, cn, tables, params, (y_hat, y_sym, y_idx), "decode_latents"),
+                         words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
                          cdfs=cdf.data_ptr(), cdf_stride=cdf.shape[1], cdf_lengths=length.data_ptr(),
-                         cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(tables.gc.length.sum()),
-                         y_hat=y_hat.data_ptr(), symbols=y_sym.data_ptr(), indexes=y_idx.data_ptr(),
-                         status=status.data_ptr(), N=N, H=hy, W=wy, C=128, cluster=cluster)
+                         cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(gl.sum()),
+                         status=status.data_ptr(), cluster=cluster)
     L.check(lib.tdvc_ar_decode(C.byref(p), stream.cuda_stream), "ar_decode")
     with torch.cuda.stream(stream):
         status_h = _pinned_like(status)

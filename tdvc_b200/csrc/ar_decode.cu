@@ -29,13 +29,6 @@ constexpr int ARD_IN_MAX = 512;      // widest layer input (ep0: params | ctx)
 // of static shared memory fit beside it.
 constexpr size_t ARD_SMEM = (size_t)ARD_CDF_MAX * sizeof(int32_t);
 constexpr int64_t ARD_BAD_TABLES = -2;   // status: the CDF tables are not valid rows
-constexpr uint64_t ARD_RANS_L = 1ull << 31;
-constexpr int ARD_PRECISION = 16, ARD_BYPASS = 4;
-constexpr uint32_t ARD_MAX_BYPASS = (1u << ARD_BYPASS) - 1;
-
-struct ArdDev {
-  TdvcArDecodeParams a;
-};
 
 // the rANS decoder state of one image, held identically by the 32 lanes of the decoding warp; a window of 32 stream words
 // (lane j holds word win + j) keeps the renormalisation reads off the L2 latency
@@ -57,7 +50,7 @@ struct ArdRans {
     return true;
   }
   __device__ __forceinline__ bool renorm() {
-    if (x < ARD_RANS_L) {
+    if (x < RANS64_L) {
       uint32_t v;
       if (!next(v)) return false;
       x = (x << 32) | v;
@@ -65,8 +58,8 @@ struct ArdRans {
     return true;
   }
   __device__ __forceinline__ bool bits(uint32_t& v) {
-    v = (uint32_t)(x & ARD_MAX_BYPASS);
-    x >>= ARD_BYPASS;
+    v = (uint32_t)(x & RANS_MAX_BYPASS);
+    x >>= RANS_BYPASS;
     return renorm();
   }
 };
@@ -76,7 +69,7 @@ struct ArdRans {
 // one shared-memory load and one ballot for a 3,133-entry row.  false: corrupt or truncated stream.
 __device__ __forceinline__ bool ard_decode_symbol(ArdRans& r, const int32_t* cdf, int len, int32_t offset, int32_t& sym) {
   const int lane = threadIdx.x & 31;
-  const uint32_t cum = (uint32_t)(r.x & ((1u << ARD_PRECISION) - 1));
+  const uint32_t cum = (uint32_t)(r.x & ((1u << RANS_PRECISION) - 1));
   if ((uint32_t)cdf[len - 1] <= cum) return false;
   int lo = 0, hi = len - 1;   // the symbol s = max{j < len - 1 : cdf[j] <= cum} lies in [lo, hi)
   while (hi - lo > 1) {
@@ -90,43 +83,8 @@ __device__ __forceinline__ bool ard_decode_symbol(ArdRans& r, const int32_t* cdf
   }
   const int s = lo;
   const uint32_t start = (uint32_t)cdf[s], freq = (uint32_t)(cdf[s + 1] - cdf[s]);
-  r.x = (uint64_t)freq * (r.x >> ARD_PRECISION) + (r.x & ((1u << ARD_PRECISION) - 1)) - start;
-  if (!r.renorm()) return false;
-  int64_t value = s;
-  const int max_value = len - 2;
-  if (s == max_value) {
-    uint32_t v;
-    if (!r.bits(v)) return false;
-    int n_bypass = (int)v;
-    while (v == ARD_MAX_BYPASS) {
-      if (n_bypass > 16 || !r.bits(v)) return false;
-      n_bypass += (int)v;
-    }
-    if (n_bypass > 16) return false;
-    uint64_t raw = 0;
-    for (int j = 0; j < n_bypass; ++j) {
-      if (!r.bits(v)) return false;
-      raw |= (uint64_t)v << (j * ARD_BYPASS);
-    }
-    if ((raw >> 1) > (1ull << 32)) return false;
-    value = (int64_t)(raw >> 1);
-    if (raw & 1) value = -value - 1;
-    else value += max_value;
-  }
-  value += offset;
-  if (value < INT32_MIN || value > INT32_MAX) return false;
-  sym = (int32_t)value;
-  return true;
-}
-
-// encoder column count of the CTA that owns output channel n of a layer with `total` outputs (R encoder CTAs)
-__device__ __forceinline__ int ard_encoder_ns(int total, int n, int R) {
-  for (int r = 0; r < R; ++r) {
-    int n0, n1;
-    ar_slice(total, 4, r, R, n0, n1);
-    if (n >= n0 && n < n1) return n1 - n0;
-  }
-  return 0;
+  r.x = (uint64_t)freq * (r.x >> RANS_PRECISION) + (r.x & ((1u << RANS_PRECISION) - 1)) - start;
+  return r.renorm() && rans_symbol(s, len - 2, offset, [&](uint32_t& v) { return r.bits(v); }, sym);
 }
 
 // split partials of this CTA's outputs of layer w for one position: part[ks][nl] = the encoder's fmaf chain of split ks of
@@ -175,13 +133,13 @@ __device__ __forceinline__ void ard_publish(cg::cluster_group& cluster, int RD, 
   }
 }
 
-__global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const ArdDev d) {
+__global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const TdvcArDecodeParams p) {
   cg::cluster_group cluster = cg::this_cluster();
   const int RD = (int)cluster.num_blocks();
   const int rank = (int)cluster.block_rank();
   const int n = blockIdx.x / RD;
-  const TdvcArDecodeParams& a = d.a;
-  const int H = a.H, W = a.W, Re = a.cluster;
+  const TdvcArChain& a = p.chain;
+  const int H = a.H, W = a.W;
   constexpr int C = AR_C, C2 = 2 * AR_C;
   extern __shared__ __align__(16) int32_t ard_cdf[];   // [cdf_total]: the CDF rows back to back (CTA 0)
   __shared__ __align__(16) float s_taps[AR_TAPS * C];  // context-model input: the 12 causal taps of y_hat
@@ -198,21 +156,23 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const ArdDev d
   __shared__ int s_row[ARD_TABLES_MAX + 1], s_len[ARD_TABLES_MAX], s_off[ARD_TABLES_MAX];
   __shared__ int s_stop;                               // written by CTA 0 into every CTA: stop decoding this image
 
-  int n0, n1;
-  ar_slice(C2, 4, rank, RD, n0, n1);
-  const ArW wA{a.w_ctx, C2, AR_TAPS * C, n0, n1 - n0, 0};
-  ar_slice(a.c1, 4, rank, RD, n0, n1);
-  const ArW wB{a.w1, a.c1_pad, 2 * C2, n0, n1 - n0, 0};
-  ar_slice(a.c2, 4, rank, RD, n0, n1);
-  const ArW wC{a.w2, a.c2_pad, (a.c1 + 3) & ~3, n0, n1 - n0, 0};
-  ar_slice(C, 4, rank, RD, n0, n1);
-  const ArW wD{a.w3, C2, (a.c2 + 3) & ~3, n0, 2 * (n1 - n0), n1 - n0};
-
+  const ArW wA = ar_layer(a, AR_CTX, rank, RD), wB = ar_layer(a, AR_EP0, rank, RD), wC = ar_layer(a, AR_EP2, rank, RD),
+            wD = ar_layer(a, AR_EP4, rank, RD);
+  // column count of the encoder CTA (of a cluster of p.cluster) that owns output j of this CTA's layer L: it fixes the
+  // output's K splits
+  auto encoder_ns = [&](ArLayer L, const ArW& w, int j) {
+    const int ch = w.n0 + (w.split && j >= w.split ? j - w.split : j);   // ep4: the latent channel of a scale or mean
+    for (int r = 0; r < p.cluster; ++r) {
+      const ArW e = ar_layer(a, L, r, p.cluster);
+      if (ch >= e.n0 && ch < e.n0 + (e.split ? e.split : e.ns)) return e.ns;
+    }
+    return 0;
+  };
   for (int i = threadIdx.x; i < ARD_NO_MAX; i += AR_THREADS) {
-    s_ns[0][i] = i < wA.ns ? ard_encoder_ns(C2, wA.n0 + i, Re) : 0;
-    s_ns[1][i] = i < wB.ns ? ard_encoder_ns(a.c1, wB.n0 + i, Re) : 0;
-    s_ns[2][i] = i < wC.ns ? ard_encoder_ns(a.c2, wC.n0 + i, Re) : 0;
-    s_ns[3][i] = i < wD.ns ? 2 * ard_encoder_ns(C, wD.n0 + (i < wD.split ? i : i - wD.split), Re) : 0;
+    s_ns[AR_CTX][i] = i < wA.ns ? encoder_ns(AR_CTX, wA, i) : 0;
+    s_ns[AR_EP0][i] = i < wB.ns ? encoder_ns(AR_EP0, wB, i) : 0;
+    s_ns[AR_EP2][i] = i < wC.ns ? encoder_ns(AR_EP2, wC, i) : 0;
+    s_ns[AR_EP4][i] = i < wD.ns ? encoder_ns(AR_EP4, wD, i) : 0;
   }
   for (int i = threadIdx.x; i < ARD_IN_MAX; i += AR_THREADS) s_in2[i] = s_in3[i] = 0.f;
   for (int i = threadIdx.x; i < a.n_scales - 1; i += AR_THREADS) s_table[i] = a.scale_table[i];
@@ -224,28 +184,28 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const ArdDev d
     if (threadIdx.x == 0) {
       int total = 0;
       bool ok = true;
-      for (int t = 0; t < a.n_tables; ++t) {
-        const int len = a.cdf_lengths[t];
-        ok = ok && len >= 2 && len <= a.cdf_stride;
+      for (int t = 0; t < p.n_tables; ++t) {
+        const int len = p.cdf_lengths[t];
+        ok = ok && len >= 2 && len <= p.cdf_stride;
         s_row[t] = total;
         s_len[t] = len;
-        s_off[t] = a.cdf_offsets[t];
+        s_off[t] = p.cdf_offsets[t];
         total += ok ? len : 0;
       }
-      ok = ok && total == a.cdf_total;
-      const int64_t w0 = a.word_offsets[n], w1 = a.word_offsets[n + 1];
+      ok = ok && total == p.cdf_total;
+      const int64_t w0 = p.word_offsets[n], w1 = p.word_offsets[n + 1];
       s_stop = ok && w1 - w0 >= 2 ? 0 : 1;
-      a.status[n] = !ok ? ARD_BAD_TABLES : (s_stop ? 0 : -1);
+      p.status[n] = !ok ? ARD_BAD_TABLES : (s_stop ? 0 : -1);
     }
     __syncthreads();
     if (!s_stop) {
-      for (int t = 0; t < a.n_tables; ++t)
-        for (int i = threadIdx.x; i < s_len[t]; i += AR_THREADS) ard_cdf[s_row[t] + i] = a.cdfs[(int64_t)t * a.cdf_stride + i];
+      for (int t = 0; t < p.n_tables; ++t)
+        for (int i = threadIdx.x; i < s_len[t]; i += AR_THREADS) ard_cdf[s_row[t] + i] = p.cdfs[(int64_t)t * p.cdf_stride + i];
     }
     if (coder) {
-      const int64_t w0 = a.word_offsets[n];
-      rs.words = a.words + w0;
-      rs.nw = a.word_offsets[n + 1] - w0;
+      const int64_t w0 = p.word_offsets[n];
+      rs.words = p.words + w0;
+      rs.nw = p.word_offsets[n + 1] - w0;
       rs.pos = 2;
       rs.win = -64;
       if (!s_stop) rs.x = (uint64_t)__ldg(rs.words) | ((uint64_t)__ldg(rs.words + 1) << 32);
@@ -272,26 +232,26 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const ArdDev d
     for (int i = threadIdx.x; i < C2; i += AR_THREADS) s_in1[i] = __ldg(prm + (int64_t)pix * a.params_ld + i);
     __syncthreads();
     // ---- context model -> ctx half of ep0's input
-    ard_partials(wA, s_ns[0], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_taps + k); });
+    ard_partials(wA, s_ns[AR_CTX], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_taps + k); });
     __syncthreads();
-    ard_publish<false>(cluster, RD, wA, a.b_ctx, s_ns[0], P, s_part, s_out, s_in1 + C2);
+    ard_publish<false>(cluster, RD, wA, a.b_ctx, s_ns[AR_CTX], P, s_part, s_out, s_in1 + C2);
     cluster.sync();
     // ---- ep0: (params | ctx) -> c1, LeakyReLU
-    ard_partials(wB, s_ns[1], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_in1 + k); });
+    ard_partials(wB, s_ns[AR_EP0], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_in1 + k); });
     __syncthreads();
-    ard_publish<true>(cluster, RD, wB, a.b1, s_ns[1], P, s_part, s_out, s_in2);
+    ard_publish<true>(cluster, RD, wB, a.b1, s_ns[AR_EP0], P, s_part, s_out, s_in2);
     cluster.sync();
     // ---- ep2: c1 -> c2, LeakyReLU
-    ard_partials(wC, s_ns[2], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_in2 + k); });
+    ard_partials(wC, s_ns[AR_EP2], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_in2 + k); });
     __syncthreads();
-    ard_publish<true>(cluster, RD, wC, a.b2, s_ns[2], P, s_part, s_out, s_in3);
+    ard_publish<true>(cluster, RD, wC, a.b2, s_ns[AR_EP2], P, s_part, s_out, s_in3);
     cluster.sync();
     // ---- ep4: c2 -> (scales | means) of this CTA's latent channels, to CTA 0
-    ard_partials(wD, s_ns[3], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_in3 + k); });
+    ard_partials(wD, s_ns[AR_EP4], P, s_part, [&](int k) { return *reinterpret_cast<const float4*>(s_in3 + k); });
     __syncthreads();
     for (int j = threadIdx.x; j < wD.split; j += AR_THREADS) {
-      const float scale = ard_output(wD, a.b3, s_ns[3], P, s_part, j);
-      const float mean = ard_output(wD, a.b3, s_ns[3], P, s_part, wD.split + j);
+      const float scale = ard_output(wD, a.b3, s_ns[AR_EP4], P, s_part, j);
+      const float mean = ard_output(wD, a.b3, s_ns[AR_EP4], P, s_part, wD.split + j);
       *cluster.map_shared_rank(&s_mean[wD.n0 + j], 0) = mean;
       *cluster.map_shared_rank(&s_idx[wD.n0 + j], 0) = ar_scale_index(scale, s_table, n_cmp);
     }
@@ -317,7 +277,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const ArdDev d
           yhat[o] = __fadd_rn((float)s_sym[c], s_mean[c]);
         }
       } else if (threadIdx.x == 0) {
-        a.status[n] = (int64_t)pix * C + bad;
+        p.status[n] = (int64_t)pix * C + bad;
         for (int r = 0; r < RD; ++r) *cluster.map_shared_rank(&s_stop, r) = 1;
       }
       __threadfence();
@@ -333,53 +293,16 @@ using namespace tdvc;
 
 extern "C" int tdvc_ar_decode(const TdvcArDecodeParams* p, void* stream) {
   TDVC_REQUIRE(p != nullptr, "ar_decode: null params");
-  TDVC_REQUIRE(p->params && p->w_ctx && p->b_ctx && p->w1 && p->b1 && p->w2 && p->b2 && p->w3 && p->b3 && p->scale_table &&
-                   p->words && p->word_offsets && p->cdfs && p->cdf_lengths && p->cdf_offsets && p->y_hat && p->symbols &&
-                   p->indexes && p->status, "ar_decode: null pointer");
-  TDVC_REQUIRE(p->C == AR_C, "ar_decode: C=%d (only %d latent channels)", p->C, AR_C);
-  TDVC_REQUIRE(p->N > 0 && p->H > 0 && p->W > 0, "ar_decode: bad shape");
-  TDVC_REQUIRE(p->params_ld >= 2 * AR_C && p->params_ld % 4 == 0, "ar_decode: bad leading dimension");
-  TDVC_REQUIRE(p->c1 >= 16 && p->c2 >= 16 && p->c2 <= p->c1 && p->c1 <= ARD_IN_MAX && p->c1_pad % 4 == 0 &&
-                   p->c1_pad >= ((p->c1 + 3) & ~3) && p->c2_pad % 4 == 0 && p->c2_pad >= ((p->c2 + 3) & ~3) &&
-                   (p->c1 + 7) / 8 + 1 <= AR_NS_MAX, "ar_decode: hidden widths %d, %d", p->c1, p->c2);
-  TDVC_REQUIRE(p->n_scales >= 2 && p->n_scales <= 65, "ar_decode: scale table of %d entries", p->n_scales);
-  TDVC_REQUIRE(p->n_tables >= p->n_scales && p->n_tables <= ARD_TABLES_MAX && p->cdf_stride >= 3,
-               "ar_decode: %d tables for %d scales", p->n_tables, p->n_scales);
+  const int rc = ar_check_chain(p->chain, "ar_decode");
+  if (rc != TDVC_OK) return rc;
+  TDVC_REQUIRE(p->words && p->word_offsets && p->cdfs && p->cdf_lengths && p->cdf_offsets && p->status,
+               "ar_decode: null pointer");
+  TDVC_REQUIRE(p->n_tables >= p->chain.n_scales && p->n_tables <= ARD_TABLES_MAX && p->cdf_stride >= 3,
+               "ar_decode: %d tables for %d scales", p->n_tables, p->chain.n_scales);
   TDVC_REQUIRE(p->cdf_total > 0 && p->cdf_total <= ARD_CDF_MAX, "ar_decode: %d CDF entries (at most %d)", p->cdf_total,
                ARD_CDF_MAX);
   TDVC_REQUIRE(p->cluster == 8 || p->cluster == 16, "ar_decode: encoder cluster size %d (8 or 16)", p->cluster);
-  cudaStream_t st = (cudaStream_t)stream;
-  static int smem_done[kMaxDevices] = {};
-  {
-    const int rc = ensure_dynamic_smem(ar_decode_kernel, ARD_SMEM, smem_done, "ar_decode");
-    if (rc != TDVC_OK) return rc;
-  }
-  ArdDev d;
-  d.a = *p;
-  // 16 CTAs per image (non-portable cluster size), 8 where that cannot launch; the result does not depend on it
-  for (int R = 16;; R = 8) {
-    cudaError_t e = cudaSuccess;
-    if (R > 8) e = cudaFuncSetAttribute(ar_decode_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    if (e == cudaSuccess) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3((unsigned)(p->N * R));
-      cfg.blockDim = dim3(AR_THREADS);
-      cfg.dynamicSmemBytes = ARD_SMEM;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = (unsigned)R;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      e = cudaLaunchKernelEx(&cfg, ar_decode_kernel, d);
-    }
-    if (e == cudaSuccess) return TDVC_OK;
-    (void)cudaGetLastError();
-    if (R == 8) {
-      set_error("ar_decode: launch with clusters of %d CTAs failed: %s", R, cudaGetErrorString(e));
-      return TDVC_ECUDA;
-    }
-  }
+  // 16 CTAs per image, 8 where that cannot launch; the result does not depend on it
+  int R = 16;
+  return ar_launch_clusters<ar_decode_kernel>(*p, p->chain.N, R, true, ARD_SMEM, (cudaStream_t)stream, "ar_decode");
 }

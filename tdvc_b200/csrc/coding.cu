@@ -184,7 +184,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   const int R = (int)cluster.num_blocks();
   const int rank = (int)cluster.block_rank();
   const int n = blockIdx.x / R;
-  const TdvcArParams& a = d.a;
+  const TdvcArChain& a = d.a.chain;
   const int H = a.H, W = a.W;
   constexpr int C = AR_C, C2 = 2 * AR_C;
   extern __shared__ __align__(16) float ar_smem[];
@@ -197,7 +197,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   const int n_cmp = a.n_scales - 1;
 
   float* yhat = a.y_hat + (int64_t)n * H * W * C;
-  const float* y = a.y + (int64_t)n * H * W * a.y_ld;
+  const float* y = d.a.y + (int64_t)n * H * W * d.a.y_ld;
   const float* prm = a.params + (int64_t)n * H * W * a.params_ld;
   float* ctx_s = d.ctx_s + (int64_t)n * AR_PCH * C2;
   float* h1_s = d.h1_s + (int64_t)n * AR_PCH * a.c1_pad;
@@ -205,16 +205,8 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   int32_t* sym = a.symbols + (int64_t)n * H * W * C;
   int32_t* idx = a.indexes + (int64_t)n * H * W * C;
 
-  int n0, n1;
-  ar_slice(C2, 4, rank, R, n0, n1);
-  // the 12 live taps of mask 'A' are the first 12 of the 25 in raster order: weight row = tap * C + c = k
-  const ArW wA{a.w_ctx, C2, AR_TAPS * C, n0, n1 - n0, 0};
-  ar_slice(a.c1, 4, rank, R, n0, n1);
-  const ArW wB{a.w1, a.c1_pad, 2 * C2, n0, n1 - n0, 0};                 // (params | ctx) -> c1
-  ar_slice(a.c2, 4, rank, R, n0, n1);
-  const ArW wC{a.w2, a.c2_pad, (a.c1 + 3) & ~3, n0, n1 - n0, 0};        // c1 -> c2
-  ar_slice(C, 4, rank, R, n0, n1);                                      // latent channels [n0, n1) of this CTA
-  const ArW wD{a.w3, C2, (a.c2 + 3) & ~3, n0, 2 * (n1 - n0), n1 - n0};  // c2 -> (scales | means)
+  const ArW wA = ar_layer(a, AR_CTX, rank, R), wB = ar_layer(a, AR_EP0, rank, R), wC = ar_layer(a, AR_EP2, rank, R),
+            wD = ar_layer(a, AR_EP4, rank, R);
 
   ar_prefetch_w(wA, sW);
   unsigned long long t_last = d.dbg != nullptr ? ar_now() : 0ull;
@@ -298,7 +290,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
           const float mean = ar_sum(red, KS, P, p, nch + j) + __ldg(a.b3 + C + ch);
           const int hh = hc + p, ww = t - 3 * hh;
           const int64_t pix = (int64_t)hh * W + ww;
-          const float q = rintf(__fsub_rn(__ldg(y + pix * a.y_ld + ch), mean));
+          const float q = rintf(__fsub_rn(__ldg(y + pix * d.a.y_ld + ch), mean));
           yhat[pix * C + ch] = __fadd_rn(q, mean);
           sym[pix * C + ch] = (int32_t)q;
           idx[pix * C + ch] = ar_scale_index(scale, s_table, n_cmp);
@@ -314,10 +306,6 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
 }
 
 // ------------------------------------------------------------------------------------------------ host rANS
-constexpr uint64_t RANS64_L = 1ull << 31;
-constexpr int RANS_PRECISION = 16, RANS_BYPASS = 4;
-constexpr int32_t RANS_MAX_BYPASS = (1 << RANS_BYPASS) - 1;
-
 struct RansSym {
   uint32_t start;
   uint32_t range;   // 0 = bypass digit (value in `start`)
@@ -334,20 +322,14 @@ extern "C" size_t tdvc_ar_code_workspace_bytes(int N, int c1_pad, int c2_pad) {
 
 extern "C" int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t workspace_bytes, void* stream) {
   TDVC_REQUIRE(p != nullptr, "ar_code: null params");
-  TDVC_REQUIRE(p->y && p->params && p->w_ctx && p->b_ctx && p->w1 && p->b1 && p->w2 && p->b2 && p->w3 && p->b3 &&
-                   p->scale_table && p->y_hat && p->symbols && p->indexes, "ar_code: null pointer");
-  TDVC_REQUIRE(p->C == AR_C, "ar_code: C=%d (only %d latent channels)", p->C, AR_C);
-  TDVC_REQUIRE(p->N > 0 && p->H > 0 && p->W > 0, "ar_code: bad shape");
-  TDVC_REQUIRE(p->y_ld >= AR_C && p->params_ld >= 2 * AR_C && p->params_ld % 4 == 0, "ar_code: bad leading dimensions");
-  TDVC_REQUIRE(p->c1 > 0 && p->c1_pad >= ((p->c1 + 3) & ~3) && p->c1_pad % 4 == 0 && p->c2 > 0 &&
-                   p->c2_pad >= ((p->c2 + 3) & ~3) && p->c2_pad % 4 == 0, "ar_code: bad hidden widths");
-  TDVC_REQUIRE(p->n_scales >= 2 && p->n_scales <= 65, "ar_code: scale table of %d entries", p->n_scales);
-  const bool auto_r = p->cluster <= 0;   // auto: 16 CTAs per image (non-portable cluster size), 8 where that cannot launch
+  const int rc = ar_check_chain(p->chain, "ar_code");
+  if (rc != TDVC_OK) return rc;
+  const TdvcArChain& a = p->chain;
+  TDVC_REQUIRE(p->y && p->y_ld >= AR_C, "ar_code: bad y");
+  const bool auto_r = p->cluster <= 0;   // auto: 16 CTAs per image, 8 where that cannot launch
   int R = auto_r ? 16 : p->cluster;
   TDVC_REQUIRE(R == 8 || R == 16, "ar_code: cluster size %d (8 or 16)", R);
-  TDVC_REQUIRE((p->c1 + 7) / 8 + 1 <= AR_NS_MAX && p->c1 >= 16 && p->c2 >= 16 && p->c2 <= p->c1,
-               "ar_code: hidden widths %d, %d", p->c1, p->c2);
-  const size_t need = tdvc_ar_code_workspace_bytes(p->N, p->c1_pad, p->c2_pad);
+  const size_t need = tdvc_ar_code_workspace_bytes(a.N, a.c1_pad, a.c2_pad);
   TDVC_REQUIRE(workspace != nullptr && workspace_bytes >= need, "ar_code: workspace of %zu bytes, %zu needed", workspace_bytes, need);
   cudaStream_t st = (cudaStream_t)stream;
   // the padded tail of the hidden rows is read (times zero weight rows): it must hold finite numbers
@@ -358,8 +340,8 @@ extern "C" int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t works
   ArDev d;
   d.a = *p;
   d.ctx_s = (float*)workspace;
-  d.h1_s = d.ctx_s + (size_t)p->N * AR_PCH * 2 * AR_C;
-  d.h2_s = d.h1_s + (size_t)p->N * AR_PCH * p->c1_pad;
+  d.h1_s = d.ctx_s + (size_t)a.N * AR_PCH * 2 * AR_C;
+  d.h2_s = d.h1_s + (size_t)a.N * AR_PCH * a.c1_pad;
   d.dbg = nullptr;
   static unsigned long long* dbg_buf = nullptr;
   const bool debug = getenv("TDVC_B200_AR_DEBUG") != nullptr;
@@ -368,46 +350,18 @@ extern "C" int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t works
     cudaMemsetAsync(dbg_buf, 0, 16 * sizeof(unsigned long long), st);
     d.dbg = dbg_buf;
   }
-  static int smem_done[kMaxDevices] = {};
-  {
-    const int rc = ensure_dynamic_smem(ar_code_kernel, AR_SMEM, smem_done, "ar_code");
-    if (rc != TDVC_OK) return rc;
+  const int lrc = ar_launch_clusters<ar_code_kernel>(d, a.N, R, auto_r, AR_SMEM, st, "ar_code");
+  if (lrc != TDVC_OK) return lrc;
+  if (p->cluster_used_host != nullptr) *p->cluster_used_host = R;
+  if (debug) {
+    unsigned long long h[16];
+    cudaStreamSynchronize(st);
+    cudaMemcpy(h, dbg_buf, sizeof(h), cudaMemcpyDeviceToHost);
+    static const char* nm[12] = {"A chunks", "A sums", "A fence+barrier", "B chunks", "B sums", "B fence+barrier",
+                                 "C chunks", "C sums", "C fence+barrier", "D chunks", "D sums", "D fence+barrier"};
+    for (int i = 0; i < 12; ++i) fprintf(stderr, "ar_code[R=%d] %-16s %8.3f ms\n", R, nm[i], h[i] * 1e-6);
   }
-  for (;;) {
-    cudaError_t e = cudaSuccess;
-    if (R > 8) e = cudaFuncSetAttribute(ar_code_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    if (e == cudaSuccess) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3((unsigned)(p->N * R));
-      cfg.blockDim = dim3(AR_THREADS);
-      cfg.dynamicSmemBytes = AR_SMEM;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = (unsigned)R;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      e = cudaLaunchKernelEx(&cfg, ar_code_kernel, d);
-    }
-    if (e == cudaSuccess) {
-      if (p->cluster_used_host != nullptr) *p->cluster_used_host = R;
-      if (debug) {
-        unsigned long long h[16];
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h, dbg_buf, sizeof(h), cudaMemcpyDeviceToHost);
-        static const char* nm[12] = {"A chunks", "A sums", "A fence+barrier", "B chunks", "B sums", "B fence+barrier",
-                                     "C chunks", "C sums", "C fence+barrier", "D chunks", "D sums", "D fence+barrier"};
-        for (int i = 0; i < 12; ++i) fprintf(stderr, "ar_code[R=%d] %-16s %8.3f ms\n", R, nm[i], h[i] * 1e-6);
-      }
-      return TDVC_OK;
-    }
-    (void)cudaGetLastError();
-    if (auto_r && R == 16) { R = 8; continue; }
-    set_error("ar_code: launch with clusters of %d CTAs failed: %s", R, cudaGetErrorString(e));
-    return TDVC_ECUDA;
-  }
+  return TDVC_OK;
 }
 
 // compressai `pmf_to_quantized_cdf` (C++ in its `_CXX` module, always on the host): cdf has n + 1 entries.
@@ -487,12 +441,12 @@ extern "C" int64_t tdvc_rans_encode_with_indexes(const int32_t* symbols, const i
     if (value == max_value) {
       int32_t n_bypass = 0;
       while ((raw >> (n_bypass * RANS_BYPASS)) != 0) ++n_bypass;
-      int32_t val = n_bypass;
+      uint32_t val = (uint32_t)n_bypass;
       while (val >= RANS_MAX_BYPASS) {
-        syms.push_back({(uint32_t)RANS_MAX_BYPASS, 0u});
+        syms.push_back({RANS_MAX_BYPASS, 0u});
         val -= RANS_MAX_BYPASS;
       }
-      syms.push_back({(uint32_t)val, 0u});
+      syms.push_back({val, 0u});
       for (int32_t j = 0; j < n_bypass; ++j) syms.push_back({(uint32_t)((raw >> (j * RANS_BYPASS)) & RANS_MAX_BYPASS), 0u});
     }
   }
@@ -540,7 +494,7 @@ extern "C" int tdvc_rans_decode_with_indexes(const uint8_t* data, int64_t nbytes
     return true;
   };
   auto bits = [&](uint32_t& v) -> bool {
-    v = (uint32_t)(x & ((1u << RANS_BYPASS) - 1));
+    v = (uint32_t)(x & RANS_MAX_BYPASS);
     x >>= RANS_BYPASS;
     return renorm();
   };
@@ -558,26 +512,8 @@ extern "C" int tdvc_rans_decode_with_indexes(const uint8_t* data, int64_t nbytes
     const uint32_t start = (uint32_t)cdf[s], freq = (uint32_t)(cdf[s + 1] - cdf[s]);
     x = (uint64_t)freq * (x >> RANS_PRECISION) + (x & mask) - start;
     TDVC_REQUIRE(renorm(), "rans_decode: stream ends at symbol %lld", (long long)i);
-    int64_t value = s;
-    if (s == max_value) {
-      uint32_t val;
-      TDVC_REQUIRE(bits(val), "rans_decode: stream ends at symbol %lld", (long long)i);
-      int32_t n_bypass = (int32_t)val;
-      while (val == (uint32_t)RANS_MAX_BYPASS) {
-        TDVC_REQUIRE(bits(val), "rans_decode: stream ends at symbol %lld", (long long)i);
-        n_bypass += (int32_t)val;
-      }
-      TDVC_REQUIRE(n_bypass <= 16, "rans_decode: corrupt bypass code at symbol %lld", (long long)i);
-      uint64_t raw = 0;
-      for (int32_t j = 0; j < n_bypass; ++j) {
-        TDVC_REQUIRE(bits(val), "rans_decode: stream ends at symbol %lld", (long long)i);
-        raw |= (uint64_t)val << (j * RANS_BYPASS);
-      }
-      value = (int64_t)(raw >> 1);
-      if (raw & 1) value = -value - 1;
-      else value += max_value;
-    }
-    symbols[i] = (int32_t)(value + offsets[ci]);
+    TDVC_REQUIRE(rans_symbol(s, max_value, offsets[ci], bits, symbols[i]),
+                 "rans_decode: truncated or corrupt bypass code at symbol %lld", (long long)i);
   }
   return TDVC_OK;
 }

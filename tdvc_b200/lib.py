@@ -41,24 +41,22 @@ class DcnParams(C.Structure):
                 ("params_planar", C.c_int32)]
 
 
-class ArParams(C.Structure):
-    _fields_ = [("y", c_fp), ("y_ld", C.c_int32), ("params", c_fp), ("params_ld", C.c_int32),
-                ("w_ctx", c_fp), ("b_ctx", c_fp), ("w1", c_fp), ("b1", c_fp), ("c1", C.c_int32), ("c1_pad", C.c_int32),
-                ("w2", c_fp), ("b2", c_fp), ("c2", C.c_int32), ("c2_pad", C.c_int32), ("w3", c_fp), ("b3", c_fp),
-                ("scale_table", c_fp), ("n_scales", C.c_int32), ("y_hat", c_fp), ("symbols", c_fp), ("indexes", c_fp),
-                ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32), ("cluster", C.c_int32),
-                ("cluster_used_host", c_fp)]
-
-
-class ArDecodeParams(C.Structure):
+class ArChain(C.Structure):
     _fields_ = [("params", c_fp), ("params_ld", C.c_int32),
                 ("w_ctx", c_fp), ("b_ctx", c_fp), ("w1", c_fp), ("b1", c_fp), ("c1", C.c_int32), ("c1_pad", C.c_int32),
                 ("w2", c_fp), ("b2", c_fp), ("c2", C.c_int32), ("c2_pad", C.c_int32), ("w3", c_fp), ("b3", c_fp),
-                ("scale_table", c_fp), ("n_scales", C.c_int32), ("words", c_fp), ("word_offsets", c_fp),
+                ("scale_table", c_fp), ("n_scales", C.c_int32), ("y_hat", c_fp), ("symbols", c_fp), ("indexes", c_fp),
+                ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32)]
+
+
+class ArParams(C.Structure):
+    _fields_ = [("chain", ArChain), ("y", c_fp), ("y_ld", C.c_int32), ("cluster", C.c_int32), ("cluster_used_host", c_fp)]
+
+
+class ArDecodeParams(C.Structure):
+    _fields_ = [("chain", ArChain), ("words", c_fp), ("word_offsets", c_fp),
                 ("cdfs", c_fp), ("cdf_stride", C.c_int32), ("cdf_lengths", c_fp), ("cdf_offsets", c_fp),
-                ("n_tables", C.c_int32), ("cdf_total", C.c_int32),
-                ("y_hat", c_fp), ("symbols", c_fp), ("indexes", c_fp), ("status", c_fp),
-                ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32), ("cluster", C.c_int32)]
+                ("n_tables", C.c_int32), ("cdf_total", C.c_int32), ("status", c_fp), ("cluster", C.c_int32)]
 
 
 i32, i64, f32, vp, sz = C.c_int32, C.c_int64, C.c_float, C.c_void_p, C.c_size_t

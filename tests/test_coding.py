@@ -91,6 +91,24 @@ def test_host_rans_rejects_bad_input(oracle_model):
         coding.rans_decode(good[:8], np.full(100, 20, np.int32), tabs)                 # truncated stream
 
 
+def test_host_rans_rejects_an_escape_outside_int32(oracle_model, monkeypatch):
+    """An escape of 16 bypass digits 0xF folds to a value near 2^63: the encoder never writes one, and the host decoder
+    must raise on it (as the device decoder stops on it) instead of returning a wrapped symbol."""
+    from oracle import rans
+    from tdvc_b200 import coding
+    gc = _gc_tables(oracle_model)
+    tabs = _as_tables(gc)
+    cdf, lens, offs = gc._tables()
+    t = 20
+    mv = lens[t] - 2
+    esc = [(cdf[t][mv], cdf[t][mv + 1] - cdf[t][mv], False)]
+    digits = [(15, 16, True), (1, 2, True)] + [(15, 16, True)] * 16   # digit count 15 + 1, then 16 digits 0xF
+    monkeypatch.setattr(rans, "_rans_symbols", lambda *a: esc + digits)
+    data = rans.encode_with_indexes([0], [t], cdf, lens, offs)
+    with pytest.raises(RuntimeError):
+        coding.rans_decode(data, np.array([t], np.int32), tabs)
+
+
 def test_oracle_compress_round_trip(oracle_model):
     """compress -> decompress restores y_hat exactly and the strings are as long as the tables say (oracle only)."""
     from oracle import rans

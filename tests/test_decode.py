@@ -11,8 +11,6 @@ import numpy as np
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
 
 @pytest.fixture(scope="module")
 def oracle_model(oracle_model):
@@ -22,18 +20,6 @@ def oracle_model(oracle_model):
 
 
 # ------------------------------------------------------------------------------------------------------ CPU
-def test_decode_params_layout_matches_header():
-    import ctypes
-    import tempfile
-    from tdvc_b200 import lib as L
-    src = '#include <stdio.h>\n#include "tdvc_b200.h"\nint main(){printf("%zu\\n", sizeof(TdvcArDecodeParams));return 0;}\n'
-    with tempfile.TemporaryDirectory() as d:
-        open(os.path.join(d, "s.c"), "w").write(src)
-        subprocess.check_call(["gcc", "-I", os.path.join(ROOT, "include"), os.path.join(d, "s.c"), "-o", os.path.join(d, "s")])
-        size = int(subprocess.check_output([os.path.join(d, "s")]))
-    assert size == ctypes.sizeof(L.ArDecodeParams)
-
-
 def test_decode_refuses_malformed_strings_on_the_host():
     """Strings that cannot be rANS output (not whole 32-bit words, shorter than the 8-byte final state), a string count that
     does not match the batch and an unknown encoder cluster size are refused before anything reaches the device."""

@@ -32,17 +32,23 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_struct_layouts_match_header():
-    """ctypes mirrors of the parameter structs must have the C sizes (checked against a tiny C program)."""
+    """ctypes mirrors of the parameter structs must have the C sizes, and the chain the encoder and the decoder of y share
+    must sit at offset 0 of both (checked against a tiny C program)."""
     import ctypes
     import subprocess
     import tempfile
     from tdvc_b200 import lib as L
-    src = '#include <stdio.h>\n#include "tdvc_b200.h"\nint main(){printf("%zu %zu %zu\\n", sizeof(TdvcConvParams), sizeof(TdvcDcnParams), sizeof(TdvcArParams));return 0;}\n'
+    structs = {"TdvcConvParams": L.ConvParams, "TdvcDcnParams": L.DcnParams, "TdvcArChain": L.ArChain,
+               "TdvcArParams": L.ArParams, "TdvcArDecodeParams": L.ArDecodeParams}
+    prints = "".join(f'printf("%zu\\n", sizeof({s}));' for s in structs)
+    prints += 'printf("%zu\\n%zu\\n", offsetof(TdvcArParams, chain), offsetof(TdvcArDecodeParams, chain));'
+    src = f'#include <stddef.h>\n#include <stdio.h>\n#include "tdvc_b200.h"\nint main(){{{prints}return 0;}}\n'
     with tempfile.TemporaryDirectory() as d:
         open(os.path.join(d, "s.c"), "w").write(src)
         subprocess.check_call(["gcc", "-I", os.path.join(ROOT, "include"), os.path.join(d, "s.c"), "-o", os.path.join(d, "s")])
-        a, b, c = subprocess.check_output([os.path.join(d, "s")]).split()
-    assert int(a) == ctypes.sizeof(L.ConvParams) and int(b) == ctypes.sizeof(L.DcnParams) and int(c) == ctypes.sizeof(L.ArParams)
+        got = [int(v) for v in subprocess.check_output([os.path.join(d, "s")]).split()]
+    assert got == [ctypes.sizeof(t) for t in structs.values()] + [0, 0]
+    assert L.ArParams.chain.offset == 0 and L.ArDecodeParams.chain.offset == 0
 
 
 def test_state_dict_matches_reference_key_set(oracle_model):

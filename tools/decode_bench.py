@@ -1,7 +1,10 @@
 """Time the device decoder of the y latent (`tdvc_ar_decode`) against the encoder (`tdvc_ar_code`) on a 1920x1024 P-frame
-(64x120 latent, 7,680 dependent decode steps per coder), both coders, strings coded with 16 CTAs per image.
+(64x120 latent, 7,680 dependent decode steps per coder), both coders.  The encoder's cluster size is 16 CTAs per image by
+default; 8, or 0 (16 where that launches, else 8), time the other variants, and the decoder reproduces whichever ran.
 CUDA events around each launch after warm-up; the GPU's name and power limit are read in the same run.
-python tools/decode_bench.py [reps]  ->  one JSON line."""
+TDVC_B200_AR_DEBUG=1 adds the encoder's per-phase times on stderr.
+python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}]  ->  one JSON line."""
+import argparse
 import json
 import subprocess
 import sys
@@ -29,7 +32,11 @@ def timed(fn):
 
 
 def main():
-    reps = int(sys.argv[1]) if len(sys.argv) > 1 else 5
+    ap = argparse.ArgumentParser()
+    ap.add_argument("reps", nargs="?", type=int, default=5)
+    ap.add_argument("--encoder-cluster", type=int, choices=(0, 8, 16), default=16)
+    args = ap.parse_args()
+    reps, cl = args.reps, args.encoder_cluster
     dev = torch.device("cuda:0")
     orc = build_oracle()
     net = VideoCompressor().eval()
@@ -41,15 +48,16 @@ def main():
     W = net._weights(dev)
     plan = net._plan(1, 1024, 1920, dev)
     hy, wy = 64, 120
-    res = {"gpu": gpu_info(), "frame": "1920x1024", "latent": [hy, wy], "encoder_cluster": 16}
+    res = {"gpu": gpu_info(), "frame": "1920x1024", "latent": [hy, wy], "encoder_cluster": cl}
     for cn in ("mv", "rs"):
         tabs = W["_tables"][cn]
         params = plan.buf(f"{cn}.params", 1, hy, wy, 256)
         enc_ms, dec_ms = [], []
         for rep in range(reps + 1):   # rep 0: warm-up
-            t_enc, h = timed(lambda: coding.launch_coding(plan, W, cn, tabs, cluster=16))
+            t_enc, h = timed(lambda: coding.launch_coding(plan, W, cn, tabs, cluster=cl))
             enc = coding.finish_coding(h, keep=True)
-            t_dec, h = timed(lambda: coding.launch_decoding(W, cn, tabs, enc["strings"][0], params, 16))
+            res["encoder_cluster_used"] = enc["cluster"]
+            t_dec, h = timed(lambda: coding.launch_decoding(W, cn, tabs, enc["strings"][0], params, enc["cluster"]))
             dec = coding.finish_decoding(h)
             assert torch.equal(dec["y_hat"], enc["y_hat"]) and torch.equal(dec["y_symbols"], enc["y_symbols"])
             if rep:
