@@ -148,7 +148,8 @@ def test_ar_decode_is_lossless(oracle_model, hw, seed, n):
 
 @pytest.mark.gpu
 def test_ar_decode_is_lossless_full_size(oracle_model):
-    """1920x1024: a 64x120 latent, 7,680 dependent decode steps per coder, wavefront chunks of every length 1..40."""
+    """1920x1024: a 64x120 latent, 7,680 dependent decode steps per coder, wavefronts of 1..40 positions, each coded as
+    one chunk (waves of two and three chunks: tests/test_ar_edges.py)."""
     dev = torch.device("cuda:0")
     net = _net(oracle_model, dev)
     W, plan = _frame(net, 1, (1024, 1920), 0, dev)
