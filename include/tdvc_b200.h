@@ -309,6 +309,8 @@ int tdvc_chan_dot(const float* a, const float* b_or_null, float* out, int N, int
  *   tail mass) -> n + 1 cumulative 16-bit counts; empty bins steal from the smallest bin above 1.
  * Symbols (`compress`):
  *   eb_symbols: z NHWC -> symbols round(z - median) and table indexes (= channel) in NCHW order.
+ *   eb_dequantize (decoder side): the inverse, symbols in NCHW order -> z_hat NHWC (row stride ld >= C) = symbol + median,
+ *     the same fp32 addition as eb_bits' z_hat, so the decoder's z_hat is bit-identical to the encoder's.
  *   TdvcArChain: the autoregressive chain of compressai's y coding, which ar_code and ar_decode must compute identically.
  *     All pointers are DEVICE pointers.  `params`: the hyper-decoder output, NHWC rows of params_ld >= 2C floats.  Weights
  *     in the fp32 layout of tdvc_conv2d ([tap][cin_pad][cout_pad]): w_ctx the masked 5x5 context model (C -> 2C), w1 / w2
@@ -366,6 +368,7 @@ typedef struct TdvcArDecodeParams {
 int tdvc_pmf_to_quantized_cdf(const float* pmf, int n, int precision, int32_t* cdf);
 int tdvc_eb_symbols(const float* z, int ld, const float* medians, int N, int HW, int C, int32_t* symbols, int32_t* indexes,
                     void* stream);
+int tdvc_eb_dequantize(const int32_t* symbols, const float* medians, int N, int HW, int C, float* z_hat, int ld, void* stream);
 size_t tdvc_ar_code_workspace_bytes(int N, int c1_pad, int c2_pad);
 int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t workspace_bytes, void* stream);
 int tdvc_ar_decode(const TdvcArDecodeParams* p, void* stream);

@@ -18,6 +18,9 @@ What runs where:
   pass left in the plan; rANS over the symbols on the host (`tdvc_rans_encode_with_indexes`), as in compressai.
 * `decode_latents`: y strings back to symbols and y_hat on the device (`tdvc_ar_decode`, csrc/ar_decode.cu), bit-identical
   to what `tdvc_ar_code` produced when told the encoder's cluster size.
+* `decode_z_symbols` / `dequantize_z`: z strings back to symbols on the host (rANS, as in compressai) and z_hat = symbol +
+  median on the device (`tdvc_eb_dequantize`); `VideoCompressor.decompress_latents` runs h_s on it to get the `params`
+  decode_latents needs, so that a container alone decodes.
 """
 import ctypes as C
 import math
@@ -332,6 +335,38 @@ def finish_decoding(h):
 
 def decode_latents(W, cn, tables, y_strings, params, cluster, stream=None):
     return finish_decoding(launch_decoding(W, cn, tables, y_strings, params, cluster, stream=stream))
+
+
+def eb_indexes(hz, wz, C=128):
+    """compressai `EntropyBottleneck._build_indexes` of one image: the table index of every z symbol, in coding (CHW) order,
+    is its channel."""
+    return np.repeat(np.arange(C, dtype=np.int32), hz * wz)
+
+
+def decode_z_symbols(cn, z_strings, tables, hz, wz, C=128):
+    """Host half of compressai `EntropyBottleneck.decompress` for coder `cn` ("mv" | "rs"): one z string per image ->
+    int32 symbols (N, C, hz, wz), the NCHW order they were coded in.  A string that does not decode raises RuntimeError
+    naming the coder and the image (rANS cannot detect every corruption: a garbled string may decode to other symbols)."""
+    idx = eb_indexes(hz, wz, C)
+    out = np.empty((len(z_strings), C, hz, wz), dtype=np.int32)
+    for i, s_ in enumerate(z_strings):
+        try:
+            out[i] = rans_decode(s_, idx, tables.eb).reshape(C, hz, wz)
+        except RuntimeError as e:
+            raise RuntimeError(f"decompress_latents: the {cn} z string of image {i} is truncated or corrupt ({e})") from None
+    return out
+
+
+def dequantize_z(symbols, medians, z_hat, stream=None):
+    """compressai `dequantize`: z_hat = symbol + median (`tdvc_eb_dequantize`).  symbols: int32 CUDA tensor (N, C, hz, wz);
+    medians: the coder's fp32 medians (W[f"{cn}.eb"][3]); z_hat: a channels-last Act (N, hz, wz, C), bit-identical to the
+    z_hat the encoder's forward pass computed from the same symbols."""
+    N, Cc, hz, wz = symbols.shape
+    if (z_hat.N, z_hat.H, z_hat.W, z_hat.C) != (N, hz, wz, Cc) or symbols.dtype != torch.int32 or not symbols.is_contiguous():
+        raise RuntimeError("dequantize_z: symbols and z_hat do not match")
+    stream = stream or torch.cuda.current_stream(symbols.device)
+    L.check(L.load().tdvc_eb_dequantize(symbols.data_ptr(), medians.data_ptr(), N, hz * wz, Cc, z_hat.ptr, z_hat.ld,
+                                        stream.cuda_stream), "eb_dequantize")
 
 
 # ----------------------------------------------------------------------------------------------- bitstream container

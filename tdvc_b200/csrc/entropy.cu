@@ -230,6 +230,24 @@ __global__ void eb_symbols_kernel(const float* __restrict__ z, int ld, const flo
   }
 }
 
+// eb_dequantize: the decoder's inverse of eb_symbols (compressai EntropyBottleneck.decompress -> dequantize): int32 symbols in
+// NCHW order -> z_hat NHWC = symbol + median.  eb_bits_kernel writes the encoder's z_hat as __fadd_rn(rintf(z - med), med);
+// rintf(z - med) is the float of the symbol, so this is the same fp32 addition on the same operands, bit for bit.
+// One thread per output element in NHWC order: the writes are coalesced, the reads stride by HW (z is H/64 x W/64, small).
+__global__ void eb_dequantize_kernel(const int32_t* __restrict__ symbols, const float* __restrict__ medians, int N, int HW,
+                                     int C, float* __restrict__ z_hat, int ld) {
+  const int64_t total = (int64_t)N * HW * C;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    const int c = (int)(i % C);
+    const int64_t np = i / C;   // n * HW + p
+    const int p = (int)(np % HW);
+    const int n = (int)(np / HW);
+    const int32_t s = __ldg(symbols + ((int64_t)n * C + c) * HW + p);
+    z_hat[np * ld + c] = __fadd_rn((float)s, __ldg(medians + c));
+  }
+}
+
 // ---- backward of the two likelihood-to-bits reductions in training (noise) mode (SURVEY.md 8f row 1; the reference takes these
 // gradients from autograd through compressai's entropy models, tools/train.py:132-145).  S = sum ln max(p, 1e-9); `gS` is
 // d loss / d S (device scalar).  compressai's LowerBound passes a gradient where the input is above the bound OR the gradient
@@ -482,6 +500,16 @@ extern "C" int tdvc_eb_symbols(const float* z, int ld, const float* medians, int
   if (grid > kNumSMs * 8) grid = kNumSMs * 8;
   eb_symbols_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(z, ld, medians, N, HW, C, symbols, indexes);
   TDVC_CHECK_LAUNCH("eb_symbols");
+  return TDVC_OK;
+}
+
+extern "C" int tdvc_eb_dequantize(const int32_t* symbols, const float* medians, int N, int HW, int C, float* z_hat, int ld,
+                                  void* stream) {
+  TDVC_REQUIRE(symbols && medians && z_hat && N > 0 && HW > 0 && C > 0 && ld >= C, "eb_dequantize: bad args");
+  int grid = cdiv((int64_t)N * HW * C, 256);
+  if (grid > kNumSMs * 8) grid = kNumSMs * 8;
+  eb_dequantize_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(symbols, medians, N, HW, C, z_hat, ld);
+  TDVC_CHECK_LAUNCH("eb_dequantize");
   return TDVC_OK;
 }
 

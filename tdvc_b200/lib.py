@@ -115,6 +115,7 @@ SIGNATURES = {
     "tdvc_chan_dot": [vp, vp, vp, i32, i64, i32, f32, vp, sz, vp],
     "tdvc_pmf_to_quantized_cdf": [vp, i32, i32, vp],
     "tdvc_eb_symbols": [vp, i32, vp, i32, i32, i32, vp, vp, vp],
+    "tdvc_eb_dequantize": [vp, vp, i32, i32, i32, vp, i32, vp],
     "tdvc_ar_code_workspace_bytes": [i32, i32, i32],
     "tdvc_ar_code": [C.POINTER(ArParams), vp, sz, vp],
     "tdvc_ar_decode": [C.POINTER(ArDecodeParams), vp],

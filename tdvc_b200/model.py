@@ -920,12 +920,7 @@ class _Plan:
         else:
             self.call("tdvc_eb_bits", z.ptr, zh.ptr, mats.data_ptr(), biases.data_ptr(), factors.data_ptr(), med.data_ptr(),
                       z.N * z.H * z.W, 128, self.acc.data_ptr() + 8 * (acc_off + 1))
-        # ---- h_s
-        s = self.conv([zh], W[f"{cn}.hs0"], b("hs0", z.H, z.W), **lr)
-        s = self.conv([s], W[f"{cn}.hs2"], b("hs2", 2 * z.H, 2 * z.W), **lr)
-        s = self.conv([s], W[f"{cn}.hs4"], b("hs4", s.H, s.W, 192), **lr)
-        s = self.conv([s], W[f"{cn}.hs6"], b("hs6", 2 * s.H, 2 * s.W, 192), **lr)
-        params = self.conv([s], W[f"{cn}.hs8"], b("params", s.H, s.W, 256))
+        params = self.hyper_synthesis(W, cn, zh, b)
         # ---- context model, entropy parameters, conditional likelihood
         ctx = self.conv([yh], W[f"{cn}.ctx"], b("ctx", y.H, y.W, 256))
         c0, c2 = W[f"{cn}.ep0"].cout, W[f"{cn}.ep2"].cout
@@ -939,6 +934,17 @@ class _Plan:
             self.call("tdvc_gc_bits", y.ptr, gp.ptr, gp.ld, y.N * y.H * y.W, 128, self.acc.data_ptr() + 8 * acc_off,
                       nbytes=12 * y.N * y.H * y.W * 128)
         return gp, z, zh
+
+    def hyper_synthesis(self, W, cn, zh, b):
+        """h_s of coder `cn`: z_hat (N, H/64, W/64, 128) -> params (N, H/16, W/16, 256), the scales and means the entropy
+        parameters start from.  The one h_s of both ends: the encoder runs it on its quantised z (`_hyper_path`), the decoder
+        (`VideoCompressor.decompress_latents`) on the z_hat it decoded.  b(name, h, w, c=128, **kw) allocates the buffers."""
+        lr = dict(act=L.ACT_LRELU, slope=0.01)
+        s = self.conv([zh], W[f"{cn}.hs0"], b("hs0", zh.H, zh.W), **lr)
+        s = self.conv([s], W[f"{cn}.hs2"], b("hs2", 2 * zh.H, 2 * zh.W), **lr)
+        s = self.conv([s], W[f"{cn}.hs4"], b("hs4", s.H, s.W, 192), **lr)
+        s = self.conv([s], W[f"{cn}.hs6"], b("hs6", 2 * s.H, 2 * s.W, 192), **lr)
+        return self.conv([s], W[f"{cn}.hs8"], b("params", s.H, s.W, 256))
 
     # ---------------------------------------------------------------- cache keys and the variant of a frame
     def _variant(self, refs, cache, ref_keys=None):
@@ -1486,20 +1492,13 @@ class VideoCompressor(nn.Module):
         out, pending = {}, []
         main = torch.cuda.current_stream(plan.dev)
         side = plan._side_stream()
-        tabs = Wt.setdefault("_tables", {})
         for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
-            if cn not in tabs:   # update(force=True) recomputes the same tables from the same parameters: once per pack
-                tabs[cn] = coding.CoderTables(Wt, cn, plan.dev)
-                src = self._source()
-                smod = src.mvCoder if cn == "mv" else src.resCoder
-                for m, t in ((smod.entropy_bottleneck, tabs[cn].eb), (smod.gaussian_conditional, tabs[cn].gc)):
-                    m._quantized_cdf, m._cdf_length, m._offset = t.tensors(plan.dev)   # compressai's buffers, as update() leaves them
-                smod.gaussian_conditional.scale_table = tabs[cn].scale_table.clone()
+            tabs = self._coder_tables(Wt, cn, plan.dev)
             # the two coders' autoregressive passes (one 8-16 SM cluster per image each) run side by side on two streams;
             # the host codes the motion strings while the residual pass is still running
             if stream is not main:
                 stream.wait_stream(main)
-            pending.append((nm, coding.launch_coding(plan, Wt, cn, tabs[cn], stream=stream)))
+            pending.append((nm, coding.launch_coding(plan, Wt, cn, tabs, stream=stream)))
         for nm, h in pending:
             enc = coding.finish_coding(h, keep=taps is not None)
             enc["ac_bpp"] = sum(len(s[0]) for s in enc["strings"]) * 8.0 / num_pixels
@@ -1508,6 +1507,89 @@ class VideoCompressor(nn.Module):
                     taps[f"{nm}.ac.{k}"] = enc.pop(k)
             out[nm] = enc
         main.wait_stream(side)
+        return out
+
+    def _coder_tables(self, Wt, cn, dev):
+        """`update(force=True)` of coder `cn` ("mv" | "rs"), shared by the encoder and the decoder: its coding tables
+        (coding.CoderTables) from the packed weights Wt, and compressai's buffers on the source module filled as update()
+        leaves them.  update() recomputes the same tables from the same parameters: built once per pack."""
+        from tdvc_b200 import coding
+        tabs = Wt.setdefault("_tables", {})
+        if cn not in tabs:
+            tabs[cn] = coding.CoderTables(Wt, cn, dev)
+            src = self._source()
+            smod = src.mvCoder if cn == "mv" else src.resCoder
+            for m, t in ((smod.entropy_bottleneck, tabs[cn].eb), (smod.gaussian_conditional, tabs[cn].gc)):
+                m._quantized_cdf, m._cdf_length, m._offset = t.tensors(dev)   # compressai's buffers, as update() leaves them
+            smod.gaussian_conditional.scale_table = tabs[cn].scale_table.clone()
+        return tabs[cn]
+
+    def decompress_latents(self, data):
+        """Both coders' latents of one P-frame from the bytes of a version-2 container (`coding.pack_frame(net.last_coded,
+        frame=...)`) and the weights alone: no reference frames and nothing the encoder left behind.  Per coder: the z strings
+        are rANS-decoded on the host (compressai `EntropyBottleneck.decompress`), z_hat = symbol + median on the device, h_s
+        (`_Plan.hyper_synthesis`, the encoder's own) gives the params, and `tdvc_ar_decode` decodes y with the cluster size the
+        container records.  The motion coder runs on the current stream, the residual coder on the plan's side stream.
+        Returns {"frame": {"size", "N", "precision"}, "mv" | "res": {"y_hat", "y_symbols", "y_indexes": (N, H/16, W/16, 128),
+        "z_hat": (N, H/64, W/64, 128)}}, channels-last tensors of their own.
+        The result is bit-identical to the encoder's latents only with the same kernels on sm_100a and the same `conv_impl`
+        as the encoder ran with: h_s feeds every predicted mean and scale, and the container does not record conv_impl.
+        A malformed container raises RuntimeError before any device work; a broken z string raises naming the coder and
+        the image, a broken y string naming the latent position."""
+        from tdvc_b200 import coding
+        box = coding.unpack_frame(data)
+        frame = box.get("frame")
+        if frame is None:
+            raise RuntimeError("decompress_latents: a version-1 container records no cluster sizes, so its y strings cannot "
+                               "be decoded exactly (write version 2: pack_frame(..., frame=...))")
+        (H, Wd), N = frame["size"], frame["N"]
+        if N < 1 or H < 64 or Wd < 64 or H % 64 or Wd % 64:
+            raise RuntimeError(f"decompress_latents: frame {H}x{Wd}, N={N} (H and W multiples of 64, N >= 1)")
+        for nm in ("mv", "res"):
+            enc = box.get(nm)
+            if enc is None:
+                raise RuntimeError(f"decompress_latents: the container has no {nm} coder")
+            if tuple(enc["shape"]) != (H // 64, Wd // 64):
+                raise RuntimeError(f"decompress_latents: {nm} hyper-latent shape {tuple(enc['shape'])} for a {H}x{Wd} "
+                                   f"frame (expected {(H // 64, Wd // 64)})")
+            if len(enc["strings"]) != 2 or any(len(lst) != N for lst in enc["strings"]):
+                raise RuntimeError(f"decompress_latents: {nm} has {[len(lst) for lst in enc['strings']]} strings (two "
+                                   f"lists, y and z, of {N})")
+        dev = self.mvCoder.entropy_bottleneck.quantiles.device
+        if dev.type != "cuda":
+            raise RuntimeError("tdvc_b200.VideoCompressor runs on CUDA (sm_100a) only; there is no CPU fallback")
+        hz, wz = H // 64, Wd // 64
+        with torch.cuda.device(dev), torch.no_grad():
+            Wt = self._weights(dev)
+            plan = self._plan(N, H, Wd, dev)
+            plan.bind(Wt)
+            # h_s is fp32-class in both precision modes (only rs.g_s* and lf.* take one-product weights), so the container's
+            # `precision` does not affect the latents and plan.precision is left as the last forward set it
+            plan.impl = self.conv_impl
+            main = torch.cuda.current_stream(dev)
+            side = plan._side_stream()
+            side.wait_stream(main)
+            pending = []
+            for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
+                tabs = self._coder_tables(Wt, cn, dev)
+                enc = box[nm]
+                z_sym = coding.decode_z_symbols(cn, enc["strings"][1], tabs, hz, wz)
+                # every buffer under dec.{cn}.*: the forward pass and launch_coding never read what the decoder writes
+                b = lambda nme, h, w, c=128, cn=cn, **kw: plan.buf(f"dec.{cn}.{nme}", N, h, w, c, **kw)
+                with torch.cuda.stream(stream):
+                    sym_d = torch.from_numpy(z_sym).to(dev)
+                    zh = b("z_hat", hz, wz)
+                    coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
+                    params = plan.hyper_synthesis(Wt, cn, zh, b)
+                # the motion chain is already decoding on the device while the host decodes the residual z strings
+                h = coding.launch_decoding(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream)
+                pending.append((nm, zh, h))
+            main.wait_stream(side)
+            out = {"frame": dict(frame)}
+            for nm, zh, h in pending:
+                y = coding.finish_decoding(h)
+                out[nm] = {k: v.clone() for k, v in y.items()}
+                out[nm]["z_hat"] = zh.t.clone()
         return out
 
     def _forward_training(self, input_image, refer_frames, taps=None, noise=None):

@@ -3,11 +3,16 @@
 default; 8, or 0 (16 where that launches, else 8), time the other variants, and the decoder reproduces whichever ran.
 CUDA events around each launch after warm-up; the GPU's name and power limit are read in the same run.
 TDVC_B200_AR_DEBUG=1 adds the encoder's per-phase times on stderr.
-python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}]  ->  one JSON line."""
+--container: also time `VideoCompressor.decompress_latents` end to end (host clock around the call, which returns only
+once both coders' latents are on the device) on the version-2 container of the frame `forward(is_compress=True)` coded,
+decoded by a second module loaded from the same weights; the per-coder `tdvc_ar_decode` times of the same run stand beside
+it, so the overlap of the two coders' chains can be read off.
+python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}] [--container]  ->  one JSON line."""
 import argparse
 import json
 import subprocess
 import sys
+import time
 
 import torch
 
@@ -35,6 +40,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("reps", nargs="?", type=int, default=5)
     ap.add_argument("--encoder-cluster", type=int, choices=(0, 8, 16), default=16)
+    ap.add_argument("--container", action="store_true", help="also time decompress_latents on the frame's container")
     args = ap.parse_args()
     reps, cl = args.reps, args.encoder_cluster
     dev = torch.device("cuda:0")
@@ -43,12 +49,32 @@ def main():
     net.load_state_dict(orc.state_dict())
     net = net.to(dev)
     x, refs = synth.make_frame_pair(1024, 1920, seed=0)
+    gt = {}
     with torch.no_grad():
-        net(x.to(dev), refs.to(dev), False, is_compress=True)
+        net(x.to(dev), refs.to(dev), False, is_compress=True, taps=gt)
+    blob = coding.pack_frame(net.last_coded, frame={"size": (1024, 1920), "N": 1, "precision": "exact"})
     W = net._weights(dev)
     plan = net._plan(1, 1024, 1920, dev)
     hy, wy = 64, 120
     res = {"gpu": gpu_info(), "frame": "1920x1024", "latent": [hy, wy], "encoder_cluster": cl}
+    if args.container:
+        # before the loop below recodes the plan's latents: the container holds forward()'s strings (automatic cluster)
+        dec = VideoCompressor().eval()
+        dec.load_state_dict(orc.state_dict())
+        dec = dec.to(dev)
+        ms = []
+        for rep in range(reps + 1):   # rep 0: warm-up (packs the weights, builds the tables and the decoder's plan)
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            out = dec.decompress_latents(blob)
+            ms.append(1e3 * (time.perf_counter() - t0))
+            for nm in ("mv", "res"):
+                assert torch.equal(out[nm]["y_hat"], gt[f"{nm}.ac.y_hat"]), nm
+                assert torch.equal(out[nm]["z_hat"], gt[f"{nm}.z_hat"].permute(0, 2, 3, 1)), nm
+        ms = ms[1:]
+        res["container"] = {"bytes": len(blob), "clusters": [net.last_coded[nm]["cluster"] for nm in ("mv", "res")],
+                            "decompress_latents_ms": round(sorted(ms)[len(ms) // 2], 3),
+                            "decompress_latents_ms_all": [round(t, 3) for t in ms]}
     for cn in ("mv", "rs"):
         tabs = W["_tables"][cn]
         params = plan.buf(f"{cn}.params", 1, hy, wy, 256)
