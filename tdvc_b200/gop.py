@@ -117,6 +117,36 @@ def code_gop(net, i_frame, p_frames, enable_amp=False, keep_recon=False, with_ms
     return out
 
 
+def compress_gop(net, i_frame, p_frames, enable_amp=False):
+    """Closed-loop coding of one GOP with `VideoCompressor.compress`: each frame's reconstruction - the frame the decoder
+    rebuilds - is the next frame's reference, so encoder and decoder never drift apart.  i_frame (1,3,h,w): the (decoded)
+    I-frame; p_frames (T,3,h,w).  Frames are padded to multiples of 64 and cropped back as in `code_gop`.
+    Returns (containers: one version-2 container (bytes) per P-frame, recon: the cropped reconstructions)."""
+    T, _, h, w = p_frames.shape
+    refs = RefBuffer(pad(i_frame, 64))
+    containers, recons = [], []
+    for i in range(T):
+        window, keys = refs.window()
+        recon, data = net.compress(pad(p_frames[i:i + 1], 64), window, enable_amp, ref_keys=keys)
+        refs.push(recon)
+        containers.append(data)
+        recons.append(crop(recon, (h, w)))
+    return containers, recons
+
+
+def decompress_gop(net, i_frame, containers, size):
+    """Decoder of `compress_gop`: the same I-frame (1,3,h,w), the containers in order and the frame size (h, w) ->
+    the cropped reconstructions, bit-identical to the encoder's."""
+    refs = RefBuffer(pad(i_frame, 64))
+    recons = []
+    for data in containers:
+        window, keys = refs.window()
+        recon = net.decompress(data, window, ref_keys=keys)
+        refs.push(recon)
+        recons.append(crop(recon, size))
+    return recons
+
+
 def validate(dataset, net, enable_amp=True, device=None, with_msssim=True, gops=None):
     """The reference's `validation` (reference tools/predict.py:35-110) over a `tdvc_b200.data.GopDataset`: every GOP is coded
     by `code_gop`; bpp / PSNR / MS-SSIM are averaged over ALL frames, the BPG-coded I-frame of each GOP included with the bpp /

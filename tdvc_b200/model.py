@@ -823,49 +823,7 @@ class _Plan:
 
     def coder(self, W, cn, x, acc_off, taps, final_res=None, out=None):
         """Cheng2020Anchor.forward with the reference's g_a / g_s (SURVEY App. A; encoder_v3.py:14-69)."""
-        N, H, Wd = x.N, x.H, x.W
-        lr = dict(act=L.ACT_LRELU, slope=0.01)
-        b = lambda nme, h, w, c=128, **kw: self.buf(f"{cn}.{nme}", N, h, w, c, **kw)
-
-        # GDN / IGDN: the layer that produces the GDN input also maintains max |t2| (one atomic per epilogue warp); the GDN
-        # kernel pre-scales x*x by a power of two from it so that the fp16 operands cannot saturate (csrc/conv_tc.cu)
-        def rb_stride(i, x, h, w):
-            am = self.absmax_ptr(f"{cn}.ga{i}")
-            idt = self.conv([x], W[f"{cn}.ga{i}.skip"], b(f"ga{i}.id", h, w), stride=2)
-            t = self.conv([x], W[f"{cn}.ga{i}.conv1"], b(f"ga{i}.t", h, w), stride=2, **lr)
-            t2 = self.conv([t], W[f"{cn}.ga{i}.conv2"], b(f"ga{i}.t2", h, w), absmax_out=am)
-            return self.conv([t2], W[f"{cn}.ga{i}.gdn"], b(f"ga{i}.o", h, w), in_square=True, post=L.POST_GDN,
-                             mul=t2, res1=idt, absmax_in=am, csum=(i == 2))
-
-        def rb(pfx, i, x):
-            t = self.conv([x], W[f"{cn}.{pfx}{i}.conv1"], b(f"{pfx}{i}.t", x.H, x.W), **lr)
-            return self.conv([t], W[f"{cn}.{pfx}{i}.conv2"], b(f"{pfx}{i}.o", x.H, x.W), res1=x, **lr)
-
-        def rb_up(i, x):
-            h, w = 2 * x.H, 2 * x.W
-            am = self.absmax_ptr(f"{cn}.gs{i}")
-            t = self.conv([x], W[f"{cn}.gs{i}.subpel"], b(f"gs{i}.t", h, w), **lr)
-            t2 = self.conv([t], W[f"{cn}.gs{i}.conv"], b(f"gs{i}.t2", h, w), absmax_out=am)
-            idt = self.conv([x], W[f"{cn}.gs{i}.upsample"], b(f"gs{i}.id", h, w))
-            return self.conv([t2], W[f"{cn}.gs{i}.igdn"], b(f"gs{i}.o", h, w), in_square=True, post=L.POST_IGDN,
-                             mul=t2, res1=idt, absmax_in=am, csum=(i == 4))
-
-        # ---- g_a
-        a = rb_stride(0, x, H // 2, Wd // 2)
-        a = rb("ga", 1, a)
-        a = rb_stride(2, a, H // 4, Wd // 4)
-        a = self.se(a, W[f"{cn}.ga3"], b("ga3.o", a.H, a.W), csum=self.last_csum)
-        a = rb("ga", 4, a)
-        a = rb_stride(5, a, H // 8, Wd // 8)
-        a = rb("ga", 6, a)
-        a = self.conv([a], W[f"{cn}.ga7"], b("ga7.o", H // 16, Wd // 16), stride=2, csum=True)
-        y = self.se(a, W[f"{cn}.ga8"], b("y", a.H, a.W), csum=self.last_csum)
-        # ---- y_hat first: both the synthesis transform and the entropy model start from it
-        yh = b("y_hat", y.H, y.W)
-        if self.training:   # compressai quantize(y, "noise"): y + U(-0.5, 0.5)   (JointAutoregressiveHierarchicalPriors.forward)
-            self.call("tdvc_axpby", y.ptr, self.noise[f"{cn}.y"].ptr, yh.ptr, y.N * y.H * y.W * 128, 1.0, 1.0)
-        else:
-            self.call("tdvc_round_half_even", y.ptr, yh.ptr, y.N * y.H * y.W * 128, nbytes=8 * y.N * y.H * y.W * 128)
+        y, yh = self.analysis(W, cn, x)
         # The hyperprior / context / entropy-parameter chain only feeds the bit count (x_hat depends on round(y) alone,
         # SURVEY.md App. A): ~17 small, latency-bound launches at H/16..H/64.  They run on a side stream, concurrently
         # with the (equally small) first layers of g_s, and are joined before this coder returns.  (Serialised when the
@@ -875,18 +833,8 @@ class _Plan:
         if side is not None:
             side.wait_stream(main)
         with torch.cuda.stream(side if side is not None else main):
-            gp, z, zh = self._hyper_path(W, cn, y, yh, acc_off, b, lr)
-        # ---- g_s
-        g = self.se(yh, W[f"{cn}.gs0"], b("gs0.o", y.H, y.W))
-        g = rb("gs", 1, g)
-        g = rb_up(2, g)
-        g = rb("gs", 3, g)
-        g = rb_up(4, g)
-        g = self.se(g, W[f"{cn}.gs5"], b("gs5.o", g.H, g.W), csum=self.last_csum)
-        g = rb("gs", 6, g)
-        g = rb_up(7, g)
-        g = rb("gs", 8, g)
-        xh = self.conv([g], W[f"{cn}.gs9"], out if out is not None else b("x_hat", H, Wd, 64), res1=final_res)
+            gp, z, zh = self._hyper_path(W, cn, y, yh, acc_off)
+        xh = self.synthesis(W, cn, yh, final_res=final_res, out=out)
         if side is not None:
             main.wait_stream(side)
         if taps is not None:
@@ -895,13 +843,89 @@ class _Plan:
                          f"{nm}.scales_hat": gp.chan(0, 128).nchw(), f"{nm}.means_hat": gp.chan(128, 128).nchw()})
         return xh
 
+    def _cbuf(self, cn, N):
+        """Buffer allocator of coder `cn`'s layers: b(name, h, w, c=128, **kw) -> plan buffer "{cn}.{name}"."""
+        return lambda nme, h, w, c=128, **kw: self.buf(f"{cn}.{nme}", N, h, w, c, **kw)
+
+    def analysis(self, W, cn, x):
+        """g_a of coder `cn` and the quantiser of the forward pass: x (N, H, W, 64) -> (y, y_hat) at H/16 x W/16, y_hat =
+        round(y) (eval) or y + U(-0.5, 0.5) (training).  Only the bit count and forward's reconstruction use this y_hat: a
+        decoder sees the autoregressive one (`launch_coding`'s `{cn}.ac.y_hat`), which `compress` synthesises from."""
+        N, H, Wd = x.N, x.H, x.W
+        lr = dict(act=L.ACT_LRELU, slope=0.01)
+        b = self._cbuf(cn, N)
+
+        # GDN: the layer that produces the GDN input also maintains max |t2| (one atomic per epilogue warp); the GDN
+        # kernel pre-scales x*x by a power of two from it so that the fp16 operands cannot saturate (csrc/conv_tc.cu)
+        def rb_stride(i, x, h, w):
+            am = self.absmax_ptr(f"{cn}.ga{i}")
+            idt = self.conv([x], W[f"{cn}.ga{i}.skip"], b(f"ga{i}.id", h, w), stride=2)
+            t = self.conv([x], W[f"{cn}.ga{i}.conv1"], b(f"ga{i}.t", h, w), stride=2, **lr)
+            t2 = self.conv([t], W[f"{cn}.ga{i}.conv2"], b(f"ga{i}.t2", h, w), absmax_out=am)
+            return self.conv([t2], W[f"{cn}.ga{i}.gdn"], b(f"ga{i}.o", h, w), in_square=True, post=L.POST_GDN,
+                             mul=t2, res1=idt, absmax_in=am, csum=(i == 2))
+
+        rb = self._rb(W, cn, b, lr)
+        a = rb_stride(0, x, H // 2, Wd // 2)
+        a = rb("ga", 1, a)
+        a = rb_stride(2, a, H // 4, Wd // 4)
+        a = self.se(a, W[f"{cn}.ga3"], b("ga3.o", a.H, a.W), csum=self.last_csum)
+        a = rb("ga", 4, a)
+        a = rb_stride(5, a, H // 8, Wd // 8)
+        a = rb("ga", 6, a)
+        a = self.conv([a], W[f"{cn}.ga7"], b("ga7.o", H // 16, Wd // 16), stride=2, csum=True)
+        y = self.se(a, W[f"{cn}.ga8"], b("y", a.H, a.W), csum=self.last_csum)
+        yh = b("y_hat", y.H, y.W)
+        if self.training:   # compressai quantize(y, "noise"): y + U(-0.5, 0.5)   (JointAutoregressiveHierarchicalPriors.forward)
+            self.call("tdvc_axpby", y.ptr, self.noise[f"{cn}.y"].ptr, yh.ptr, y.N * y.H * y.W * 128, 1.0, 1.0)
+        else:
+            self.call("tdvc_round_half_even", y.ptr, yh.ptr, y.N * y.H * y.W * 128, nbytes=8 * y.N * y.H * y.W * 128)
+        return y, yh
+
+    def _rb(self, W, cn, b, lr):
+        def rb(pfx, i, x):
+            t = self.conv([x], W[f"{cn}.{pfx}{i}.conv1"], b(f"{pfx}{i}.t", x.H, x.W), **lr)
+            return self.conv([t], W[f"{cn}.{pfx}{i}.conv2"], b(f"{pfx}{i}.o", x.H, x.W), res1=x, **lr)
+        return rb
+
+    def synthesis(self, W, cn, yh, final_res=None, out=None):
+        """g_s of coder `cn` on a given y_hat (N, h, w, 128) -> x_hat (N, 16h, 16w, 64) (+ final_res, fused into the last
+        convolution; written to `out` if given).  The one g_s of forward, compress and decompress."""
+        N, H, Wd = yh.N, 16 * yh.H, 16 * yh.W
+        lr = dict(act=L.ACT_LRELU, slope=0.01)
+        b = self._cbuf(cn, N)
+        rb = self._rb(W, cn, b, lr)
+
+        # IGDN: as the GDN of g_a (analysis)
+        def rb_up(i, x):
+            h, w = 2 * x.H, 2 * x.W
+            am = self.absmax_ptr(f"{cn}.gs{i}")
+            t = self.conv([x], W[f"{cn}.gs{i}.subpel"], b(f"gs{i}.t", h, w), **lr)
+            t2 = self.conv([t], W[f"{cn}.gs{i}.conv"], b(f"gs{i}.t2", h, w), absmax_out=am)
+            idt = self.conv([x], W[f"{cn}.gs{i}.upsample"], b(f"gs{i}.id", h, w))
+            return self.conv([t2], W[f"{cn}.gs{i}.igdn"], b(f"gs{i}.o", h, w), in_square=True, post=L.POST_IGDN,
+                             mul=t2, res1=idt, absmax_in=am, csum=(i == 4))
+
+        g = self.se(yh, W[f"{cn}.gs0"], b("gs0.o", yh.H, yh.W))
+        g = rb("gs", 1, g)
+        g = rb_up(2, g)
+        g = rb("gs", 3, g)
+        g = rb_up(4, g)
+        g = self.se(g, W[f"{cn}.gs5"], b("gs5.o", g.H, g.W), csum=self.last_csum)
+        g = rb("gs", 6, g)
+        g = rb_up(7, g)
+        g = rb("gs", 8, g)
+        return self.conv([g], W[f"{cn}.gs9"], out if out is not None else b("x_hat", H, Wd, 64), res1=final_res)
+
     def _side_stream(self):
         if self._side is None:
             self._side = torch.cuda.Stream(device=self.dev)
         return self._side
 
-    def _hyper_path(self, W, cn, y, yh, acc_off, b, lr):
+    def _hyper_path(self, W, cn, y, yh, acc_off):
         """h_a, factorised prior on z, h_s, context model, entropy parameters, conditional likelihood -> sum ln p."""
+        lr = dict(act=L.ACT_LRELU, slope=0.01)
+        b = self._cbuf(cn, y.N)
         # ---- h_a
         h = self.conv([y], W[f"{cn}.ha0"], b("ha0", y.H, y.W), **lr)
         h = self.conv([h], W[f"{cn}.ha2"], b("ha2", y.H, y.W), **lr)
@@ -1001,21 +1025,8 @@ class _Plan:
         if_miss, assign, misses, keys = self._variant(refs_nchw, cache, ref_keys)
         # ---- prologue (eager: reads the caller's tensors): NCHW -> NHWC (ld 4) of what this frame needs
         imgs = self.buf("imgs", 2 * N, H, Wd, 3, ld=4)        # [0:N] = input, [N:2N] = x^(t-1)
-        ifr = self.buf("iframe", N, H, Wd, 3, ld=4)
-        fr = 3 * H * Wd * 4
         self.call("tdvc_nchw_to_nhwc", x_nchw.data_ptr(), imgs.ptr, N, 3, H, Wd, 4, nbytes=28 * N * H * Wd)
-        miss_imgs = {}
-        for n in range(N):
-            base = refs_nchw.data_ptr() + n * 4 * fr
-            if if_miss:
-                self.call("tdvc_nchw_to_nhwc", base, ifr.batch(n).ptr, 1, 3, H, Wd, 4, nbytes=28 * H * Wd)
-            self.call("tdvc_nchw_to_nhwc", base + 3 * fr, imgs.batch(N + n).ptr, 1, 3, H, Wd, 4, nbytes=28 * H * Wd)
-            for e, j in misses:
-                if j == 2:
-                    miss_imgs[e] = imgs.batch(N, N)
-                else:
-                    mi = miss_imgs.setdefault(e, self.buf(f"mf.img{j}", N, H, Wd, 3, ld=4))
-                    self.call("tdvc_nchw_to_nhwc", base + (j + 1) * fr, mi.batch(n).ptr, 1, 3, H, Wd, 4, nbytes=28 * H * Wd)
+        miss_imgs = self._load_refs(refs_nchw, if_miss, misses, imgs.batch(N, N))
         variant = (if_miss, assign, tuple((e, j) for e, j in misses), self.impl, self.precision)
         pre = self.launches
         if graph and taps is None and self.prof is None:
@@ -1034,7 +1045,31 @@ class _Plan:
                 self.launches = pre + g[1]
         else:
             self.body(W, if_miss, assign, misses, miss_imgs, taps)
-        # ---- the caches now hold what this frame computed
+        self._commit(cache, keys, assign, misses)
+        return self.raw("recon", (N, 3, H, Wd)), self.bpp
+
+    def _load_refs(self, refs_nchw, if_miss, misses, last):
+        """NCHW -> NHWC (ld 4) of the reference slices a frame reads: refer_frames[:, 3] into `last` (N images) always, the
+        I-frame and the references whose fusion front missed the ring only when they missed.  Returns {ring entry: images}."""
+        N, H, Wd = self.N, self.H, self.W
+        ifr = self.buf("iframe", N, H, Wd, 3, ld=4)
+        fr = 3 * H * Wd * 4
+        miss_imgs = {}
+        for n in range(N):
+            base = refs_nchw.data_ptr() + n * 4 * fr
+            if if_miss:
+                self.call("tdvc_nchw_to_nhwc", base, ifr.batch(n).ptr, 1, 3, H, Wd, 4, nbytes=28 * H * Wd)
+            self.call("tdvc_nchw_to_nhwc", base + 3 * fr, last.batch(n).ptr, 1, 3, H, Wd, 4, nbytes=28 * H * Wd)
+            for e, j in misses:
+                if j == 2:
+                    miss_imgs[e] = last
+                else:
+                    mi = miss_imgs.setdefault(e, self.buf(f"mf.img{j}", N, H, Wd, 3, ld=4))
+                    self.call("tdvc_nchw_to_nhwc", base + (j + 1) * fr, mi.batch(n).ptr, 1, 3, H, Wd, 4, nbytes=28 * H * Wd)
+        return miss_imgs
+
+    def _commit(self, cache, keys, assign, misses):
+        """The caches now hold what this frame computed."""
         self.frame_no += 1
         if cache:
             self.if_key = keys[0]
@@ -1044,32 +1079,62 @@ class _Plan:
                 self.ring_used[e] = self.frame_no
         else:
             self.if_key, self.ring = None, [None, None, None]
-        return self.raw("recon", (N, 3, H, Wd)), self.bpp
+
+    def _frame_start(self, W, if_miss, misses, miss_imgs):
+        """Per-frame state (bit sums, GDN maxima) to zero, then the per-GOP / per-reference features that missed their cache."""
+        self._order = 0
+        self.call("tdvc_zero_bytes", self.fstate.data_ptr(), self.fstate.numel() * 8)
+        self.launches -= 1   # a memset node, not a kernel
+        if if_miss:
+            self.loopfilter_ref(W, self.buf("iframe", self.N, self.H, self.W, 3, ld=4))
+        for e, j in misses:
+            self.mcfilter_front(W, miss_imgs[e], e)
 
     def body(self, W, if_miss, assign, misses, miss_imgs, taps):
         """Everything of the frame that only touches plan buffers (graph-capturable)."""
         N, H, Wd = self.N, self.H, self.W
-        lib = self.lib
-        lr1 = dict(act=L.ACT_LRELU, slope=0.1)
-        self._order = 0
-        self.call("tdvc_zero_bytes", self.fstate.data_ptr(), self.fstate.numel() * 8)
-        self.launches -= 1   # a memset node, not a kernel
+        self._frame_start(W, if_miss, misses, miss_imgs)
         imgs = self.buf("imgs", 2 * N, H, Wd, 3, ld=4)
-        ifr = self.buf("iframe", N, H, Wd, 3, ld=4)
-        # ---- per-GOP / per-reference features that missed their cache
-        if if_miss:
-            self.loopfilter_ref(W, ifr)
-        for e, j in misses:
-            self.mcfilter_front(W, miss_imgs[e], e)
         # ---- feature extraction on both images (pnet.py:29-30, 86-96)
-        f0 = self.conv([imgs], W["extra_fea.conv_first"], self.buf("fe.0", 2 * N, H, Wd, 64), **lr1)
-        feats = self.res_stack(W, "extra_fea.res", 2, f0, "fe", out_last=self.buf("feats", 2 * N, H, Wd, 64))
+        feats = self.features(W, imgs)
         in_f, ref_f = feats.batch(0, N), feats.batch(N, N)
         # ---- motion estimation (pnet.py:131-167)
         estmv = self.motion_est(W, feats, imgs, taps)
         # ---- motion coder (pnet.py:34-43)
         mv_xhat = self.coder(W, "mv", estmv, 0, taps)
-        # ---- motion compensation (pnet.py:52, 179-184; dcn_v2_amp.py:219-234)
+        # ---- prediction (pnet.py:52-53); the residual input_feat - prediction of pnet.py:55 is written by the same pass
+        resid = self.buf("resid", N, H, Wd, 64)
+        pred1, pred = self.predict(W, mv_xhat, ref_f, assign, in_f, resid, taps)
+        # ---- residual coder (pnet.py:55-67, 76)
+        rec_f = self.coder(W, "rs", resid, 2, taps, final_res=pred, out=self.buf("rec_f", N, H, Wd, 64))
+        self.finish(W, rec_f, taps)
+        # ---- bpp (pnet.py:38-43, 62-67): sum ln p / (-ln2 * N*H*W), per coder
+        self.call("tdvc_bpp_finish", self.acc.data_ptr(), self.bpp.data_ptr(), C.c_double(-1.0 / (_LN2 * N * H * Wd)))
+        if taps is not None:
+            self._stage_taps(taps, mv_xhat, pred1, pred, rec_f)
+            taps.update({"input_feat": in_f.nchw(), "ref_feat": ref_f.nchw(), "estmv": estmv.nchw(),
+                         "input_residual": resid.nchw()})
+
+    @staticmethod
+    def _stage_taps(taps, mv_xhat, pred1, pred, rec_f):
+        taps.update({"mv.x_hat": mv_xhat.nchw(), "prediction1": pred1.nchw(), "prediction": pred.nchw(),
+                     "recon_feat": rec_f.nchw()})
+
+    def features(self, W, imgs, tag="fe", out="feats"):
+        """extra_fea (pnet.py:86-96) on a batch of images (N, H, W, 3 in ld 4) -> (N, H, W, 64).  Every launch works on
+        tiles of one image and picks its configuration from nothing but the layer's shape, so an image's features do not
+        depend on what else is in the batch: the decoder's reference-only batch reproduces the encoder's [input; ref]."""
+        f0 = self.conv([imgs], W["extra_fea.conv_first"], self.buf(tag + ".0", imgs.N, imgs.H, imgs.W, 64),
+                       act=L.ACT_LRELU, slope=0.1)
+        return self.res_stack(W, "extra_fea.res", 2, f0, tag, out_last=self.buf(out, imgs.N, imgs.H, imgs.W, 64))
+
+    def predict(self, W, mv_xhat, ref_f, assign, sub_from=None, out2=None, taps=None):
+        """The prediction from the decoded motion x_hat and the reference features: motion compensation (pnet.py:52,
+        179-184; dcn_v2_amp.py:219-234) and the multi-frame fusion (:53, 277-293, 309-317) over the references of ring
+        entries `assign`.  Returns (prediction1, prediction); with sub_from / out2 the fusion's last pass also writes
+        out2 = sub_from - prediction (the residual of pnet.py:55)."""
+        N, H, Wd = self.N, self.H, self.W
+        lr1 = dict(act=L.ACT_LRELU, slope=0.1)
         dcn_out = self.buf("mc.dcn", N, H, Wd, 64)
         dp = L.DcnParams()
         wb = W.get("mc.dcn.w_f16")
@@ -1086,43 +1151,98 @@ class _Plan:
             dp.offset, dp.off_ld = om.data_ptr(), 216
             dp.mask, dp.mask_ld, dp.mask_is_logit = om.data_ptr() + 4 * 144 * H * Wd, 216, 1
             dp.weight_f16 = wb.data_ptr()
-            om_nchw = om
         else:
             om = self.conv([mv_xhat], W["mc.offmask"], self.buf("mc.om", N, H, Wd, 216, ld=216))
             dp.input, dp.in_ld = ref_f.ptr, ref_f.ld
             dp.offset, dp.off_ld = om.ptr, om.ld
             dp.mask, dp.mask_ld, dp.mask_is_logit = om.chan(144, 72).ptr, om.ld, 1
-            om_nchw = None
         dp.weight_packed, dp.bias = W["mc.dcn.w"].data_ptr(), W["mc.dcn.b"].data_ptr()
         dp.out, dp.out_ld = dcn_out.ptr, dcn_out.ld
         dp.N, dp.H, dp.W, dp.C, dp.O, dp.O_pad, dp.dg = N, H, Wd, 64, 64, 64, 8
         dp.round_fp16, dp.act, dp.slope = 1, L.ACT_LRELU, 0.1
         dp.impl = self.impl
         e0 = self._prof_begin()
-        L.check(lib.tdvc_dcn_nhwc(dp, self._st()), "dcn_nhwc")
+        L.check(self.lib.tdvc_dcn_nhwc(dp, self._st()), "dcn_nhwc")
         # algorithmic bytes: ref 256 + offsets 576 + masks 288 + out 256 B/px (SURVEY.md 8d)
         self._prof_end(e0, "dcn_tc" if tc_dcn else "dcn_nhwc", macs=N * H * Wd * 576 * 64, nbytes=N * H * Wd * 1376,
                        products=4 if tc_dcn else 0)
         self.launches += 1
         o2 = self.conv([dcn_out, ref_f], W["mc.conv"], self.buf("mc.o2", N, H, Wd, 64), **lr1)
         pred1 = self.res_stack(W, "mc.res", 3, o2, "mc", last_res2=dcn_out, out_last=self.buf("pred1", N, H, Wd, 64))
-        # ---- multi-frame fusion (pnet.py:277-293, 309-317)
-        # (the residual input_feat - prediction of pnet.py:55 is written by the same pass that finishes the prediction)
-        resid = self.buf("resid", N, H, Wd, 64)
-        pred = self.mcfilter(W, pred1, assign, in_f, resid)
-        # ---- residual coder (pnet.py:55-67, 76)
-        rec_f = self.coder(W, "rs", resid, 2, taps, final_res=pred, out=self.buf("rec_f", N, H, Wd, 64))
-        # ---- reference-based in-loop filter (pnet.py:213-263) + clamp (:78)
+        pred = self.mcfilter(W, pred1, assign, sub_from, out2)
+        if taps is not None:
+            taps.update({"mcnet.om": om.clone() if tc_dcn else om.nchw(), "mcnet.dcn_act": dcn_out.nchw()})
+        return pred1, pred
+
+    def finish(self, W, rec_f, taps):
+        """The reconstruction from the reconstructed features (residual x_hat + prediction): reference-based in-loop filter
+        (pnet.py:213-263) with the clamp (:78) in its last convolution, then NCHW.  Returns the plan's recon buffer."""
+        N, H, Wd = self.N, self.H, self.W
         recon4 = self.loopfilter(W, rec_f, taps)
         recon = self.raw("recon", (N, 3, H, Wd))
         self.call("tdvc_nhwc_to_nchw", recon4.ptr, recon4.ld, recon.data_ptr(), N, 3, H, Wd, nbytes=28 * N * H * Wd)
-        # ---- bpp (pnet.py:38-43, 62-67): sum ln p / (-ln2 * N*H*W), per coder
-        self.call("tdvc_bpp_finish", self.acc.data_ptr(), self.bpp.data_ptr(), C.c_double(-1.0 / (_LN2 * N * H * Wd)))
+        return recon
+
+    # ---------------------------------------------------------------- the closed loop: encoder and decoder of one P-frame
+    def compress(self, W, tables, x_nchw, refs_nchw, cache=True, ref_keys=None, taps=None):
+        """Closed-loop encoder of one P-frame (eager).  Both syntheses run on the autoregressive y_hat the strings code
+        (round(y - mu) + mu, `launch_coding`), not on forward's round(y), so the reconstruction is the frame a decoder
+        rebuilds.  The residual coder's input depends on the motion coder's autoregressive pass, so the two passes run one
+        after the other; the host rANS of both (`coding.finish_coding`) is left to the caller and overlaps what is queued.
+        tables: {"mv" | "rs": coding.CoderTables}.  Returns (the plan's recon buffer, {"mv" | "res": launch_coding handle})."""
+        N, H, Wd = self.N, self.H, self.W
+        self.launches = 0
+        if_miss, assign, misses, keys = self._variant(refs_nchw, cache, ref_keys)
+        imgs = self.buf("imgs", 2 * N, H, Wd, 3, ld=4)
+        self.call("tdvc_nchw_to_nhwc", x_nchw.data_ptr(), imgs.ptr, N, 3, H, Wd, 4, nbytes=28 * N * H * Wd)
+        miss_imgs = self._load_refs(refs_nchw, if_miss, misses, imgs.batch(N, N))
+        self._frame_start(W, if_miss, misses, miss_imgs)
+        feats = self.features(W, imgs)
+        in_f, ref_f = feats.batch(0, N), feats.batch(N, N)
+        estmv = self.motion_est(W, feats, imgs, None)
+        handles = {}
+        handles["mv"], mv_yh = self._analyse_and_code(W, tables, "mv", estmv, 0)
+        mv_xhat = self.synthesis(W, "mv", mv_yh)
+        resid = self.buf("resid", N, H, Wd, 64)
+        pred1, pred = self.predict(W, mv_xhat, ref_f, assign, in_f, resid)
+        handles["res"], rs_yh = self._analyse_and_code(W, tables, "rs", resid, 2)
+        rec_f = self.synthesis(W, "rs", rs_yh, final_res=pred, out=self.buf("rec_f", N, H, Wd, 64))
+        recon = self.finish(W, rec_f, None)
         if taps is not None:
-            taps.update({"input_feat": in_f.nchw(), "ref_feat": ref_f.nchw(), "estmv": estmv.nchw(),
-                         "mv.x_hat": mv_xhat.nchw(), "mcnet.om": om_nchw.clone() if om_nchw is not None else om.nchw(), "mcnet.dcn_act": dcn_out.nchw(),
-                         "prediction1": pred1.nchw(), "prediction": pred.nchw(), "input_residual": resid.nchw(),
-                         "recon_feat": rec_f.nchw()})
+            self._stage_taps(taps, mv_xhat, pred1, pred, rec_f)
+        self._commit(cache, keys, assign, misses)
+        return recon, handles
+
+    def _analyse_and_code(self, W, tables, cn, x, acc_off):
+        """g_a, the hyper path (as forward runs it) and the device half of coding for coder `cn`.  Returns (launch_coding
+        handle, its autoregressive y_hat as an Act over the same memory)."""
+        from tdvc_b200 import coding
+        y, yh = self.analysis(W, cn, x)
+        self._hyper_path(W, cn, y, yh, acc_off)
+        h = coding.launch_coding(self, W, cn, tables[cn])
+        t = h["dev"]["y_hat"]
+        return h, Act(t, t.data_ptr(), y.N, y.H, y.W, 128, 128)
+
+    def decompress(self, W, y_hat, refs_nchw, cache=True, ref_keys=None, taps=None):
+        """Decoder of one P-frame from both coders' decoded y_hat ({"mv" | "rs": Act (N, H/16, W/16, 128)}) and the
+        reference frames: extra_fea of refer_frames[:, -1], motion g_s, the prediction, residual g_s + prediction and the
+        in-loop filter - the encoder's launches on the same shapes.  The per-GOP caches serve as in `run`.  Returns the
+        plan's recon buffer."""
+        N, H, Wd = self.N, self.H, self.W
+        self.launches = 0
+        if_miss, assign, misses, keys = self._variant(refs_nchw, cache, ref_keys)
+        ref = self.buf("dec.ref", N, H, Wd, 3, ld=4)
+        miss_imgs = self._load_refs(refs_nchw, if_miss, misses, ref)
+        self._frame_start(W, if_miss, misses, miss_imgs)
+        ref_f = self.features(W, ref, "dec.fe", "dec.ref_f")
+        mv_xhat = self.synthesis(W, "mv", y_hat["mv"])
+        pred1, pred = self.predict(W, mv_xhat, ref_f, assign)
+        rec_f = self.synthesis(W, "rs", y_hat["rs"], final_res=pred, out=self.buf("rec_f", N, H, Wd, 64))
+        recon = self.finish(W, rec_f, None)
+        if taps is not None:
+            self._stage_taps(taps, mv_xhat, pred1, pred, rec_f)
+        self._commit(cache, keys, assign, misses)
+        return recon
 
     def fusion_and_filter(self, W, pred1_nchw, refs_nchw, recf_nchw):
         """BASELINE config 5: the multi-frame feature fusion (reference pnet.py:266-293, 296-317) and the reference-based
@@ -1489,7 +1609,7 @@ class VideoCompressor(nn.Module):
         and drops them (the return tuple is unchanged); here they stay readable in `self.last_coded`:
         {"mv" | "res": {"strings": [y_strings, z_strings], "shape": (h, w), "ac_bpp": float}}."""
         from tdvc_b200 import coding
-        out, pending = {}, []
+        pending = []
         main = torch.cuda.current_stream(plan.dev)
         side = plan._side_stream()
         for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
@@ -1499,6 +1619,15 @@ class VideoCompressor(nn.Module):
             if stream is not main:
                 stream.wait_stream(main)
             pending.append((nm, coding.launch_coding(plan, Wt, cn, tabs, stream=stream)))
+        out = self._finish_coding(pending, num_pixels, taps)
+        main.wait_stream(side)
+        return out
+
+    @staticmethod
+    def _finish_coding(pending, num_pixels, taps=None):
+        """Host half of coding, in the order given: [(name, launch_coding handle), ...] -> `last_coded`."""
+        from tdvc_b200 import coding
+        out = {}
         for nm, h in pending:
             enc = coding.finish_coding(h, keep=taps is not None)
             enc["ac_bpp"] = sum(len(s[0]) for s in enc["strings"]) * 8.0 / num_pixels
@@ -1506,7 +1635,6 @@ class VideoCompressor(nn.Module):
                 for k in ("y_symbols", "y_indexes", "y_hat", "z_symbols"):
                     taps[f"{nm}.ac.{k}"] = enc.pop(k)
             out[nm] = enc
-        main.wait_stream(side)
         return out
 
     def _coder_tables(self, Wt, cn, dev):
@@ -1524,6 +1652,72 @@ class VideoCompressor(nn.Module):
             smod.gaussian_conditional.scale_table = tabs[cn].scale_table.clone()
         return tabs[cn]
 
+    def compress(self, input_image, refer_frames, enabled_amp=False, ref_keys=None, taps=None):
+        """Closed-loop encoder of one P-frame: -> (recon (N,3,H,W) fp32, data: the version-2 container's bytes).
+        Unlike `forward`, both coders' syntheses run on the y_hat the strings carry (quantised relative to the predicted
+        mean, round(y - mu) + mu), so `recon` is the frame `decompress(data, refer_frames)` rebuilds bit for bit; the
+        prediction and the residual are computed from the decoded motion.  A GOP feeds this recon to the next frame
+        (`tdvc_b200.gop.compress_gop`).  `self.last_coded` is left as `forward(..., is_compress=True)` leaves it.
+        Runs eagerly (no CUDA graph) and shares the plan and the per-GOP feature caches with `forward`.
+        enabled_amp / ref_keys as in `forward`; the precision mode goes into the container.  taps: also records "mv.x_hat",
+        "prediction1", "prediction", "recon_feat" and each coder's "ac.*" symbols, indexes and y_hat."""
+        if self.training:
+            raise RuntimeError("compress is served in eval() mode (the reference switches both coders to eval() before it "
+                               "codes, pnet.py:46,70)")
+        N, H, W = self._check(input_image, refer_frames, 3)
+        if refer_frames.device != input_image.device:
+            raise RuntimeError("compress: input_image and refer_frames are on different devices")
+        if ref_keys is not None and len(ref_keys) != 4:
+            raise RuntimeError("ref_keys: expected four identities, one per reference slice")
+        from tdvc_b200 import coding
+        dev = input_image.device
+        with torch.cuda.device(dev), torch.no_grad():
+            x = input_image.detach().float().contiguous()
+            refs = refer_frames.detach().float().contiguous()
+            Wt = self._weights(dev)
+            plan = self._plan(N, H, W, dev)
+            plan.bind(Wt)
+            plan.impl, plan.precision = self.conv_impl, self._precision(enabled_amp)
+            tables = {cn: self._coder_tables(Wt, cn, dev) for cn in ("mv", "rs")}
+            recon, handles = plan.compress(Wt, tables, x, refs, cache=self.cache_features, ref_keys=ref_keys, taps=taps)
+            recon = recon.clone()
+            # the host codes the motion strings while the residual half of the frame is still running on the device
+            self.last_coded = self._finish_coding(list(handles.items()), N * H * W, taps)
+        return recon, coding.pack_frame(self.last_coded, frame={"size": (H, W), "N": N, "precision": plan.precision})
+
+    def decompress(self, data, refer_frames, ref_keys=None, taps=None):
+        """Decoder of one P-frame: a version-2 container (`compress`) and the same refer_frames (N,4,3,H,W) the encoder
+        used -> recon (N,3,H,W) fp32, bit-identical to `compress`'s recon.  Both coders' y_hat come from the path of
+        `decompress_latents`; then extra_fea of refer_frames[:, -1], motion g_s, the prediction, residual g_s + prediction
+        and the in-loop filter run on the encoder's launches.  The precision mode is the container's; the per-GOP feature
+        caches serve as in `forward` (ref_keys likewise).  Exactness needs the encoder's kernels on sm_100a and its
+        `conv_impl`, which the container does not record: this module's own is used.
+        A malformed container, or refer_frames that do not match its frame, raise RuntimeError before any device work; a
+        broken string raises as in `decompress_latents`.  taps: records "mv.x_hat", "prediction1", "prediction",
+        "recon_feat"."""
+        box = self._container(data, "decompress")
+        (H, Wd), N = box["frame"]["size"], box["frame"]["N"]
+        if not isinstance(refer_frames, torch.Tensor) or tuple(refer_frames.shape) != (N, 4, 3, H, Wd):
+            got = tuple(refer_frames.shape) if isinstance(refer_frames, torch.Tensor) else type(refer_frames).__name__
+            raise RuntimeError(f"decompress: refer_frames {got} do not match the container's frame (expected "
+                               f"{(N, 4, 3, H, Wd)})")
+        if ref_keys is not None and len(ref_keys) != 4:
+            raise RuntimeError("ref_keys: expected four identities, one per reference slice")
+        dev = self._decoder_device()
+        if refer_frames.device != dev:
+            raise RuntimeError(f"decompress: refer_frames are on {refer_frames.device}, the module on {dev}")
+        with torch.cuda.device(dev), torch.no_grad():
+            refs = refer_frames.detach().float().contiguous()
+            Wt = self._weights(dev)
+            plan = self._plan(N, H, Wd, dev)
+            plan.bind(Wt)
+            plan.impl, plan.precision = self.conv_impl, box["frame"]["precision"]
+            lat = self._decode_latents(box, plan, Wt, dev)
+            y_hat = {cn: Act(t, t.data_ptr(), *t.shape, t.shape[3])
+                     for cn, t in (("mv", lat["mv"]["y_hat"]), ("rs", lat["res"]["y_hat"]))}
+            recon = plan.decompress(Wt, y_hat, refs, cache=self.cache_features, ref_keys=ref_keys, taps=taps)
+            return recon.clone()
+
     def decompress_latents(self, data):
         """Both coders' latents of one P-frame from the bytes of a version-2 container (`coding.pack_frame(net.last_coded,
         frame=...)`) and the weights alone: no reference frames and nothing the encoder left behind.  Per coder: the z strings
@@ -1536,29 +1730,9 @@ class VideoCompressor(nn.Module):
         as the encoder ran with: h_s feeds every predicted mean and scale, and the container does not record conv_impl.
         A malformed container raises RuntimeError before any device work; a broken z string raises naming the coder and
         the image, a broken y string naming the latent position."""
-        from tdvc_b200 import coding
-        box = coding.unpack_frame(data)
-        frame = box.get("frame")
-        if frame is None:
-            raise RuntimeError("decompress_latents: a version-1 container records no cluster sizes, so its y strings cannot "
-                               "be decoded exactly (write version 2: pack_frame(..., frame=...))")
-        (H, Wd), N = frame["size"], frame["N"]
-        if N < 1 or H < 64 or Wd < 64 or H % 64 or Wd % 64:
-            raise RuntimeError(f"decompress_latents: frame {H}x{Wd}, N={N} (H and W multiples of 64, N >= 1)")
-        for nm in ("mv", "res"):
-            enc = box.get(nm)
-            if enc is None:
-                raise RuntimeError(f"decompress_latents: the container has no {nm} coder")
-            if tuple(enc["shape"]) != (H // 64, Wd // 64):
-                raise RuntimeError(f"decompress_latents: {nm} hyper-latent shape {tuple(enc['shape'])} for a {H}x{Wd} "
-                                   f"frame (expected {(H // 64, Wd // 64)})")
-            if len(enc["strings"]) != 2 or any(len(lst) != N for lst in enc["strings"]):
-                raise RuntimeError(f"decompress_latents: {nm} has {[len(lst) for lst in enc['strings']]} strings (two "
-                                   f"lists, y and z, of {N})")
-        dev = self.mvCoder.entropy_bottleneck.quantiles.device
-        if dev.type != "cuda":
-            raise RuntimeError("tdvc_b200.VideoCompressor runs on CUDA (sm_100a) only; there is no CPU fallback")
-        hz, wz = H // 64, Wd // 64
+        box = self._container(data, "decompress_latents")
+        (H, Wd), N = box["frame"]["size"], box["frame"]["N"]
+        dev = self._decoder_device()
         with torch.cuda.device(dev), torch.no_grad():
             Wt = self._weights(dev)
             plan = self._plan(N, H, Wd, dev)
@@ -1566,30 +1740,72 @@ class VideoCompressor(nn.Module):
             # h_s is fp32-class in both precision modes (only rs.g_s* and lf.* take one-product weights), so the container's
             # `precision` does not affect the latents and plan.precision is left as the last forward set it
             plan.impl = self.conv_impl
-            main = torch.cuda.current_stream(dev)
-            side = plan._side_stream()
-            side.wait_stream(main)
-            pending = []
-            for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
-                tabs = self._coder_tables(Wt, cn, dev)
-                enc = box[nm]
-                z_sym = coding.decode_z_symbols(cn, enc["strings"][1], tabs, hz, wz)
-                # every buffer under dec.{cn}.*: the forward pass and launch_coding never read what the decoder writes
-                b = lambda nme, h, w, c=128, cn=cn, **kw: plan.buf(f"dec.{cn}.{nme}", N, h, w, c, **kw)
-                with torch.cuda.stream(stream):
-                    sym_d = torch.from_numpy(z_sym).to(dev)
-                    zh = b("z_hat", hz, wz)
-                    coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
-                    params = plan.hyper_synthesis(Wt, cn, zh, b)
-                # the motion chain is already decoding on the device while the host decodes the residual z strings
-                h = coding.launch_decoding(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream)
-                pending.append((nm, zh, h))
-            main.wait_stream(side)
-            out = {"frame": dict(frame)}
-            for nm, zh, h in pending:
-                y = coding.finish_decoding(h)
-                out[nm] = {k: v.clone() for k, v in y.items()}
-                out[nm]["z_hat"] = zh.t.clone()
+            lat = self._decode_latents(box, plan, Wt, dev)
+            out = {"frame": dict(box["frame"])}
+            for nm in ("mv", "res"):
+                out[nm] = {k: v.clone() for k, v in lat[nm].items() if k != "z_hat"}
+                out[nm]["z_hat"] = lat[nm]["z_hat"].t.clone()
+        return out
+
+    @staticmethod
+    def _container(data, who):
+        """Unpack a container and check, on the host, that it can be decoded: version 2, both coders, a frame size of
+        multiples of 64, hyper-latent shapes that fit it, two string lists of N per coder.  -> the unpacked container."""
+        from tdvc_b200 import coding
+        box = coding.unpack_frame(data)
+        frame = box.get("frame")
+        if frame is None:
+            raise RuntimeError(f"{who}: a version-1 container records no cluster sizes, so its y strings cannot "
+                               "be decoded exactly (write version 2: pack_frame(..., frame=...))")
+        (H, Wd), N = frame["size"], frame["N"]
+        if N < 1 or H < 64 or Wd < 64 or H % 64 or Wd % 64:
+            raise RuntimeError(f"{who}: frame {H}x{Wd}, N={N} (H and W multiples of 64, N >= 1)")
+        for nm in ("mv", "res"):
+            enc = box.get(nm)
+            if enc is None:
+                raise RuntimeError(f"{who}: the container has no {nm} coder")
+            if tuple(enc["shape"]) != (H // 64, Wd // 64):
+                raise RuntimeError(f"{who}: {nm} hyper-latent shape {tuple(enc['shape'])} for a {H}x{Wd} "
+                                   f"frame (expected {(H // 64, Wd // 64)})")
+            if len(enc["strings"]) != 2 or any(len(lst) != N for lst in enc["strings"]):
+                raise RuntimeError(f"{who}: {nm} has {[len(lst) for lst in enc['strings']]} strings (two "
+                                   f"lists, y and z, of {N})")
+        return box
+
+    def _decoder_device(self):
+        dev = self.mvCoder.entropy_bottleneck.quantiles.device
+        if dev.type != "cuda":
+            raise RuntimeError("tdvc_b200.VideoCompressor runs on CUDA (sm_100a) only; there is no CPU fallback")
+        return dev
+
+    def _decode_latents(self, box, plan, Wt, dev):
+        """Device half of decompress_latents on a checked container: {"mv" | "res": {"y_hat", "y_symbols", "y_indexes":
+        tensors of their own, "z_hat": the plan's dec.{cn}.z_hat Act}}, both coders finished."""
+        from tdvc_b200 import coding
+        N = box["frame"]["N"]
+        hz, wz = box["mv"]["shape"]
+        main = torch.cuda.current_stream(dev)
+        side = plan._side_stream()
+        side.wait_stream(main)
+        pending = []
+        for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
+            tabs = self._coder_tables(Wt, cn, dev)
+            enc = box[nm]
+            z_sym = coding.decode_z_symbols(cn, enc["strings"][1], tabs, hz, wz)
+            # every buffer under dec.{cn}.*: the forward pass and launch_coding never read what the decoder writes
+            b = lambda nme, h, w, c=128, cn=cn, **kw: plan.buf(f"dec.{cn}.{nme}", N, h, w, c, **kw)
+            with torch.cuda.stream(stream):
+                sym_d = torch.from_numpy(z_sym).to(dev)
+                zh = b("z_hat", hz, wz)
+                coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
+                params = plan.hyper_synthesis(Wt, cn, zh, b)
+            # the motion chain is already decoding on the device while the host decodes the residual z strings
+            h = coding.launch_decoding(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream)
+            pending.append((nm, zh, h))
+        main.wait_stream(side)
+        out = {}
+        for nm, zh, h in pending:
+            out[nm] = dict(coding.finish_decoding(h), z_hat=zh)
         return out
 
     def _forward_training(self, input_image, refer_frames, taps=None, noise=None):

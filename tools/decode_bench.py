@@ -7,7 +7,11 @@ TDVC_B200_AR_DEBUG=1 adds the encoder's per-phase times on stderr.
 once both coders' latents are on the device) on the version-2 container of the frame `forward(is_compress=True)` coded,
 decoded by a second module loaded from the same weights; the per-coder `tdvc_ar_decode` times of the same run stand beside
 it, so the overlap of the two coders' chains can be read off.
-python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}] [--container]  ->  one JSON line."""
+--codec: also time the closed-loop codec end to end: `VideoCompressor.compress` (features to container bytes, host rANS
+included) and `VideoCompressor.decompress` of its container by a second module (container to reconstruction), each with a
+host clock around the call and a device synchronise after it, median of `reps` after a warm-up.  The per-GOP feature caches
+are off, so every frame computes everything a GOP's first P-frame computes; the round trip is checked bit for bit.
+python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}] [--container] [--codec]  ->  one JSON line."""
 import argparse
 import json
 import subprocess
@@ -41,6 +45,7 @@ def main():
     ap.add_argument("reps", nargs="?", type=int, default=5)
     ap.add_argument("--encoder-cluster", type=int, choices=(0, 8, 16), default=16)
     ap.add_argument("--container", action="store_true", help="also time decompress_latents on the frame's container")
+    ap.add_argument("--codec", action="store_true", help="also time compress and decompress end to end")
     args = ap.parse_args()
     reps, cl = args.reps, args.encoder_cluster
     dev = torch.device("cuda:0")
@@ -93,7 +98,34 @@ def main():
         res[cn] = {"ar_code_ms": round(sorted(enc_ms)[len(enc_ms) // 2], 3), "ar_decode_ms": round(dec_med, 3),
                    "ar_decode_us_per_step": round(1e3 * dec_med / (hy * wy), 3),
                    "ar_decode_ms_all": [round(t, 3) for t in dec_ms]}
+    if args.codec:
+        enc, dec = (_module(orc, dev, cache=False) for _ in range(2))
+        xd, rd = x.to(dev), refs.to(dev)
+        c_ms, d_ms = [], []
+        for rep in range(reps + 1):   # rep 0: warm-up (packs the weights, builds the tables and both plans)
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            recon, data = enc.compress(xd, rd)
+            torch.cuda.synchronize()
+            t1 = time.perf_counter()
+            got = dec.decompress(data, rd)
+            torch.cuda.synchronize()
+            t2 = time.perf_counter()
+            assert torch.equal(got, recon)
+            c_ms.append(1e3 * (t1 - t0))
+            d_ms.append(1e3 * (t2 - t1))
+        c_ms, d_ms = c_ms[1:], d_ms[1:]
+        res["codec"] = {"bytes": len(data), "compress_ms": round(sorted(c_ms)[len(c_ms) // 2], 3),
+                        "decompress_ms": round(sorted(d_ms)[len(d_ms) // 2], 3),
+                        "compress_ms_all": [round(t, 3) for t in c_ms], "decompress_ms_all": [round(t, 3) for t in d_ms]}
     print(json.dumps(res))
+
+
+def _module(orc, dev, cache=True):
+    m = VideoCompressor().eval()
+    m.load_state_dict(orc.state_dict())
+    m.cache_features = cache
+    return m.to(dev)
 
 
 if __name__ == "__main__":
