@@ -248,16 +248,24 @@ def launch_coding(plan, W, cn, tables, cluster=0, stream=None):
             "dev": {"y_symbols": y_sym, "y_indexes": y_idx, "y_hat": y_hat, "z_symbols": z_sym}}
 
 
-def finish_coding(h, keep=False):
+def finish_coding(h, keep=False, rows=False):
     """Host half: rANS over the symbols, one string per image (compressai codes batch items separately).
     Returns {"strings": [y_strings, z_strings], "shape": (h, w), "cluster": CTAs per image the y pass ran with (the
-    summation order a decoder must reproduce)} (+ clones of the device tensors if keep)."""
+    summation order a decoder must reproduce)} (+ clones of the device tensors if keep).
+    rows: y as row streams (container version 3, this project's own format): one string per latent row, N * h_y strings
+    in (image, row) order, each the symbols of one row in (w, c) order; their concatenation is the symbol sequence of the
+    one-string-per-image layout.  The output then also holds "y_streams": "rows"."""
     h["done"].synchronize()
     hs = [t.numpy() for t in h["host"]]
     tables = h["tables"]
-    y_strings = [rans_encode(hs[0][i], hs[1][i], tables.gc) for i in range(h["N"])]
+    if rows:
+        y_strings = [rans_encode(hs[0][i, r], hs[1][i, r], tables.gc) for i in range(h["N"]) for r in range(hs[0].shape[1])]
+    else:
+        y_strings = [rans_encode(hs[0][i], hs[1][i], tables.gc) for i in range(h["N"])]
     z_strings = [rans_encode(hs[2][i], hs[3][i], tables.eb) for i in range(h["N"])]
     out = {"strings": [y_strings, z_strings], "shape": h["shape"], "cluster": h["cluster"]}
+    if rows:
+        out["y_streams"] = "rows"
     if keep:
         out.update({k: v.clone() for k, v in h["dev"].items()})
     return out
@@ -265,6 +273,17 @@ def finish_coding(h, keep=False):
 
 def code_latents(plan, W, cn, tables, cluster=0, keep=False):
     return finish_coding(launch_coding(plan, W, cn, tables, cluster=cluster), keep=keep)
+
+
+def _gc_rows_ok(tables, max_total):
+    gl = tables.gc.length
+    return not (gl.size > 64 or (gl < 2).any() or (gl > tables.gc.cdf.shape[1]).any() or int(gl.sum()) > max_total)
+
+
+def _check_word_strings(strings, who, what):
+    for i, s_ in enumerate(strings):
+        if len(s_) < 8 or len(s_) % 4:
+            raise RuntimeError(f"{who}: {what(i)} has {len(s_)} bytes (rANS strings are whole 32-bit words, at least two)")
 
 
 def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
@@ -280,12 +299,9 @@ def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
         raise RuntimeError(f"decode_latents: encoder cluster size {cluster} (8 or 16)")
     if len(y_strings) != N:
         raise RuntimeError(f"decode_latents: {len(y_strings)} {cn} y strings for {N} images")
-    for i, s_ in enumerate(y_strings):
-        if len(s_) < 8 or len(s_) % 4:
-            raise RuntimeError(f"decode_latents: {cn} y string of image {i} has {len(s_)} bytes (rANS strings are whole "
-                               "32-bit words, at least two)")
+    _check_word_strings(y_strings, "decode_latents", lambda i: f"{cn} y string of image {i}")
     gl = tables.gc.length
-    if gl.size > 64 or (gl < 2).any() or (gl > tables.gc.cdf.shape[1]).any() or int(gl.sum()) > 32768:
+    if not _gc_rows_ok(tables, 32768):
         raise RuntimeError("decode_latents: the Gaussian CDF tables are not valid rows for the device decoder")
     stream = stream or torch.cuda.current_stream(dev)
     words = np.frombuffer(b"".join(bytes(s_) for s_ in y_strings), dtype="<i4")
@@ -314,12 +330,59 @@ def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
             "y_hat": y_hat, "y_symbols": y_sym, "y_indexes": y_idx}
 
 
+ROW_CDF_MAX = 27392   # CDF entries tdvc_ar_decode_rows holds in shared memory (64 Gaussian rows: 27,256)
+
+
+def launch_decoding_rows(W, cn, tables, y_strings, params, cluster, stream=None):
+    """Device decoding of ROW STREAMS of coder `cn` (finish_coding(..., rows=True), container version 3): N * h strings, one
+    per latent row in (image, row) order.  `tdvc_ar_decode_rows` is the encoder's own wavefront kernel with a decoding
+    epilogue, so the rows of a wavefront decode in parallel; it launches with the encoder's cluster size (8 or 16) and
+    nothing else.  Strings that are not whole words, or fewer than two, and a wrong string count raise RuntimeError before
+    any device work.  Returns a handle for finish_decoding."""
+    lib = L.load()
+    N, hy, wy = params.N, params.H, params.W
+    dev = params.t.device
+    if cluster not in (8, 16):
+        raise RuntimeError(f"decode_latents: encoder cluster size {cluster} (8 or 16)")
+    if len(y_strings) != N * hy:
+        raise RuntimeError(f"decode_latents: {len(y_strings)} {cn} y row strings for {N} images of {hy} rows")
+    _check_word_strings(y_strings, "decode_latents", lambda i: f"{cn} y row {i % hy} of image {i // hy}")
+    if not _gc_rows_ok(tables, ROW_CDF_MAX):
+        raise RuntimeError("decode_latents: the Gaussian CDF tables are not valid rows for the device decoder")
+    stream = stream or torch.cuda.current_stream(dev)
+    words = np.frombuffer(b"".join(bytes(s_) for s_ in y_strings), dtype="<i4")
+    offsets = np.cumsum([0] + [len(s_) // 4 for s_ in y_strings]).astype(np.int64)
+    cdf, length, offset = tables.gc.on(dev)
+    with torch.cuda.stream(stream):
+        words_d = torch.from_numpy(words.copy()).to(dev)
+        offsets_d = torch.from_numpy(offsets).to(dev)
+        y_hat = torch.empty((N, hy, wy, 128), device=dev)
+        y_sym = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
+        y_idx = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
+        status = torch.empty((N,), device=dev, dtype=torch.int64)
+        chain = _ar_chain(W, cn, tables, params, (y_hat, y_sym, y_idx), "decode_latents")
+        need = lib.tdvc_ar_decode_rows_workspace_bytes(N, hy, chain.c1_pad, chain.c2_pad)
+        ws = torch.empty(((need + 15) // 16 * 4,), device=dev)
+    p = L.ArRowDecodeParams(chain=chain, words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
+                            cdfs=cdf.data_ptr(), cdf_stride=cdf.shape[1], cdf_lengths=length.data_ptr(),
+                            cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(tables.gc.length.sum()),
+                            status=status.data_ptr(), cluster=cluster)
+    L.check(lib.tdvc_ar_decode_rows(C.byref(p), ws.data_ptr(), ws.numel() * 4, stream.cuda_stream), "ar_decode_rows")
+    with torch.cuda.stream(stream):
+        status_h = _pinned_like(status)
+        status_h.copy_(status, non_blocking=True)
+        done = torch.cuda.Event()
+        done.record(stream)
+    return {"cn": cn, "done": done, "status": status_h, "keep": (words_d, offsets_d, ws), "shape": (hy, wy),
+            "rows": True, "y_hat": y_hat, "y_symbols": y_sym, "y_indexes": y_idx}
+
+
 def _pinned_like(t):
     return torch.empty(t.shape, dtype=t.dtype).pin_memory()
 
 
 def finish_decoding(h):
-    """Waits for a launch_decoding and turns a failed image into RuntimeError (naming the coder, the image and the
+    """Waits for a launch_decoding or launch_decoding_rows and turns a failed image into RuntimeError (naming the coder, the image and the
     latent position (h, w, c) where the stream broke).  Returns {"y_hat", "y_symbols", "y_indexes"} (N, h, w, 128)."""
     h["done"].synchronize()
     wy = h["shape"][1]
@@ -328,13 +391,17 @@ def finish_decoding(h):
             raise RuntimeError(f"ar_decode: the Gaussian CDF tables of the {h['cn']} coder are not valid rows (image {i})")
         if st != -1:
             pix, c = divmod(int(st), 128)
+            if h.get("rows"):
+                raise RuntimeError(f"ar_decode_rows: {h['cn']} y row {pix // wy} of image {i} is truncated or corrupt at "
+                                   f"(h={pix // wy}, w={pix % wy}, c={c})")
             raise RuntimeError(f"ar_decode: the {h['cn']} y string of image {i} is truncated or corrupt at latent position "
                                f"(h={pix // wy}, w={pix % wy}, c={c})")
     return {k: h[k] for k in ("y_hat", "y_symbols", "y_indexes")}
 
 
-def decode_latents(W, cn, tables, y_strings, params, cluster, stream=None):
-    return finish_decoding(launch_decoding(W, cn, tables, y_strings, params, cluster, stream=stream))
+def decode_latents(W, cn, tables, y_strings, params, cluster, stream=None, rows=False):
+    launch = launch_decoding_rows if rows else launch_decoding
+    return finish_decoding(launch(W, cn, tables, y_strings, params, cluster, stream=stream))
 
 
 def eb_indexes(hz, wz, C=128):
@@ -372,6 +439,7 @@ def dequantize_z(symbols, medians, z_hat, stream=None):
 # ----------------------------------------------------------------------------------------------- bitstream container
 _MAGIC = b"TDVC"       # version 1: strings and hyper-latent shapes only
 _MAGIC_V2 = b"TDV2"    # version 2: + frame size, batch, precision mode, and each coder's autoregressive cluster size
+_MAGIC_V3 = b"TDV3"    # version 3: the layout of version 2 with y as row streams (one string per latent row)
 _PRECISIONS = ("exact", "mixed")
 
 
@@ -383,15 +451,20 @@ def pack_frame(coded, frame=None):
     per list: >I n_strings | per string: >I length | payload.
     frame={"size": (H, W), "N": N, "precision": "exact" | "mixed"} (version 2, what a decoder needs to reproduce the
     encoder exactly): magic "TDV2" | >2I H, W | >B N | >B precision (0 exact, 1 mixed) | >B n_coders | per coder: >4s name |
-    >B cluster (CTAs per image of the autoregressive pass: its summation order) | then as version 1."""
+    >B cluster (CTAs per image of the autoregressive pass: its summation order) | then as version 1.
+    frame={..., "y_streams": "rows"} (version 3, this project's own format, not readable by compressai): magic "TDV3", then
+    byte for byte the layout of version 2; only each coder's y list differs: N * h_y row strings in (image, latent row)
+    order (`finish_coding(..., rows=True)`), so that a decoder can decode the rows of a wavefront in parallel."""
     import struct
     if frame is None:
         out = [_MAGIC, struct.pack(">B", len(coded))]
     else:
         if frame.get("precision") not in _PRECISIONS:
             raise RuntimeError(f"pack_frame: precision must be one of {_PRECISIONS}, not {frame.get('precision')!r}")
+        if frame.get("y_streams", "rows") != "rows":
+            raise RuntimeError(f"pack_frame: y_streams must be 'rows' or absent, not {frame.get('y_streams')!r}")
         H, W = (int(v) for v in frame["size"])
-        out = [_MAGIC_V2, struct.pack(">2IBBB", H, W, int(frame["N"]), _PRECISIONS.index(frame["precision"]), len(coded))]
+        out = [_MAGIC_V3 if "y_streams" in frame else _MAGIC_V2, struct.pack(">2IBBB", H, W, int(frame["N"]), _PRECISIONS.index(frame["precision"]), len(coded))]
     for name, enc in coded.items():
         head = struct.pack(">4s", name.encode()[:4].ljust(4))
         if frame is not None:
@@ -409,12 +482,12 @@ def pack_frame(coded, frame=None):
 
 def unpack_frame(data):
     """Inverse of pack_frame -> {name: {"strings": [[bytes, ...], ...], "shape": (h, w)}}; a version-2 container adds
-    "cluster" to every coder and "frame": {"size": (H, W), "N": N, "precision": "exact" | "mixed"}.  A truncated or
-    malformed container raises RuntimeError."""
+    "cluster" to every coder and "frame": {"size": (H, W), "N": N, "precision": "exact" | "mixed"}; a version-3 container
+    returns the same plus frame["y_streams"] = "rows".  A truncated or malformed container raises RuntimeError."""
     import struct
-    if data[:4] not in (_MAGIC, _MAGIC_V2):
+    if data[:4] not in (_MAGIC, _MAGIC_V2, _MAGIC_V3):
         raise RuntimeError("unpack_frame: not a tdvc_b200 frame container")
-    v2 = data[:4] == _MAGIC_V2
+    v2 = data[:4] in (_MAGIC_V2, _MAGIC_V3)
     pos = 4
     out = {}
     try:
@@ -460,4 +533,6 @@ def unpack_frame(data):
         raise RuntimeError("unpack_frame: trailing bytes")
     if v2:
         out["frame"] = frame
+        if data[:4] == _MAGIC_V3:
+            frame["y_streams"] = "rows"
     return out

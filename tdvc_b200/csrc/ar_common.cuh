@@ -133,7 +133,7 @@ __host__ __device__ __forceinline__ void ar_tap(int ti, int& dy, int& dx) {
 }
 
 // ---- the rANS stream (ryg_rans rans64 + compressai's bypass escape): written by tdvc_rans_encode_with_indexes, read by
-// tdvc_rans_decode_with_indexes on the host and by ar_decode_kernel on the device
+// tdvc_rans_decode_with_indexes on the host and by ar_decode_kernel and ar_code_kernel<ArRowDev> on the device
 constexpr uint64_t RANS64_L = 1ull << 31;   // lower bound of the 64-bit state
 constexpr int RANS_PRECISION = 16, RANS_BYPASS = 4;
 constexpr uint32_t RANS_MAX_BYPASS = (1u << RANS_BYPASS) - 1;
@@ -168,6 +168,68 @@ __host__ __device__ __forceinline__ bool rans_symbol(int s, int max_value, int32
   if (value < INT32_MIN || value > INT32_MAX) return false;
   sym = (int32_t)value;
   return true;
+}
+
+// ---- the device rANS reader of ar_decode_kernel (one string per image) and ar_code_kernel's decode instantiation (one
+// string per latent row)
+
+// a rANS decoder state held identically by the 32 lanes of the decoding warp; a window of 32 stream words (lane j holds
+// word win + j) keeps the renormalisation reads off the L2 latency.  win = -64: nothing loaded yet.
+struct ArdRans {
+  const uint32_t* words;
+  int64_t nw, pos, win;
+  uint32_t wword;
+  uint64_t x;
+
+  __device__ __forceinline__ bool next(uint32_t& v) {
+    if (pos >= nw) return false;
+    if (pos >= win + 32) {
+      win = pos;
+      const int64_t j = pos + (threadIdx.x & 31);
+      wword = j < nw ? __ldg(words + j) : 0u;
+    }
+    v = __shfl_sync(0xffffffffu, wword, (int)(pos - win));
+    ++pos;
+    return true;
+  }
+  __device__ __forceinline__ bool renorm() {
+    if (x < RANS64_L) {
+      uint32_t v;
+      if (!next(v)) return false;
+      x = (x << 32) | v;
+    }
+    return true;
+  }
+  __device__ __forceinline__ bool bits(uint32_t& v) {
+    v = (uint32_t)(x & RANS_MAX_BYPASS);
+    x >>= RANS_BYPASS;
+    return renorm();
+  }
+};
+
+// One symbol of compressai `RansDecoder::decode_with_indexes` (the host version: tdvc_rans_decode_with_indexes), called
+// by all 32 lanes of a warp with the same arguments.  cdf(j) = entry j of the symbol's CDF row of `len` entries.  The host's
+// linear CDF scan becomes a 32-ary search: <= 3 rounds of one shared-memory load and one ballot for a 3,133-entry row.
+// false: corrupt or truncated stream.
+template <class Cdf>
+__device__ __forceinline__ bool ard_decode_symbol(ArdRans& r, Cdf cdf, int len, int32_t offset, int32_t& sym) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t cum = (uint32_t)(r.x & ((1u << RANS_PRECISION) - 1));
+  if (cdf(len - 1) <= cum) return false;
+  int lo = 0, hi = len - 1;   // the symbol s = max{j < len - 1 : cdf[j] <= cum} lies in [lo, hi)
+  while (hi - lo > 1) {
+    const int stride = (hi - lo + 31) >> 5;
+    const int j = lo + lane * stride;
+    const unsigned b = __ballot_sync(0xffffffffu, j < hi && cdf(j) <= cum);
+    const int cnt = __popc(b);
+    if (cnt == 0) return false;   // not a CDF row (cdf[0] must be 0)
+    lo += (cnt - 1) * stride;
+    if (lo + stride < hi) hi = lo + stride;
+  }
+  const int s = lo;
+  const uint32_t start = cdf(s), freq = cdf(s + 1) - cdf(s);
+  r.x = (uint64_t)freq * (r.x >> RANS_PRECISION) + (r.x & ((1u << RANS_PRECISION) - 1)) - start;
+  return r.renorm() && rans_symbol(s, len - 2, offset, [&](uint32_t& v) { return r.bits(v); }, sym);
 }
 
 // ---- host side of tdvc_ar_code and tdvc_ar_decode

@@ -30,63 +30,6 @@ constexpr int ARD_IN_MAX = 512;      // widest layer input (ep0: params | ctx)
 constexpr size_t ARD_SMEM = (size_t)ARD_CDF_MAX * sizeof(int32_t);
 constexpr int64_t ARD_BAD_TABLES = -2;   // status: the CDF tables are not valid rows
 
-// the rANS decoder state of one image, held identically by the 32 lanes of the decoding warp; a window of 32 stream words
-// (lane j holds word win + j) keeps the renormalisation reads off the L2 latency
-struct ArdRans {
-  const uint32_t* words;
-  int64_t nw, pos, win;
-  uint32_t wword;
-  uint64_t x;
-
-  __device__ __forceinline__ bool next(uint32_t& v) {
-    if (pos >= nw) return false;
-    if (pos >= win + 32) {
-      win = pos;
-      const int64_t j = pos + (threadIdx.x & 31);
-      wword = j < nw ? __ldg(words + j) : 0u;
-    }
-    v = __shfl_sync(0xffffffffu, wword, (int)(pos - win));
-    ++pos;
-    return true;
-  }
-  __device__ __forceinline__ bool renorm() {
-    if (x < RANS64_L) {
-      uint32_t v;
-      if (!next(v)) return false;
-      x = (x << 32) | v;
-    }
-    return true;
-  }
-  __device__ __forceinline__ bool bits(uint32_t& v) {
-    v = (uint32_t)(x & RANS_MAX_BYPASS);
-    x >>= RANS_BYPASS;
-    return renorm();
-  }
-};
-
-// One symbol of compressai `RansDecoder::decode_with_indexes` (the host version: tdvc_rans_decode_with_indexes), called
-// by all 32 lanes of a warp with the same arguments.  The host's linear CDF scan becomes a 32-ary search: <= 3 rounds of
-// one shared-memory load and one ballot for a 3,133-entry row.  false: corrupt or truncated stream.
-__device__ __forceinline__ bool ard_decode_symbol(ArdRans& r, const int32_t* cdf, int len, int32_t offset, int32_t& sym) {
-  const int lane = threadIdx.x & 31;
-  const uint32_t cum = (uint32_t)(r.x & ((1u << RANS_PRECISION) - 1));
-  if ((uint32_t)cdf[len - 1] <= cum) return false;
-  int lo = 0, hi = len - 1;   // the symbol s = max{j < len - 1 : cdf[j] <= cum} lies in [lo, hi)
-  while (hi - lo > 1) {
-    const int stride = (hi - lo + 31) >> 5;
-    const int j = lo + lane * stride;
-    const unsigned b = __ballot_sync(0xffffffffu, j < hi && (uint32_t)cdf[j] <= cum);
-    const int cnt = __popc(b);
-    if (cnt == 0) return false;   // not a CDF row (cdf[0] must be 0)
-    lo += (cnt - 1) * stride;
-    if (lo + stride < hi) hi = lo + stride;
-  }
-  const int s = lo;
-  const uint32_t start = (uint32_t)cdf[s], freq = (uint32_t)(cdf[s + 1] - cdf[s]);
-  r.x = (uint64_t)freq * (r.x >> RANS_PRECISION) + (r.x & ((1u << RANS_PRECISION) - 1)) - start;
-  return r.renorm() && rans_symbol(s, len - 2, offset, [&](uint32_t& v) { return r.bits(v); }, sym);
-}
-
 // split partials of this CTA's outputs of layer w for one position: part[ks][nl] = the encoder's fmaf chain of split ks of
 // output nl; in(k) = float4 of the layer input at k .. k + 3 (shared memory)
 template <class In>
@@ -261,8 +204,9 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const TdvcArDe
       int bad = -1;
       for (int c = 0; c < C; ++c) {
         const int t = s_idx[c];
+        const int32_t* row = ard_cdf + s_row[t];
         int32_t v;
-        if (!ard_decode_symbol(rs, ard_cdf + s_row[t], s_len[t], s_off[t], v)) {
+        if (!ard_decode_symbol(rs, [&](int j) { return (uint32_t)row[j]; }, s_len[t], s_off[t], v)) {
           bad = c;
           break;
         }

@@ -15,6 +15,7 @@
 #include <cooperative_groups.h>
 #include <stdlib.h>
 #include <string.h>
+#include <type_traits>
 #include <vector>
 #include "ar_common.cuh"
 
@@ -32,6 +33,29 @@ struct ArDev {
   float* h1_s;    // [N][AR_PCH][c1_pad]
   float* h2_s;    // [N][AR_PCH][c2_pad]
   unsigned long long* dbg;   // developer timing (TDVC_B200_AR_DEBUG): ns per phase, summed over the wavefronts by CTA 0
+};
+
+// The decode instantiation of ar_code_kernel (row streams, tdvc_ar_decode_rows): the encoder's members first, under the
+// same names, then the decoder's.
+// Beside the encoder's AR_SMEM of dynamic shared memory, every CTA holds the Gaussian CDF rows as uint16 (each entry but a
+// row's last is below 2^16, the last one, 2^16, is implied by the row length) and the rows' starts, lengths and offsets:
+// 176,128 + 54,784 + 784 bytes, with the 256 static bytes of the scale table within the 232,448 a block may opt in to.  The
+// staging depth stays AR_NBUF = 3.
+constexpr int ARR_CDF_MAX = 27392;   // CDF entries (64 Gaussian rows: 27,256)
+constexpr int ARR_TABLES_MAX = 64;
+constexpr size_t ARR_SMEM = AR_SMEM + (size_t)ARR_CDF_MAX * sizeof(uint16_t) + (3 * ARR_TABLES_MAX + 4) * sizeof(int);
+constexpr unsigned long long ARR_NO_FAIL = ~0ull;
+struct ArRowDev {
+  TdvcArRowDecodeParams a;
+  float* ctx_s;
+  float* h1_s;
+  float* h2_s;
+  unsigned long long* dbg;
+  float* mean_s;               // [N][AR_PCH][C]: means of the chunk's positions (ep4 -> the decoding warps)
+  int32_t* idx_s;              // [N][AR_PCH][C]: their scale indexes
+  unsigned long long* row_x;   // [N][H]: rANS state of each row between its positions
+  long long* row_pos;          // [N][H]: next word of each row
+  unsigned long long* fail;    // [N]: lowest (h * W + w) * C + c that failed, ARR_NO_FAIL
 };
 
 __device__ __forceinline__ unsigned long long ar_now() {
@@ -179,7 +203,94 @@ __device__ __forceinline__ void ar_prefetch_w(const ArW& w, float* sW) {
   cp_async_commit();
 }
 
-__global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
+// lowest latent row of image n that failed to decode (H: none), as every thread of the cluster reads it after a barrier
+__device__ __forceinline__ int arr_live_rows(const ArRowDev& d, int n, int H, int W) {
+  const unsigned long long f = *(volatile const unsigned long long*)(d.fail + n);
+  return f == ARR_NO_FAIL ? H : (int)(f / ((unsigned long long)W * AR_C));
+}
+
+// The symbol step of the row-stream decoder: the calling warp decodes the 128 symbols of position (h, w) from row h's
+// stream, with the means and scale indexes ep4 left in row p of the chunk workspace, and writes symbol, index and
+// y_hat = symbol + mean (the encoder's operation).  The row's rANS state is resumed from / saved to the workspace; at
+// w = W - 1 the row must end in the encoder's initial state (x = RANS64_L, every word consumed).  A failure records
+// (h * W + w) * C + c in d.fail[n] (the lowest one wins) and writes nothing.
+__device__ __forceinline__ void arr_decode_position(const ArRowDev& d, int n, int h, int w, int p, float* red,
+                                                    const uint16_t* cdf, const int* s_row, const int* s_len,
+                                                    const int* s_off) {
+  constexpr int C = AR_C;
+  const TdvcArChain& a = d.a.chain;
+  const int H = a.H, W = a.W;
+  const int lane = threadIdx.x & 31;
+  if (h >= arr_live_rows(d, n, H, W)) return;   // a row at or below a failed one
+  const int64_t row = (int64_t)n * H + h;
+  const int64_t w0 = d.a.word_offsets[row];
+  ArdRans rs;
+  rs.words = d.a.words + w0;
+  rs.nw = d.a.word_offsets[row + 1] - w0;
+  rs.win = -64;
+  rs.wword = 0u;
+  int bad = -1;
+  if (w == 0) {
+    rs.pos = 2;
+    rs.x = 0;
+    if (rs.nw >= 2) rs.x = (uint64_t)__ldg(rs.words) | ((uint64_t)__ldg(rs.words + 1) << 32);
+    else bad = 0;
+  } else {
+    rs.x = __ldcg(d.row_x + row);
+    rs.pos = __ldcg(d.row_pos + row);
+  }
+  // the position's means and indexes, written by every CTA of the cluster, into this warp's tile of the reduction area
+  // (free between the ep4 sums and the next chunk's first stage): one L2 round trip for the 128 channels
+  float* s_mean = red + (threadIdx.x >> 5) * AR_PT * 32;
+  int32_t* s_ix = reinterpret_cast<int32_t*>(s_mean + C);
+  const float* mrow = d.mean_s + ((int64_t)n * AR_PCH + p) * C;
+  const int32_t* irow = d.idx_s + ((int64_t)n * AR_PCH + p) * C;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    s_mean[32 * k + lane] = __ldcg(mrow + 32 * k + lane);
+    s_ix[32 * k + lane] = __ldcg(irow + 32 * k + lane);
+  }
+  __syncwarp();
+  int32_t sv[4] = {0, 0, 0, 0};   // lane l: the symbols of channels l, l + 32, l + 64, l + 96
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    for (int j = 0; j < 32 && bad < 0; ++j) {
+      const int t = s_ix[32 * k + j];
+      const uint16_t* crow = cdf + s_row[t];
+      const int len = s_len[t];
+      // the last entry of every row is 2^16, implied by the row length
+      auto entry = [&](int e) -> uint32_t { return e == len - 1 ? (1u << RANS_PRECISION) : (uint32_t)crow[e]; };
+      int32_t v;
+      if (!ard_decode_symbol(rs, entry, len, s_off[t], v)) bad = 32 * k + j;
+      else if (lane == j) sv[k] = v;
+    }
+  }
+  if (bad < 0 && w == W - 1 && !(rs.x == RANS64_L && rs.pos == rs.nw)) bad = C - 1;
+  if (bad < 0) {
+    const int64_t o = (row * W + w) * C;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int c = 32 * k + lane;
+      a.symbols[o + c] = sv[k];
+      a.indexes[o + c] = s_ix[c];
+      a.y_hat[o + c] = __fadd_rn((float)sv[k], s_mean[c]);
+    }
+    if (lane == 0) {
+      d.row_x[row] = rs.x;
+      d.row_pos[row] = rs.pos;
+    }
+  } else if (lane == 0) {
+    atomicMin(d.fail + n, ((unsigned long long)h * W + w) * C + bad);
+  }
+}
+
+// Dev = ArDev: the encoder (tdvc_ar_code).  Dev = ArRowDev: the decoder of row streams (tdvc_ar_decode_rows), the same
+// loop - chunks, staging, K splits, sums, bias and activations, so the same means and scale indexes - except for the ep4
+// epilogue: the means and indexes go to the chunk workspace, and after one more cluster barrier warp p % 16 of CTA p / 16
+// decodes position p of the chunk from its row's stream (the symbol step), then the usual barrier publishes its y_hat.
+template <class Dev>
+__global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const Dev d) {
+  constexpr bool DECODE = std::is_same<Dev, ArRowDev>::value;
   cg::cluster_group cluster = cg::this_cluster();
   const int R = (int)cluster.num_blocks();
   const int rank = (int)cluster.block_rank();
@@ -197,7 +308,8 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   const int n_cmp = a.n_scales - 1;
 
   float* yhat = a.y_hat + (int64_t)n * H * W * C;
-  const float* y = d.a.y + (int64_t)n * H * W * d.a.y_ld;
+  const float* y = nullptr;
+  if constexpr (!DECODE) y = d.a.y + (int64_t)n * H * W * d.a.y_ld;
   const float* prm = a.params + (int64_t)n * H * W * a.params_ld;
   float* ctx_s = d.ctx_s + (int64_t)n * AR_PCH * C2;
   float* h1_s = d.h1_s + (int64_t)n * AR_PCH * a.c1_pad;
@@ -208,10 +320,53 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
   const ArW wA = ar_layer(a, AR_CTX, rank, R), wB = ar_layer(a, AR_EP0, rank, R), wC = ar_layer(a, AR_EP2, rank, R),
             wD = ar_layer(a, AR_EP4, rank, R);
 
+  // decoder: the CDF rows as uint16 after the reduction tile, then their row starts, lengths and offsets
+  uint16_t* s_cdf = reinterpret_cast<uint16_t*>(red + AR_WARPS * AR_PT * 32);
+  int* s_row = reinterpret_cast<int*>(s_cdf + ARR_CDF_MAX);
+  int* s_len = s_row + ARR_TABLES_MAX;
+  int* s_off = s_len + ARR_TABLES_MAX;
+  if constexpr (DECODE) {
+    // every CTA loads and checks the tables itself, so all of them reach the same verdict without a barrier
+    const TdvcArRowDecodeParams& q = d.a;
+    if (threadIdx.x == 0) {
+      int total = 0;
+      bool ok = true;
+      for (int i = 0; i < q.n_tables; ++i) {
+        const int len = q.cdf_lengths[i];
+        ok = ok && len >= 2 && len <= q.cdf_stride;
+        s_row[i] = total;
+        s_len[i] = len;
+        s_off[i] = q.cdf_offsets[i];
+        total += ok ? len : 0;
+      }
+      s_off[ARR_TABLES_MAX] = ok && total == q.cdf_total;
+    }
+    __syncthreads();
+    bool ok = s_off[ARR_TABLES_MAX] != 0;
+    if (ok) {
+      for (int i = 0; i < q.n_tables; ++i) {
+        const int len = s_len[i];
+        for (int e = threadIdx.x; e < len; e += AR_THREADS) {
+          const int32_t v = q.cdfs[(int64_t)i * q.cdf_stride + e];
+          ok = ok && (e < len - 1 ? v >= 0 && v < (1 << RANS_PRECISION) : v == (1 << RANS_PRECISION));
+          s_cdf[s_row[i] + e] = (uint16_t)v;
+        }
+      }
+    }
+    if (!__syncthreads_and(ok)) {
+      if (rank == 0 && threadIdx.x == 0) q.status[n] = -2;
+      return;
+    }
+  }
+
   ar_prefetch_w(wA, sW);
   unsigned long long t_last = d.dbg != nullptr ? ar_now() : 0ull;
   const int waves = W + 3 * (H - 1);
   for (int t = 0; t < waves; ++t) {
+    if constexpr (DECODE) {
+      // every row above the first failed one is complete (read after a barrier: all CTAs of the cluster agree)
+      if (t > W - 1 + 3 * (arr_live_rows(d, n, H, W) - 1)) break;
+    }
     int h_lo, h_hi;
     ar_wave_rows(t, H, W, h_lo, h_hi);
     for (int hc = h_lo; hc <= h_hi; hc += AR_PCH) {
@@ -288,18 +443,38 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const ArDev d) {
           const int ch = ch0 + j;
           const float scale = ar_sum(red, KS, P, p, j) + __ldg(a.b3 + ch);
           const float mean = ar_sum(red, KS, P, p, nch + j) + __ldg(a.b3 + C + ch);
-          const int hh = hc + p, ww = t - 3 * hh;
-          const int64_t pix = (int64_t)hh * W + ww;
-          const float q = rintf(__fsub_rn(__ldg(y + pix * d.a.y_ld + ch), mean));
-          yhat[pix * C + ch] = __fadd_rn(q, mean);
-          sym[pix * C + ch] = (int32_t)q;
-          idx[pix * C + ch] = ar_scale_index(scale, s_table, n_cmp);
+          if constexpr (DECODE) {
+            d.mean_s[((int64_t)n * AR_PCH + p) * C + ch] = mean;
+            d.idx_s[((int64_t)n * AR_PCH + p) * C + ch] = ar_scale_index(scale, s_table, n_cmp);
+          } else {
+            const int hh = hc + p, ww = t - 3 * hh;
+            const int64_t pix = (int64_t)hh * W + ww;
+            const float q = rintf(__fsub_rn(__ldg(y + pix * d.a.y_ld + ch), mean));
+            yhat[pix * C + ch] = __fadd_rn(q, mean);
+            sym[pix * C + ch] = (int32_t)q;
+            idx[pix * C + ch] = ar_scale_index(scale, s_table, n_cmp);
+          }
         }
       }
       AR_MARK(10);
       __threadfence();
       cluster.sync();
       AR_MARK(11);
+      if constexpr (DECODE) {
+        // ---- symbol step: position p of the chunk, one warp each (P <= AR_PCH <= 8 CTAs x AR_WARPS)
+        const int p = rank * AR_WARPS + (threadIdx.x >> 5);
+        if (p < P) arr_decode_position(d, n, hc + p, t - 3 * (hc + p), p, red, s_cdf, s_row, s_len, s_off);
+        AR_MARK(12);
+        __threadfence();
+        cluster.sync();
+        AR_MARK(13);
+      }
+    }
+  }
+  if constexpr (DECODE) {
+    if (rank == 0 && threadIdx.x == 0) {
+      const unsigned long long f = *(volatile const unsigned long long*)(d.fail + n);
+      d.a.status[n] = f == ARR_NO_FAIL ? -1 : (int64_t)f;
     }
   }
   cp_async_wait<0>();
@@ -319,6 +494,25 @@ extern "C" size_t tdvc_ar_code_workspace_bytes(int N, int c1_pad, int c2_pad) {
   if (N <= 0 || c1_pad <= 0 || c2_pad <= 0) return 0;
   return (size_t)N * AR_PCH * (size_t)(2 * AR_C + c1_pad + c2_pad) * sizeof(float);
 }
+
+// developer timing (TDVC_B200_AR_DEBUG): a zeroed per-phase buffer, or nullptr when the variable is unset
+static unsigned long long* ar_debug_buffer(cudaStream_t st) {
+  static unsigned long long* dbg_buf = nullptr;
+  if (getenv("TDVC_B200_AR_DEBUG") == nullptr) return nullptr;
+  if (dbg_buf == nullptr) cudaMalloc(&dbg_buf, 16 * sizeof(unsigned long long));
+  cudaMemsetAsync(dbg_buf, 0, 16 * sizeof(unsigned long long), st);
+  return dbg_buf;
+}
+static void ar_debug_report(const unsigned long long* dbg, const char* who, int R, const char* const* names, int n,
+                            cudaStream_t st) {
+  unsigned long long h[16];
+  cudaStreamSynchronize(st);
+  cudaMemcpy(h, dbg, sizeof(h), cudaMemcpyDeviceToHost);
+  for (int i = 0; i < n; ++i) fprintf(stderr, "%s[R=%d] %-16s %8.3f ms\n", who, R, names[i], h[i] * 1e-6);
+}
+static const char* const AR_PHASES[14] = {"A chunks", "A sums", "A fence+barrier", "B chunks", "B sums", "B fence+barrier",
+                                          "C chunks", "C sums", "C fence+barrier", "D chunks", "D sums", "D fence+barrier",
+                                          "symbols", "S fence+barrier"};
 
 extern "C" int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t workspace_bytes, void* stream) {
   TDVC_REQUIRE(p != nullptr, "ar_code: null params");
@@ -342,25 +536,58 @@ extern "C" int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t works
   d.ctx_s = (float*)workspace;
   d.h1_s = d.ctx_s + (size_t)a.N * AR_PCH * 2 * AR_C;
   d.h2_s = d.h1_s + (size_t)a.N * AR_PCH * a.c1_pad;
-  d.dbg = nullptr;
-  static unsigned long long* dbg_buf = nullptr;
-  const bool debug = getenv("TDVC_B200_AR_DEBUG") != nullptr;
-  if (debug) {
-    if (dbg_buf == nullptr) cudaMalloc(&dbg_buf, 16 * sizeof(unsigned long long));
-    cudaMemsetAsync(dbg_buf, 0, 16 * sizeof(unsigned long long), st);
-    d.dbg = dbg_buf;
-  }
-  const int lrc = ar_launch_clusters<ar_code_kernel>(d, a.N, R, auto_r, AR_SMEM, st, "ar_code");
+  d.dbg = ar_debug_buffer(st);
+  const int lrc = ar_launch_clusters<ar_code_kernel<ArDev>>(d, a.N, R, auto_r, AR_SMEM, st, "ar_code");
   if (lrc != TDVC_OK) return lrc;
   if (p->cluster_used_host != nullptr) *p->cluster_used_host = R;
-  if (debug) {
-    unsigned long long h[16];
-    cudaStreamSynchronize(st);
-    cudaMemcpy(h, dbg_buf, sizeof(h), cudaMemcpyDeviceToHost);
-    static const char* nm[12] = {"A chunks", "A sums", "A fence+barrier", "B chunks", "B sums", "B fence+barrier",
-                                 "C chunks", "C sums", "C fence+barrier", "D chunks", "D sums", "D fence+barrier"};
-    for (int i = 0; i < 12; ++i) fprintf(stderr, "ar_code[R=%d] %-16s %8.3f ms\n", R, nm[i], h[i] * 1e-6);
+  if (d.dbg != nullptr) ar_debug_report(d.dbg, "ar_code", R, AR_PHASES, 12, st);
+  return TDVC_OK;
+}
+
+extern "C" size_t tdvc_ar_decode_rows_workspace_bytes(int N, int H, int c1_pad, int c2_pad) {
+  const size_t chain = tdvc_ar_code_workspace_bytes(N, c1_pad, c2_pad);
+  if (chain == 0 || H <= 0) return 0;
+  return chain + (size_t)N * AR_PCH * AR_C * (sizeof(float) + sizeof(int32_t)) + (size_t)N * H * 16 + (size_t)N * 8;
+}
+
+extern "C" int tdvc_ar_decode_rows(const TdvcArRowDecodeParams* p, void* workspace, size_t workspace_bytes, void* stream) {
+  TDVC_REQUIRE(p != nullptr, "ar_decode_rows: null params");
+  const int rc = ar_check_chain(p->chain, "ar_decode_rows");
+  if (rc != TDVC_OK) return rc;
+  const TdvcArChain& a = p->chain;
+  TDVC_REQUIRE(p->words && p->word_offsets && p->cdfs && p->cdf_lengths && p->cdf_offsets && p->status,
+               "ar_decode_rows: null pointer");
+  TDVC_REQUIRE(p->n_tables >= a.n_scales && p->n_tables <= ARR_TABLES_MAX && p->cdf_stride >= 3,
+               "ar_decode_rows: %d tables for %d scales", p->n_tables, a.n_scales);
+  TDVC_REQUIRE(p->cdf_total > 0 && p->cdf_total <= ARR_CDF_MAX, "ar_decode_rows: %d CDF entries (at most %d)", p->cdf_total,
+               ARR_CDF_MAX);
+  TDVC_REQUIRE(p->cluster == 8 || p->cluster == 16, "ar_decode_rows: encoder cluster size %d (8 or 16)", p->cluster);
+  const size_t chain = tdvc_ar_code_workspace_bytes(a.N, a.c1_pad, a.c2_pad);
+  const size_t need = tdvc_ar_decode_rows_workspace_bytes(a.N, a.H, a.c1_pad, a.c2_pad);
+  TDVC_REQUIRE(workspace != nullptr && workspace_bytes >= need, "ar_decode_rows: workspace of %zu bytes, %zu needed",
+               workspace_bytes, need);
+  cudaStream_t st = (cudaStream_t)stream;
+  ArRowDev d;
+  d.a = *p;
+  d.ctx_s = (float*)workspace;
+  d.h1_s = d.ctx_s + (size_t)a.N * AR_PCH * 2 * AR_C;
+  d.h2_s = d.h1_s + (size_t)a.N * AR_PCH * a.c1_pad;
+  d.mean_s = (float*)((char*)workspace + chain);
+  d.idx_s = (int32_t*)(d.mean_s + (size_t)a.N * AR_PCH * AR_C);
+  d.row_x = (unsigned long long*)(d.idx_s + (size_t)a.N * AR_PCH * AR_C);
+  d.row_pos = (long long*)(d.row_x + (size_t)a.N * a.H);
+  d.fail = (unsigned long long*)(d.row_pos + (size_t)a.N * a.H);
+  // as in ar_code: finite numbers in the padded tail of the hidden rows; and no failure yet
+  if (cudaMemsetAsync(workspace, 0, chain, st) != cudaSuccess ||
+      cudaMemsetAsync(d.fail, 0xff, (size_t)a.N * sizeof(unsigned long long), st) != cudaSuccess) {
+    set_error("ar_decode_rows: cudaMemsetAsync failed");
+    return TDVC_ECUDA;
   }
+  d.dbg = ar_debug_buffer(st);
+  int R = p->cluster;   // the encoder's: its K splits are the summation order to reproduce
+  const int lrc = ar_launch_clusters<ar_code_kernel<ArRowDev>>(d, a.N, R, false, ARR_SMEM, st, "ar_decode_rows");
+  if (lrc != TDVC_OK) return lrc;
+  if (d.dbg != nullptr) ar_debug_report(d.dbg, "ar_decode_rows", R, AR_PHASES, 14, st);
   return TDVC_OK;
 }
 

@@ -117,17 +117,18 @@ def code_gop(net, i_frame, p_frames, enable_amp=False, keep_recon=False, with_ms
     return out
 
 
-def compress_gop(net, i_frame, p_frames, enable_amp=False):
+def compress_gop(net, i_frame, p_frames, enable_amp=False, row_streams=False):
     """Closed-loop coding of one GOP with `VideoCompressor.compress`: each frame's reconstruction - the frame the decoder
     rebuilds - is the next frame's reference, so encoder and decoder never drift apart.  i_frame (1,3,h,w): the (decoded)
     I-frame; p_frames (T,3,h,w).  Frames are padded to multiples of 64 and cropped back as in `code_gop`.
-    Returns (containers: one version-2 container (bytes) per P-frame, recon: the cropped reconstructions)."""
+    Returns (containers: one version-2 container (bytes) per P-frame, recon: the cropped reconstructions).
+    row_streams: version-3 containers (`VideoCompressor.compress(..., row_streams=True)`); decompress_gop reads either."""
     T, _, h, w = p_frames.shape
     refs = RefBuffer(pad(i_frame, 64))
     containers, recons = [], []
     for i in range(T):
         window, keys = refs.window()
-        recon, data = net.compress(pad(p_frames[i:i + 1], 64), window, enable_amp, ref_keys=keys)
+        recon, data = net.compress(pad(p_frames[i:i + 1], 64), window, enable_amp, ref_keys=keys, row_streams=row_streams)
         refs.push(recon)
         containers.append(data)
         recons.append(crop(recon, (h, w)))

@@ -1624,13 +1624,16 @@ class VideoCompressor(nn.Module):
         return out
 
     @staticmethod
-    def _finish_coding(pending, num_pixels, taps=None):
-        """Host half of coding, in the order given: [(name, launch_coding handle), ...] -> `last_coded`."""
+    def _finish_coding(pending, num_pixels, taps=None, rows=False):
+        """Host half of coding, in the order given: [(name, launch_coding handle), ...] -> `last_coded`.  rows: y as row
+        streams (coding.finish_coding); ac_bpp then counts image 0's y row strings and its z string, as the reference's
+        len(s[0]) counts image 0's string of each list."""
         from tdvc_b200 import coding
         out = {}
         for nm, h in pending:
-            enc = coding.finish_coding(h, keep=taps is not None)
-            enc["ac_bpp"] = sum(len(s[0]) for s in enc["strings"]) * 8.0 / num_pixels
+            enc = coding.finish_coding(h, keep=taps is not None, rows=rows)
+            hy = len(enc["strings"][0]) // len(enc["strings"][1]) if rows else 1
+            enc["ac_bpp"] = (sum(len(s_) for s_ in enc["strings"][0][:hy]) + len(enc["strings"][1][0])) * 8.0 / num_pixels
             if taps is not None:
                 for k in ("y_symbols", "y_indexes", "y_hat", "z_symbols"):
                     taps[f"{nm}.ac.{k}"] = enc.pop(k)
@@ -1652,8 +1655,11 @@ class VideoCompressor(nn.Module):
             smod.gaussian_conditional.scale_table = tabs[cn].scale_table.clone()
         return tabs[cn]
 
-    def compress(self, input_image, refer_frames, enabled_amp=False, ref_keys=None, taps=None):
+    def compress(self, input_image, refer_frames, enabled_amp=False, ref_keys=None, taps=None, row_streams=False):
         """Closed-loop encoder of one P-frame: -> (recon (N,3,H,W) fp32, data: the version-2 container's bytes).
+        row_streams: write a version-3 container instead, whose y strings are one rANS stream per latent row (this
+        project's own format, about 12 bytes more per extra row and coder; compressai cannot read it), which `decompress`
+        decodes wavefront by wavefront on the device.  The device pass, the symbols, y_hat and recon are the same.
         Unlike `forward`, both coders' syntheses run on the y_hat the strings carry (quantised relative to the predicted
         mean, round(y - mu) + mu), so `recon` is the frame `decompress(data, refer_frames)` rebuilds bit for bit; the
         prediction and the residual are computed from the decoded motion.  A GOP feeds this recon to the next frame
@@ -1682,8 +1688,11 @@ class VideoCompressor(nn.Module):
             recon, handles = plan.compress(Wt, tables, x, refs, cache=self.cache_features, ref_keys=ref_keys, taps=taps)
             recon = recon.clone()
             # the host codes the motion strings while the residual half of the frame is still running on the device
-            self.last_coded = self._finish_coding(list(handles.items()), N * H * W, taps)
-        return recon, coding.pack_frame(self.last_coded, frame={"size": (H, W), "N": N, "precision": plan.precision})
+            self.last_coded = self._finish_coding(list(handles.items()), N * H * W, taps, rows=row_streams)
+        frame = {"size": (H, W), "N": N, "precision": plan.precision}
+        if row_streams:
+            frame["y_streams"] = "rows"
+        return recon, coding.pack_frame(self.last_coded, frame=frame)
 
     def decompress(self, data, refer_frames, ref_keys=None, taps=None):
         """Decoder of one P-frame: a version-2 container (`compress`) and the same refer_frames (N,4,3,H,W) the encoder
@@ -1749,8 +1758,9 @@ class VideoCompressor(nn.Module):
 
     @staticmethod
     def _container(data, who):
-        """Unpack a container and check, on the host, that it can be decoded: version 2, both coders, a frame size of
-        multiples of 64, hyper-latent shapes that fit it, two string lists of N per coder.  -> the unpacked container."""
+        """Unpack a container and check, on the host, that it can be decoded: version 2 or 3, both coders, a frame size of
+        multiples of 64, hyper-latent shapes that fit it, two string lists per coder: N y strings (version 3: N * H / 16
+        row strings) and N z strings.  -> the unpacked container."""
         from tdvc_b200 import coding
         box = coding.unpack_frame(data)
         frame = box.get("frame")
@@ -1767,9 +1777,15 @@ class VideoCompressor(nn.Module):
             if tuple(enc["shape"]) != (H // 64, Wd // 64):
                 raise RuntimeError(f"{who}: {nm} hyper-latent shape {tuple(enc['shape'])} for a {H}x{Wd} "
                                    f"frame (expected {(H // 64, Wd // 64)})")
-            if len(enc["strings"]) != 2 or any(len(lst) != N for lst in enc["strings"]):
+            ny = N * (H // 16) if frame.get("y_streams") == "rows" else N
+            if len(enc["strings"]) != 2 or [len(lst) for lst in enc["strings"]] != [ny, N]:
                 raise RuntimeError(f"{who}: {nm} has {[len(lst) for lst in enc['strings']]} strings (two "
-                                   f"lists, y and z, of {N})")
+                                   f"lists, y and z, of {ny} and {N})")
+            if frame.get("y_streams") == "rows":
+                for i, s_ in enumerate(enc["strings"][0]):
+                    if len(s_) < 8 or len(s_) % 4:
+                        raise RuntimeError(f"{who}: {nm} y row {i % (H // 16)} of image {i // (H // 16)} has {len(s_)} "
+                                           "bytes (rANS strings are whole 32-bit words, at least two)")
         return box
 
     def _decoder_device(self):
@@ -1800,7 +1816,8 @@ class VideoCompressor(nn.Module):
                 coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
                 params = plan.hyper_synthesis(Wt, cn, zh, b)
             # the motion chain is already decoding on the device while the host decodes the residual z strings
-            h = coding.launch_decoding(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream)
+            launch = coding.launch_decoding_rows if box["frame"].get("y_streams") == "rows" else coding.launch_decoding
+            h = launch(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream)
             pending.append((nm, zh, h))
         main.wait_stream(side)
         out = {}

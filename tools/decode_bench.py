@@ -11,7 +11,11 @@ it, so the overlap of the two coders' chains can be read off.
 included) and `VideoCompressor.decompress` of its container by a second module (container to reconstruction), each with a
 host clock around the call and a device synchronise after it, median of `reps` after a warm-up.  The per-GOP feature caches
 are off, so every frame computes everything a GOP's first P-frame computes; the round trip is checked bit for bit.
-python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}] [--container] [--codec]  ->  one JSON line."""
+--row-streams: also time the row-stream decoder `tdvc_ar_decode_rows` per coder (one rANS string per latent row, decoded
+wavefront by wavefront) in the same loop as `tdvc_ar_code` and `tdvc_ar_decode`; with --codec also
+`compress(row_streams=True)` and `decompress` of its version-3 container, and both containers' sizes.
+python tools/decode_bench.py [reps] [--encoder-cluster {0,8,16}] [--container] [--codec] [--row-streams]  ->  one JSON
+line."""
 import argparse
 import json
 import subprocess
@@ -46,6 +50,7 @@ def main():
     ap.add_argument("--encoder-cluster", type=int, choices=(0, 8, 16), default=16)
     ap.add_argument("--container", action="store_true", help="also time decompress_latents on the frame's container")
     ap.add_argument("--codec", action="store_true", help="also time compress and decompress end to end")
+    ap.add_argument("--row-streams", action="store_true", help="also time the row-stream decoder (container version 3)")
     args = ap.parse_args()
     reps, cl = args.reps, args.encoder_cluster
     dev = torch.device("cuda:0")
@@ -83,39 +88,51 @@ def main():
     for cn in ("mv", "rs"):
         tabs = W["_tables"][cn]
         params = plan.buf(f"{cn}.params", 1, hy, wy, 256)
-        enc_ms, dec_ms = [], []
+        enc_ms, dec_ms, row_ms = [], [], []
         for rep in range(reps + 1):   # rep 0: warm-up
             t_enc, h = timed(lambda: coding.launch_coding(plan, W, cn, tabs, cluster=cl))
+            hold = dict(h)   # the pinned host symbols stay valid until the next launch_coding
             enc = coding.finish_coding(h, keep=True)
             res["encoder_cluster_used"] = enc["cluster"]
             t_dec, h = timed(lambda: coding.launch_decoding(W, cn, tabs, enc["strings"][0], params, enc["cluster"]))
             dec = coding.finish_decoding(h)
             assert torch.equal(dec["y_hat"], enc["y_hat"]) and torch.equal(dec["y_symbols"], enc["y_symbols"])
+            if args.row_streams:
+                rows = coding.finish_coding(hold, rows=True)["strings"][0]
+                t_row, h = timed(lambda: coding.launch_decoding_rows(W, cn, tabs, rows, params, enc["cluster"]))
+                dec = coding.finish_decoding(h)
+                assert torch.equal(dec["y_hat"], enc["y_hat"]) and torch.equal(dec["y_symbols"], enc["y_symbols"])
             if rep:
                 enc_ms.append(t_enc)
                 dec_ms.append(t_dec)
+                if args.row_streams:
+                    row_ms.append(t_row)
         dec_med = sorted(dec_ms)[len(dec_ms) // 2]
         res[cn] = {"ar_code_ms": round(sorted(enc_ms)[len(enc_ms) // 2], 3), "ar_decode_ms": round(dec_med, 3),
                    "ar_decode_us_per_step": round(1e3 * dec_med / (hy * wy), 3),
                    "ar_decode_ms_all": [round(t, 3) for t in dec_ms]}
+        if args.row_streams:
+            res[cn].update({"ar_decode_rows_ms": round(sorted(row_ms)[len(row_ms) // 2], 3),
+                            "ar_decode_rows_ms_all": [round(t, 3) for t in row_ms]})
     if args.codec:
         enc, dec = (_module(orc, dev, cache=False) for _ in range(2))
         xd, rd = x.to(dev), refs.to(dev)
-        c_ms, d_ms = [], []
-        for rep in range(reps + 1):   # rep 0: warm-up (packs the weights, builds the tables and both plans)
-            torch.cuda.synchronize()
-            t0 = time.perf_counter()
-            recon, data = enc.compress(xd, rd)
-            torch.cuda.synchronize()
-            t1 = time.perf_counter()
-            got = dec.decompress(data, rd)
-            torch.cuda.synchronize()
-            t2 = time.perf_counter()
-            assert torch.equal(got, recon)
-            c_ms.append(1e3 * (t1 - t0))
-            d_ms.append(1e3 * (t2 - t1))
-        c_ms, d_ms = c_ms[1:], d_ms[1:]
-        res["codec"] = {"bytes": len(data), "compress_ms": round(sorted(c_ms)[len(c_ms) // 2], 3),
+        for key, rows in (("codec", False), ("codec_rows", True)) if args.row_streams else (("codec", False),):
+            c_ms, d_ms = [], []
+            for rep in range(reps + 1):   # rep 0: warm-up (packs the weights, builds the tables and both plans)
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                recon, data = enc.compress(xd, rd, row_streams=rows)
+                torch.cuda.synchronize()
+                t1 = time.perf_counter()
+                got = dec.decompress(data, rd)
+                torch.cuda.synchronize()
+                t2 = time.perf_counter()
+                assert torch.equal(got, recon)
+                c_ms.append(1e3 * (t1 - t0))
+                d_ms.append(1e3 * (t2 - t1))
+            c_ms, d_ms = c_ms[1:], d_ms[1:]
+            res[key] = {"bytes": len(data), "compress_ms": round(sorted(c_ms)[len(c_ms) // 2], 3),
                         "decompress_ms": round(sorted(d_ms)[len(d_ms) // 2], 3),
                         "compress_ms_all": [round(t, 3) for t in c_ms], "decompress_ms_all": [round(t, 3) for t in d_ms]}
     print(json.dumps(res))
