@@ -344,18 +344,30 @@ typedef struct TdvcArParams {
   int32_t cluster;
   int32_t* cluster_used_host;
 } TdvcArParams;
-/* ar_decode: the inverse of ar_code (compressai `_decompress_ar`), one thread-block cluster per image walking the latent in
- *   raster order: per position the context model over the already decoded y_hat, the three entropy-parameter layers, then
- *   the 128 symbols of the position from the rANS stream (on the device, compressai's bypass escape included), y_hat =
- *   symbol + mean.  The predictions are bit-identical to ar_code's for the same chain only if ar_code ran with `cluster`
- *   CTAs per image (its K splits, and so its fp32 summation order, depend on it): pass the encoder's cluster size (8 or 16;
- *   a container records it).  All pointers are DEVICE pointers.  `words` / `word_offsets`: the N y strings as 32-bit
- *   little-endian words, string n = words[word_offsets[n] .. word_offsets[n + 1]).  `cdfs` [n_tables][cdf_stride],
- *   `cdf_lengths`, `cdf_offsets`: the Gaussian tables of the rANS coder; cdf_total = sum of cdf_lengths.  Outputs those of
- *   the chain plus `status` [N]: -1 when image n decoded, -2 when the CDF tables are not valid rows (lengths outside
- *   [2, cdf_stride] or not summing to cdf_total; nothing is decoded), else the index (h * W + w) * C + c of the first
- *   symbol that could not be decoded (truncated or corrupt stream; nothing after it is written).  A malformed stream never
- *   faults the kernel: the caller reads `status` after the stream synchronises.                                            */
+/* TdvcArDecodeParams: the arguments of both decoders of y, the inverses of ar_code (compressai `_decompress_ar`).  Their
+ *   predictions are bit-identical to ar_code's for the same chain only if ar_code ran with `cluster` CTAs per image (its K
+ *   splits, and so its fp32 summation order, depend on it): pass the encoder's cluster size (8 or 16; a container records
+ *   it).  All pointers are DEVICE pointers.  `words` / `word_offsets`: the y strings as 32-bit little-endian words, string
+ *   s = words[word_offsets[s] .. word_offsets[s + 1]).  `cdfs` [n_tables][cdf_stride] (n_tables <= 64), `cdf_lengths`,
+ *   `cdf_offsets`: the Gaussian tables of the rANS coder; cdf_total = sum of cdf_lengths.  Outputs those of the chain plus
+ *   `status` [N]: -1 when image n decoded, -2 when the CDF tables are not valid rows (lengths outside [2, cdf_stride] or not
+ *   summing to cdf_total; nothing is decoded), else the index (h * W + w) * C + c of a symbol that could not be decoded
+ *   (what each decoder reports: below).  A malformed stream never faults the kernel: the caller reads `status` after the
+ *   stream synchronises.
+ * ar_decode: one string per image (N strings, word_offsets [N + 1]), symbols in raster (h, w, c) order; cdf_total <= 32768.
+ *   One thread-block cluster per image walks the latent in raster order: per position the context model over the already
+ *   decoded y_hat, the three entropy-parameter layers, then the 128 symbols of the position from the rANS stream (on the
+ *   device, compressai's bypass escape included), y_hat = symbol + mean.  `status`: the first symbol that could not be
+ *   decoded (truncated or corrupt stream; nothing after it is written).
+ * ar_decode_rows: ROW STREAMS (container version 3), one standard rANS string per latent row (N * H strings, word_offsets
+ *   [N * H + 1]), string n * H + r = row r of image n, its symbols in (w, c) order; cdf_total <= 27392, and every entry but
+ *   a row's last must be below 2^16 and the last one 2^16 (they are held as 16-bit values in every CTA's shared memory;
+ *   other tables give status -2).  The kernel is ar_code's own wavefront loop (same chunks, K splits and summation order)
+ *   with a decoding epilogue: position p of a wavefront chunk is decoded by one warp of the cluster, so the rows of a
+ *   wavefront decode in parallel.  `cluster` is launched as is (no fallback), and a launch that fails returns an error
+ *   naming it.  `status`: the failure with the lowest row h, a truncated or corrupt row or a row whose decoder does not end
+ *   in the state the encoder started from (x = 2^31 with every word consumed).  Rows above a failed row still decode; the
+ *   failed row and those below it stop.  `workspace`: tdvc_ar_decode_rows_workspace_bytes(N, H, c1_pad, c2_pad) bytes. */
 typedef struct TdvcArDecodeParams {
   TdvcArChain chain;
   const uint32_t* words;  const int64_t* word_offsets;
@@ -365,26 +377,6 @@ typedef struct TdvcArDecodeParams {
   int64_t* status;       /* [N] */
   int32_t cluster;
 } TdvcArDecodeParams;
-/* ar_decode_rows: the inverse of ar_code for ROW STREAMS (container version 3): one rANS string per latent row, row r of
- *   image n = words[word_offsets[n * H + r] .. word_offsets[n * H + r + 1]), each a standard string of the row's symbols in
- *   (w, c) order.  The kernel is ar_code's own wavefront loop (same chunks, K splits and summation order) with a decoding
- *   epilogue: position p of a wavefront chunk is decoded by one warp of the cluster, so the rows of a wavefront decode in
- *   parallel.  `cluster` must be the encoder's cluster size (8 or 16): it is launched as is (no fallback), and a launch that
- *   fails returns an error naming it.  Tables as in ar_decode; every entry but a row's last must be below 2^16 and the last
- *   one 2^16 (they are held as 16-bit values in every CTA's shared memory).  `status` [N]: -1 when image n decoded, -2 when
- *   the CDF tables are not valid rows (nothing is decoded), else (h * W + w) * C + c of the failure with the lowest row h: a
- *   truncated or corrupt row, or a row whose decoder does not end in the state the encoder started from (x = 2^31 with every
- *   word consumed).  Rows above a failed row still decode; the failed row and those below it stop.  `workspace`:
- *   tdvc_ar_decode_rows_workspace_bytes(N, H, c1_pad, c2_pad) bytes.                                                     */
-typedef struct TdvcArRowDecodeParams {
-  TdvcArChain chain;
-  const uint32_t* words;  const int64_t* word_offsets;   /* [N * H + 1] */
-  const int32_t* cdfs;   int32_t cdf_stride;
-  const int32_t* cdf_lengths;  const int32_t* cdf_offsets;
-  int32_t n_tables, cdf_total;
-  int64_t* status;       /* [N] */
-  int32_t cluster;
-} TdvcArRowDecodeParams;
 int tdvc_pmf_to_quantized_cdf(const float* pmf, int n, int precision, int32_t* cdf);
 int tdvc_eb_symbols(const float* z, int ld, const float* medians, int N, int HW, int C, int32_t* symbols, int32_t* indexes,
                     void* stream);
@@ -393,7 +385,7 @@ size_t tdvc_ar_code_workspace_bytes(int N, int c1_pad, int c2_pad);
 int tdvc_ar_code(const TdvcArParams* p, void* workspace, size_t workspace_bytes, void* stream);
 int tdvc_ar_decode(const TdvcArDecodeParams* p, void* stream);
 size_t tdvc_ar_decode_rows_workspace_bytes(int N, int H, int c1_pad, int c2_pad);
-int tdvc_ar_decode_rows(const TdvcArRowDecodeParams* p, void* workspace, size_t workspace_bytes, void* stream);
+int tdvc_ar_decode_rows(const TdvcArDecodeParams* p, void* workspace, size_t workspace_bytes, void* stream);
 int64_t tdvc_rans_encode_with_indexes(const int32_t* symbols, const int32_t* indexes, int64_t n, const int32_t* cdfs,
                                       int cdf_stride, const int32_t* cdf_lengths, const int32_t* offsets, int n_tables,
                                       uint8_t* out, int64_t capacity);

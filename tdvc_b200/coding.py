@@ -16,8 +16,9 @@ What runs where:
 * `compress`: z symbols by `tdvc_eb_symbols`; the autoregressive pass over y - compressai's per-position Python loop - by
   the wavefront kernel `tdvc_ar_code` (one launch per coder, csrc/coding.cu) on the y / hyper-decoder buffers the forward
   pass left in the plan; rANS over the symbols on the host (`tdvc_rans_encode_with_indexes`), as in compressai.
-* `decode_latents`: y strings back to symbols and y_hat on the device (`tdvc_ar_decode`, csrc/ar_decode.cu), bit-identical
-  to what `tdvc_ar_code` produced when told the encoder's cluster size.
+* `decode_latents`: y strings back to symbols and y_hat on the device (`tdvc_ar_decode`, csrc/ar_decode.cu; row streams:
+  `tdvc_ar_decode_rows`, csrc/coding.cu), bit-identical to what `tdvc_ar_code` produced when told the encoder's cluster
+  size.
 * `decode_z_symbols` / `dequantize_z`: z strings back to symbols on the host (rANS, as in compressai) and z_hat = symbol +
   median on the device (`tdvc_eb_dequantize`); `VideoCompressor.decompress_latents` runs h_s on it to get the `params`
   decode_latents needs, so that a container alone decodes.
@@ -275,79 +276,47 @@ def code_latents(plan, W, cn, tables, cluster=0, keep=False):
     return finish_coding(launch_coding(plan, W, cn, tables, cluster=cluster), keep=keep)
 
 
+AR_DECODED, AR_BAD_TABLES = -1, -2   # status of an image after the device decoders (csrc/ar_common.cuh)
+# CDF entries the device decoders hold in shared memory (64 Gaussian rows: 27,256): tdvc_ar_decode, tdvc_ar_decode_rows
+CDF_MAX, ROW_CDF_MAX = 32768, 27392
+
+
 def _gc_rows_ok(tables, max_total):
     gl = tables.gc.length
     return not (gl.size > 64 or (gl < 2).any() or (gl > tables.gc.cdf.shape[1]).any() or int(gl.sum()) > max_total)
 
 
-def _check_word_strings(strings, who, what):
+def _check_word_strings(strings, who, name, hy, rows):
+    """Every y string of coder `name` (N strings, or with rows N * hy row strings in (image, row) order) is whole 32-bit
+    words, at least two, as rANS writes them; else RuntimeError naming the coder, the image and the row."""
     for i, s_ in enumerate(strings):
         if len(s_) < 8 or len(s_) % 4:
-            raise RuntimeError(f"{who}: {what(i)} has {len(s_)} bytes (rANS strings are whole 32-bit words, at least two)")
+            what = f"{name} y row {i % hy} of image {i // hy}" if rows else f"{name} y string of image {i}"
+            raise RuntimeError(f"{who}: {what} has {len(s_)} bytes (rANS strings are whole 32-bit words, at least two)")
 
 
-def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None):
+def launch_decoding(W, cn, tables, y_strings, params, cluster, stream=None, rows=False):
     """Device decoding of the y strings of coder `cn` ("mv" | "rs"), the inverse of launch_coding's y half
-    (compressai `_decompress_ar`): `tdvc_ar_decode` runs the context model and the entropy parameters position by position
-    and decodes the rANS stream on the device.  params: the hyper-decoder output of the same images, a channels-last Act
+    (compressai `_decompress_ar`).  params: the hyper-decoder output of the same images, a channels-last Act
     (N, h, w, >= 256 channels).  cluster: the CTAs per image `tdvc_ar_code` coded the strings with (8 or 16); the
-    predictions, and so the decoded symbols, are exact only for that value.  Returns a handle for finish_decoding."""
+    predictions, and so the decoded symbols, are exact only for that value.
+    rows=False: N strings, one per image (containers of version 2).  `tdvc_ar_decode` runs the context model and the
+    entropy parameters position by position and decodes the rANS stream on the device.
+    rows=True: ROW STREAMS (finish_coding(..., rows=True), container version 3), N * h strings, one per latent row in
+    (image, row) order.  `tdvc_ar_decode_rows` is the encoder's own wavefront kernel with a decoding epilogue, so the rows
+    of a wavefront decode in parallel; it launches with the encoder's cluster size and nothing else.
+    Strings that are not whole words, or fewer than two, and a wrong string count raise RuntimeError before any device
+    work.  Returns a handle for finish_decoding."""
     lib = L.load()
     N, hy, wy = params.N, params.H, params.W
     dev = params.t.device
     if cluster not in (8, 16):
         raise RuntimeError(f"decode_latents: encoder cluster size {cluster} (8 or 16)")
-    if len(y_strings) != N:
-        raise RuntimeError(f"decode_latents: {len(y_strings)} {cn} y strings for {N} images")
-    _check_word_strings(y_strings, "decode_latents", lambda i: f"{cn} y string of image {i}")
-    gl = tables.gc.length
-    if not _gc_rows_ok(tables, 32768):
-        raise RuntimeError("decode_latents: the Gaussian CDF tables are not valid rows for the device decoder")
-    stream = stream or torch.cuda.current_stream(dev)
-    words = np.frombuffer(b"".join(bytes(s_) for s_ in y_strings), dtype="<i4")
-    offsets = np.cumsum([0] + [len(s_) // 4 for s_ in y_strings]).astype(np.int64)
-    cdf, length, offset = tables.gc.on(dev)
-    with torch.cuda.stream(stream):
-        words_d = torch.from_numpy(words.copy()).to(dev)
-        offsets_d = torch.from_numpy(offsets).to(dev)
-        y_hat = torch.empty((N, hy, wy, 128), device=dev)
-        y_sym = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
-        y_idx = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
-        status = torch.empty((N,), device=dev, dtype=torch.int64)
-    p = L.ArDecodeParams(chain=_ar_chain(W, cn, tables, params, (y_hat, y_sym, y_idx), "decode_latents"),
-                         words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
-                         cdfs=cdf.data_ptr(), cdf_stride=cdf.shape[1], cdf_lengths=length.data_ptr(),
-                         cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(gl.sum()),
-                         status=status.data_ptr(), cluster=cluster)
-    L.check(lib.tdvc_ar_decode(C.byref(p), stream.cuda_stream), "ar_decode")
-    with torch.cuda.stream(stream):
-        status_h = _pinned_like(status)
-        status_h.copy_(status, non_blocking=True)
-        done = torch.cuda.Event()
-        done.record(stream)
-    # the inputs stay referenced until the decode has run
-    return {"cn": cn, "done": done, "status": status_h, "keep": (words_d, offsets_d), "shape": (hy, wy),
-            "y_hat": y_hat, "y_symbols": y_sym, "y_indexes": y_idx}
-
-
-ROW_CDF_MAX = 27392   # CDF entries tdvc_ar_decode_rows holds in shared memory (64 Gaussian rows: 27,256)
-
-
-def launch_decoding_rows(W, cn, tables, y_strings, params, cluster, stream=None):
-    """Device decoding of ROW STREAMS of coder `cn` (finish_coding(..., rows=True), container version 3): N * h strings, one
-    per latent row in (image, row) order.  `tdvc_ar_decode_rows` is the encoder's own wavefront kernel with a decoding
-    epilogue, so the rows of a wavefront decode in parallel; it launches with the encoder's cluster size (8 or 16) and
-    nothing else.  Strings that are not whole words, or fewer than two, and a wrong string count raise RuntimeError before
-    any device work.  Returns a handle for finish_decoding."""
-    lib = L.load()
-    N, hy, wy = params.N, params.H, params.W
-    dev = params.t.device
-    if cluster not in (8, 16):
-        raise RuntimeError(f"decode_latents: encoder cluster size {cluster} (8 or 16)")
-    if len(y_strings) != N * hy:
-        raise RuntimeError(f"decode_latents: {len(y_strings)} {cn} y row strings for {N} images of {hy} rows")
-    _check_word_strings(y_strings, "decode_latents", lambda i: f"{cn} y row {i % hy} of image {i // hy}")
-    if not _gc_rows_ok(tables, ROW_CDF_MAX):
+    n, what = (N * hy, f"y row strings for {N} images of {hy} rows") if rows else (N, f"y strings for {N} images")
+    if len(y_strings) != n:
+        raise RuntimeError(f"decode_latents: {len(y_strings)} {cn} {what}")
+    _check_word_strings(y_strings, "decode_latents", cn, hy, rows)
+    if not _gc_rows_ok(tables, ROW_CDF_MAX if rows else CDF_MAX):
         raise RuntimeError("decode_latents: the Gaussian CDF tables are not valid rows for the device decoder")
     stream = stream or torch.cuda.current_stream(dev)
     words = np.frombuffer(b"".join(bytes(s_) for s_ in y_strings), dtype="<i4")
@@ -361,20 +330,26 @@ def launch_decoding_rows(W, cn, tables, y_strings, params, cluster, stream=None)
         y_idx = torch.empty((N, hy, wy, 128), device=dev, dtype=torch.int32)
         status = torch.empty((N,), device=dev, dtype=torch.int64)
         chain = _ar_chain(W, cn, tables, params, (y_hat, y_sym, y_idx), "decode_latents")
-        need = lib.tdvc_ar_decode_rows_workspace_bytes(N, hy, chain.c1_pad, chain.c2_pad)
-        ws = torch.empty(((need + 15) // 16 * 4,), device=dev)
-    p = L.ArRowDecodeParams(chain=chain, words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
-                            cdfs=cdf.data_ptr(), cdf_stride=cdf.shape[1], cdf_lengths=length.data_ptr(),
-                            cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(tables.gc.length.sum()),
-                            status=status.data_ptr(), cluster=cluster)
-    L.check(lib.tdvc_ar_decode_rows(C.byref(p), ws.data_ptr(), ws.numel() * 4, stream.cuda_stream), "ar_decode_rows")
+        ws = None
+        if rows:
+            need = lib.tdvc_ar_decode_rows_workspace_bytes(N, hy, chain.c1_pad, chain.c2_pad)
+            ws = torch.empty(((need + 15) // 16 * 4,), device=dev)
+    p = L.ArDecodeParams(chain=chain, words=words_d.data_ptr(), word_offsets=offsets_d.data_ptr(),
+                         cdfs=cdf.data_ptr(), cdf_stride=cdf.shape[1], cdf_lengths=length.data_ptr(),
+                         cdf_offsets=offset.data_ptr(), n_tables=cdf.shape[0], cdf_total=int(tables.gc.length.sum()),
+                         status=status.data_ptr(), cluster=cluster)
+    if rows:
+        L.check(lib.tdvc_ar_decode_rows(C.byref(p), ws.data_ptr(), ws.numel() * 4, stream.cuda_stream), "ar_decode_rows")
+    else:
+        L.check(lib.tdvc_ar_decode(C.byref(p), stream.cuda_stream), "ar_decode")
     with torch.cuda.stream(stream):
         status_h = _pinned_like(status)
         status_h.copy_(status, non_blocking=True)
         done = torch.cuda.Event()
         done.record(stream)
-    return {"cn": cn, "done": done, "status": status_h, "keep": (words_d, offsets_d, ws), "shape": (hy, wy),
-            "rows": True, "y_hat": y_hat, "y_symbols": y_sym, "y_indexes": y_idx}
+    # the inputs stay referenced until the decode has run
+    return {"cn": cn, "done": done, "status": status_h, "keep": (words_d, offsets_d, ws), "shape": (hy, wy), "rows": rows,
+            "y_hat": y_hat, "y_symbols": y_sym, "y_indexes": y_idx}
 
 
 def _pinned_like(t):
@@ -382,16 +357,17 @@ def _pinned_like(t):
 
 
 def finish_decoding(h):
-    """Waits for a launch_decoding or launch_decoding_rows and turns a failed image into RuntimeError (naming the coder, the image and the
-    latent position (h, w, c) where the stream broke).  Returns {"y_hat", "y_symbols", "y_indexes"} (N, h, w, 128)."""
+    """Waits for a launch_decoding and turns a failed image into RuntimeError (naming the coder, the image, with row streams
+    the row, and the latent position (h, w, c) where the stream broke).  Returns {"y_hat", "y_symbols", "y_indexes"}
+    (N, h, w, 128)."""
     h["done"].synchronize()
     wy = h["shape"][1]
     for i, st in enumerate(h["status"].tolist()):
-        if st == -2:
+        if st == AR_BAD_TABLES:
             raise RuntimeError(f"ar_decode: the Gaussian CDF tables of the {h['cn']} coder are not valid rows (image {i})")
-        if st != -1:
+        if st != AR_DECODED:
             pix, c = divmod(int(st), 128)
-            if h.get("rows"):
+            if h["rows"]:
                 raise RuntimeError(f"ar_decode_rows: {h['cn']} y row {pix // wy} of image {i} is truncated or corrupt at "
                                    f"(h={pix // wy}, w={pix % wy}, c={c})")
             raise RuntimeError(f"ar_decode: the {h['cn']} y string of image {i} is truncated or corrupt at latent position "
@@ -400,8 +376,7 @@ def finish_decoding(h):
 
 
 def decode_latents(W, cn, tables, y_strings, params, cluster, stream=None, rows=False):
-    launch = launch_decoding_rows if rows else launch_decoding
-    return finish_decoding(launch(W, cn, tables, y_strings, params, cluster, stream=stream))
+    return finish_decoding(launch_decoding(W, cn, tables, y_strings, params, cluster, stream=stream, rows=rows))
 
 
 def eb_indexes(hz, wz, C=128):
@@ -536,3 +511,32 @@ def unpack_frame(data):
         if data[:4] == _MAGIC_V3:
             frame["y_streams"] = "rows"
     return out
+
+
+def unpack_for_decoding(data, who):
+    """unpack_frame, then the host checks a decoder runs before any device work: version 2 or 3, both coders, a frame size
+    of multiples of 64, hyper-latent shapes that fit it, and two string lists per coder, y and z, of N strings each (y of
+    a version-3 container: N * H / 16 row strings), every y string whole 32-bit words.  who: the caller, named in every
+    RuntimeError.  -> (the unpacked container, rows: True when its y strings are row streams)."""
+    box = unpack_frame(data)
+    frame = box.get("frame")
+    if frame is None:
+        raise RuntimeError(f"{who}: a version-1 container records no cluster sizes, so its y strings cannot "
+                           "be decoded exactly (write version 2: pack_frame(..., frame=...))")
+    (H, Wd), N = frame["size"], frame["N"]
+    if N < 1 or H < 64 or Wd < 64 or H % 64 or Wd % 64:
+        raise RuntimeError(f"{who}: frame {H}x{Wd}, N={N} (H and W multiples of 64, N >= 1)")
+    rows = frame.get("y_streams") == "rows"
+    ny = N * (H // 16) if rows else N
+    for nm in ("mv", "res"):
+        enc = box.get(nm)
+        if enc is None:
+            raise RuntimeError(f"{who}: the container has no {nm} coder")
+        if tuple(enc["shape"]) != (H // 64, Wd // 64):
+            raise RuntimeError(f"{who}: {nm} hyper-latent shape {tuple(enc['shape'])} for a {H}x{Wd} "
+                               f"frame (expected {(H // 64, Wd // 64)})")
+        if len(enc["strings"]) != 2 or [len(lst) for lst in enc["strings"]] != [ny, N]:
+            raise RuntimeError(f"{who}: {nm} has {[len(lst) for lst in enc['strings']]} strings (two "
+                               f"lists, y and z, of {ny} and {N})")
+        _check_word_strings(enc["strings"][0], who, nm, H // 16, rows)
+    return box, rows

@@ -8,7 +8,8 @@
 // coded in and on the width of the column slice of the cluster CTA that owns the output channel (so on the cluster size).
 // Every rule that fixes that order lives here, and both kernels call these helpers.  So do the other things the two sides
 // must agree on: the layers' slicing over the cluster (ar_layer), the rANS stream format and its escape decode
-// (rans_symbol, shared with the host decoder), the host checks of the chain and the cluster launch.
+// (rans_symbol, shared with the host decoder), the decoders' CDF table scan and status values, the host checks of the
+// chain and of the decoders' arguments, and the cluster launch.
 #pragma once
 #include "common.cuh"
 
@@ -170,8 +171,28 @@ __host__ __device__ __forceinline__ bool rans_symbol(int s, int max_value, int32
   return true;
 }
 
-// ---- the device rANS reader of ar_decode_kernel (one string per image) and ar_code_kernel's decode instantiation (one
-// string per latent row)
+// ---- the device decoders of y: ar_decode_kernel (one string per image) and ar_code_kernel's decode instantiation (one
+// string per latent row), both on TdvcArDecodeParams
+
+constexpr int AR_TABLES_MAX = 64;           // CDF rows (64 Gaussian scales)
+constexpr int64_t AR_DECODED = -1;          // status: the image decoded
+constexpr int64_t AR_BAD_TABLES = -2;       // status: the CDF tables are not valid rows (nothing is decoded)
+
+// Run by one thread: starts, lengths and offsets of the n_tables CDF rows, as they lie back to back in shared memory.
+// false: the tables are not valid rows (a length outside [2, cdf_stride], or lengths not summing to cdf_total).
+__device__ __forceinline__ bool ar_cdf_rows(const TdvcArDecodeParams& p, int* row, int* len, int* off) {
+  int total = 0;
+  bool ok = true;
+  for (int t = 0; t < p.n_tables; ++t) {
+    const int l = p.cdf_lengths[t];
+    ok = ok && l >= 2 && l <= p.cdf_stride;
+    row[t] = total;
+    len[t] = l;
+    off[t] = p.cdf_offsets[t];
+    total += ok ? l : 0;
+  }
+  return ok && total == p.cdf_total;
+}
 
 // a rANS decoder state held identically by the 32 lanes of the decoding warp; a window of 32 stream words (lane j holds
 // word win + j) keeps the renormalisation reads off the L2 latency.  win = -64: nothing loaded yet.
@@ -232,9 +253,9 @@ __device__ __forceinline__ bool ard_decode_symbol(ArdRans& r, Cdf cdf, int len, 
   return r.renorm() && rans_symbol(s, len - 2, offset, [&](uint32_t& v) { return r.bits(v); }, sym);
 }
 
-// ---- host side of tdvc_ar_code and tdvc_ar_decode
+// ---- host side of tdvc_ar_code, tdvc_ar_decode and tdvc_ar_decode_rows
 
-// what both entry points require of the chain
+// what every entry point requires of the chain
 static inline int ar_check_chain(const TdvcArChain& a, const char* who) {
   TDVC_REQUIRE(a.params && a.w_ctx && a.b_ctx && a.w1 && a.b1 && a.w2 && a.b2 && a.w3 && a.b3 && a.scale_table && a.y_hat &&
                    a.symbols && a.indexes, "%s: null pointer in the chain", who);
@@ -246,6 +267,18 @@ static inline int ar_check_chain(const TdvcArChain& a, const char* who) {
                    a.c1_pad >= ((a.c1 + 3) & ~3) && a.c2_pad % 4 == 0 && a.c2_pad >= ((a.c2 + 3) & ~3),
                "%s: hidden widths %d, %d (padded %d, %d)", who, a.c1, a.c2, a.c1_pad, a.c2_pad);
   TDVC_REQUIRE(a.n_scales >= 2 && a.n_scales <= 65, "%s: scale table of %d entries", who, a.n_scales);
+  return TDVC_OK;
+}
+
+// what both decoders require of their arguments; cdf_max = the CDF entries the decoder holds in shared memory
+static inline int ar_check_decode(const TdvcArDecodeParams& p, int cdf_max, const char* who) {
+  const int rc = ar_check_chain(p.chain, who);
+  if (rc != TDVC_OK) return rc;
+  TDVC_REQUIRE(p.words && p.word_offsets && p.cdfs && p.cdf_lengths && p.cdf_offsets && p.status, "%s: null pointer", who);
+  TDVC_REQUIRE(p.n_tables >= p.chain.n_scales && p.n_tables <= AR_TABLES_MAX && p.cdf_stride >= 3,
+               "%s: %d tables for %d scales", who, p.n_tables, p.chain.n_scales);
+  TDVC_REQUIRE(p.cdf_total > 0 && p.cdf_total <= cdf_max, "%s: %d CDF entries (at most %d)", who, p.cdf_total, cdf_max);
+  TDVC_REQUIRE(p.cluster == 8 || p.cluster == 16, "%s: encoder cluster size %d (8 or 16)", who, p.cluster);
   return TDVC_OK;
 }
 

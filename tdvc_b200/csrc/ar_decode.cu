@@ -21,14 +21,12 @@ namespace cg = cooperative_groups;
 namespace tdvc {
 
 constexpr int ARD_CDF_MAX = 32768;   // CDF entries held in shared memory (64 Gaussian rows: 27,256)
-constexpr int ARD_TABLES_MAX = 64;
 constexpr int ARD_NO_MAX = 64;       // outputs of one layer per CTA (clusters of >= 8 CTAs, c1 <= 512)
 constexpr int ARD_IN_MAX = 512;      // widest layer input (ep0: params | ctx)
 // Dynamic shared memory holds the CDF rows, which only CTA 0 reads.  A launch has one dynamic size for all its CTAs, and
 // the reservation costs nothing: at 512 threads x 110 registers one CTA fills an SM's register file, and 128 KB + 20 KB
 // of static shared memory fit beside it.
 constexpr size_t ARD_SMEM = (size_t)ARD_CDF_MAX * sizeof(int32_t);
-constexpr int64_t ARD_BAD_TABLES = -2;   // status: the CDF tables are not valid rows
 
 // split partials of this CTA's outputs of layer w for one position: part[ks][nl] = the encoder's fmaf chain of split ks of
 // output nl; in(k) = float4 of the layer input at k .. k + 3 (shared memory)
@@ -96,7 +94,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const TdvcArDe
   __shared__ float s_mean[C];                          // CTA 0: means and table indexes of the position
   __shared__ int s_idx[C];
   __shared__ int s_sym[C];
-  __shared__ int s_row[ARD_TABLES_MAX + 1], s_len[ARD_TABLES_MAX], s_off[ARD_TABLES_MAX];
+  __shared__ int s_row[AR_TABLES_MAX + 1], s_len[AR_TABLES_MAX], s_off[AR_TABLES_MAX];
   __shared__ int s_stop;                               // written by CTA 0 into every CTA: stop decoding this image
 
   const ArW wA = ar_layer(a, AR_CTX, rank, RD), wB = ar_layer(a, AR_EP0, rank, RD), wC = ar_layer(a, AR_EP2, rank, RD),
@@ -125,20 +123,10 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_decode_kernel(const TdvcArDe
   const bool coder = rank == 0 && threadIdx.x < 32;
   if (rank == 0) {
     if (threadIdx.x == 0) {
-      int total = 0;
-      bool ok = true;
-      for (int t = 0; t < p.n_tables; ++t) {
-        const int len = p.cdf_lengths[t];
-        ok = ok && len >= 2 && len <= p.cdf_stride;
-        s_row[t] = total;
-        s_len[t] = len;
-        s_off[t] = p.cdf_offsets[t];
-        total += ok ? len : 0;
-      }
-      ok = ok && total == p.cdf_total;
+      const bool ok = ar_cdf_rows(p, s_row, s_len, s_off);
       const int64_t w0 = p.word_offsets[n], w1 = p.word_offsets[n + 1];
       s_stop = ok && w1 - w0 >= 2 ? 0 : 1;
-      p.status[n] = !ok ? ARD_BAD_TABLES : (s_stop ? 0 : -1);
+      p.status[n] = !ok ? AR_BAD_TABLES : (s_stop ? 0 : AR_DECODED);
     }
     __syncthreads();
     if (!s_stop) {
@@ -237,15 +225,8 @@ using namespace tdvc;
 
 extern "C" int tdvc_ar_decode(const TdvcArDecodeParams* p, void* stream) {
   TDVC_REQUIRE(p != nullptr, "ar_decode: null params");
-  const int rc = ar_check_chain(p->chain, "ar_decode");
+  const int rc = ar_check_decode(*p, ARD_CDF_MAX, "ar_decode");
   if (rc != TDVC_OK) return rc;
-  TDVC_REQUIRE(p->words && p->word_offsets && p->cdfs && p->cdf_lengths && p->cdf_offsets && p->status,
-               "ar_decode: null pointer");
-  TDVC_REQUIRE(p->n_tables >= p->chain.n_scales && p->n_tables <= ARD_TABLES_MAX && p->cdf_stride >= 3,
-               "ar_decode: %d tables for %d scales", p->n_tables, p->chain.n_scales);
-  TDVC_REQUIRE(p->cdf_total > 0 && p->cdf_total <= ARD_CDF_MAX, "ar_decode: %d CDF entries (at most %d)", p->cdf_total,
-               ARD_CDF_MAX);
-  TDVC_REQUIRE(p->cluster == 8 || p->cluster == 16, "ar_decode: encoder cluster size %d (8 or 16)", p->cluster);
   // 16 CTAs per image, 8 where that cannot launch; the result does not depend on it
   int R = 16;
   return ar_launch_clusters<ar_decode_kernel>(*p, p->chain.N, R, true, ARD_SMEM, (cudaStream_t)stream, "ar_decode");

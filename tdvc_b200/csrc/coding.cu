@@ -42,11 +42,10 @@ struct ArDev {
 // 176,128 + 54,784 + 784 bytes, with the 256 static bytes of the scale table within the 232,448 a block may opt in to.  The
 // staging depth stays AR_NBUF = 3.
 constexpr int ARR_CDF_MAX = 27392;   // CDF entries (64 Gaussian rows: 27,256)
-constexpr int ARR_TABLES_MAX = 64;
-constexpr size_t ARR_SMEM = AR_SMEM + (size_t)ARR_CDF_MAX * sizeof(uint16_t) + (3 * ARR_TABLES_MAX + 4) * sizeof(int);
+constexpr size_t ARR_SMEM = AR_SMEM + (size_t)ARR_CDF_MAX * sizeof(uint16_t) + (3 * AR_TABLES_MAX + 4) * sizeof(int);
 constexpr unsigned long long ARR_NO_FAIL = ~0ull;
 struct ArRowDev {
-  TdvcArRowDecodeParams a;
+  TdvcArDecodeParams a;
   float* ctx_s;
   float* h1_s;
   float* h2_s;
@@ -323,26 +322,14 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const Dev d) {
   // decoder: the CDF rows as uint16 after the reduction tile, then their row starts, lengths and offsets
   uint16_t* s_cdf = reinterpret_cast<uint16_t*>(red + AR_WARPS * AR_PT * 32);
   int* s_row = reinterpret_cast<int*>(s_cdf + ARR_CDF_MAX);
-  int* s_len = s_row + ARR_TABLES_MAX;
-  int* s_off = s_len + ARR_TABLES_MAX;
+  int* s_len = s_row + AR_TABLES_MAX;
+  int* s_off = s_len + AR_TABLES_MAX;
   if constexpr (DECODE) {
     // every CTA loads and checks the tables itself, so all of them reach the same verdict without a barrier
-    const TdvcArRowDecodeParams& q = d.a;
-    if (threadIdx.x == 0) {
-      int total = 0;
-      bool ok = true;
-      for (int i = 0; i < q.n_tables; ++i) {
-        const int len = q.cdf_lengths[i];
-        ok = ok && len >= 2 && len <= q.cdf_stride;
-        s_row[i] = total;
-        s_len[i] = len;
-        s_off[i] = q.cdf_offsets[i];
-        total += ok ? len : 0;
-      }
-      s_off[ARR_TABLES_MAX] = ok && total == q.cdf_total;
-    }
+    const TdvcArDecodeParams& q = d.a;
+    if (threadIdx.x == 0) s_off[AR_TABLES_MAX] = ar_cdf_rows(q, s_row, s_len, s_off);
     __syncthreads();
-    bool ok = s_off[ARR_TABLES_MAX] != 0;
+    bool ok = s_off[AR_TABLES_MAX] != 0;
     if (ok) {
       for (int i = 0; i < q.n_tables; ++i) {
         const int len = s_len[i];
@@ -354,7 +341,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const Dev d) {
       }
     }
     if (!__syncthreads_and(ok)) {
-      if (rank == 0 && threadIdx.x == 0) q.status[n] = -2;
+      if (rank == 0 && threadIdx.x == 0) q.status[n] = AR_BAD_TABLES;
       return;
     }
   }
@@ -474,7 +461,7 @@ __global__ void __launch_bounds__(AR_THREADS, 1) ar_code_kernel(const Dev d) {
   if constexpr (DECODE) {
     if (rank == 0 && threadIdx.x == 0) {
       const unsigned long long f = *(volatile const unsigned long long*)(d.fail + n);
-      d.a.status[n] = f == ARR_NO_FAIL ? -1 : (int64_t)f;
+      d.a.status[n] = f == ARR_NO_FAIL ? AR_DECODED : (int64_t)f;
     }
   }
   cp_async_wait<0>();
@@ -550,18 +537,11 @@ extern "C" size_t tdvc_ar_decode_rows_workspace_bytes(int N, int H, int c1_pad, 
   return chain + (size_t)N * AR_PCH * AR_C * (sizeof(float) + sizeof(int32_t)) + (size_t)N * H * 16 + (size_t)N * 8;
 }
 
-extern "C" int tdvc_ar_decode_rows(const TdvcArRowDecodeParams* p, void* workspace, size_t workspace_bytes, void* stream) {
+extern "C" int tdvc_ar_decode_rows(const TdvcArDecodeParams* p, void* workspace, size_t workspace_bytes, void* stream) {
   TDVC_REQUIRE(p != nullptr, "ar_decode_rows: null params");
-  const int rc = ar_check_chain(p->chain, "ar_decode_rows");
+  const int rc = ar_check_decode(*p, ARR_CDF_MAX, "ar_decode_rows");
   if (rc != TDVC_OK) return rc;
   const TdvcArChain& a = p->chain;
-  TDVC_REQUIRE(p->words && p->word_offsets && p->cdfs && p->cdf_lengths && p->cdf_offsets && p->status,
-               "ar_decode_rows: null pointer");
-  TDVC_REQUIRE(p->n_tables >= a.n_scales && p->n_tables <= ARR_TABLES_MAX && p->cdf_stride >= 3,
-               "ar_decode_rows: %d tables for %d scales", p->n_tables, a.n_scales);
-  TDVC_REQUIRE(p->cdf_total > 0 && p->cdf_total <= ARR_CDF_MAX, "ar_decode_rows: %d CDF entries (at most %d)", p->cdf_total,
-               ARR_CDF_MAX);
-  TDVC_REQUIRE(p->cluster == 8 || p->cluster == 16, "ar_decode_rows: encoder cluster size %d (8 or 16)", p->cluster);
   const size_t chain = tdvc_ar_code_workspace_bytes(a.N, a.c1_pad, a.c2_pad);
   const size_t need = tdvc_ar_decode_rows_workspace_bytes(a.N, a.H, a.c1_pad, a.c2_pad);
   TDVC_REQUIRE(workspace != nullptr && workspace_bytes >= need, "ar_decode_rows: workspace of %zu bytes, %zu needed",

@@ -59,10 +59,6 @@ class ArDecodeParams(C.Structure):
                 ("n_tables", C.c_int32), ("cdf_total", C.c_int32), ("status", c_fp), ("cluster", C.c_int32)]
 
 
-class ArRowDecodeParams(C.Structure):
-    _fields_ = ArDecodeParams._fields_
-
-
 i32, i64, f32, vp, sz = C.c_int32, C.c_int64, C.c_float, C.c_void_p, C.c_size_t
 
 # name -> argtypes, in header order (tests check that every symbol declared in include/tdvc_b200.h is here)
@@ -124,7 +120,7 @@ SIGNATURES = {
     "tdvc_ar_code": [C.POINTER(ArParams), vp, sz, vp],
     "tdvc_ar_decode": [C.POINTER(ArDecodeParams), vp],
     "tdvc_ar_decode_rows_workspace_bytes": [i32, i32, i32, i32],
-    "tdvc_ar_decode_rows": [C.POINTER(ArRowDecodeParams), vp, sz, vp],
+    "tdvc_ar_decode_rows": [C.POINTER(ArDecodeParams), vp, sz, vp],
     "tdvc_rans_encode_with_indexes": [vp, vp, i64, vp, i32, vp, vp, i32, vp, i64],
     "tdvc_rans_decode_with_indexes": [vp, i64, vp, i64, vp, i32, vp, vp, i32, vp],
     "tdvc_gc_bits_backward": [vp, vp, vp, i32, vp, vp, vp, i64, i32, vp],

@@ -1704,7 +1704,8 @@ class VideoCompressor(nn.Module):
         A malformed container, or refer_frames that do not match its frame, raise RuntimeError before any device work; a
         broken string raises as in `decompress_latents`.  taps: records "mv.x_hat", "prediction1", "prediction",
         "recon_feat"."""
-        box = self._container(data, "decompress")
+        from tdvc_b200 import coding
+        box, rows = coding.unpack_for_decoding(data, "decompress")
         (H, Wd), N = box["frame"]["size"], box["frame"]["N"]
         if not isinstance(refer_frames, torch.Tensor) or tuple(refer_frames.shape) != (N, 4, 3, H, Wd):
             got = tuple(refer_frames.shape) if isinstance(refer_frames, torch.Tensor) else type(refer_frames).__name__
@@ -1721,7 +1722,7 @@ class VideoCompressor(nn.Module):
             plan = self._plan(N, H, Wd, dev)
             plan.bind(Wt)
             plan.impl, plan.precision = self.conv_impl, box["frame"]["precision"]
-            lat = self._decode_latents(box, plan, Wt, dev)
+            lat = self._decode_latents(box, rows, plan, Wt, dev)
             y_hat = {cn: Act(t, t.data_ptr(), *t.shape, t.shape[3])
                      for cn, t in (("mv", lat["mv"]["y_hat"]), ("rs", lat["res"]["y_hat"]))}
             recon = plan.decompress(Wt, y_hat, refs, cache=self.cache_features, ref_keys=ref_keys, taps=taps)
@@ -1739,7 +1740,8 @@ class VideoCompressor(nn.Module):
         as the encoder ran with: h_s feeds every predicted mean and scale, and the container does not record conv_impl.
         A malformed container raises RuntimeError before any device work; a broken z string raises naming the coder and
         the image, a broken y string naming the latent position."""
-        box = self._container(data, "decompress_latents")
+        from tdvc_b200 import coding
+        box, rows = coding.unpack_for_decoding(data, "decompress_latents")
         (H, Wd), N = box["frame"]["size"], box["frame"]["N"]
         dev = self._decoder_device()
         with torch.cuda.device(dev), torch.no_grad():
@@ -1749,44 +1751,12 @@ class VideoCompressor(nn.Module):
             # h_s is fp32-class in both precision modes (only rs.g_s* and lf.* take one-product weights), so the container's
             # `precision` does not affect the latents and plan.precision is left as the last forward set it
             plan.impl = self.conv_impl
-            lat = self._decode_latents(box, plan, Wt, dev)
+            lat = self._decode_latents(box, rows, plan, Wt, dev)
             out = {"frame": dict(box["frame"])}
             for nm in ("mv", "res"):
                 out[nm] = {k: v.clone() for k, v in lat[nm].items() if k != "z_hat"}
                 out[nm]["z_hat"] = lat[nm]["z_hat"].t.clone()
         return out
-
-    @staticmethod
-    def _container(data, who):
-        """Unpack a container and check, on the host, that it can be decoded: version 2 or 3, both coders, a frame size of
-        multiples of 64, hyper-latent shapes that fit it, two string lists per coder: N y strings (version 3: N * H / 16
-        row strings) and N z strings.  -> the unpacked container."""
-        from tdvc_b200 import coding
-        box = coding.unpack_frame(data)
-        frame = box.get("frame")
-        if frame is None:
-            raise RuntimeError(f"{who}: a version-1 container records no cluster sizes, so its y strings cannot "
-                               "be decoded exactly (write version 2: pack_frame(..., frame=...))")
-        (H, Wd), N = frame["size"], frame["N"]
-        if N < 1 or H < 64 or Wd < 64 or H % 64 or Wd % 64:
-            raise RuntimeError(f"{who}: frame {H}x{Wd}, N={N} (H and W multiples of 64, N >= 1)")
-        for nm in ("mv", "res"):
-            enc = box.get(nm)
-            if enc is None:
-                raise RuntimeError(f"{who}: the container has no {nm} coder")
-            if tuple(enc["shape"]) != (H // 64, Wd // 64):
-                raise RuntimeError(f"{who}: {nm} hyper-latent shape {tuple(enc['shape'])} for a {H}x{Wd} "
-                                   f"frame (expected {(H // 64, Wd // 64)})")
-            ny = N * (H // 16) if frame.get("y_streams") == "rows" else N
-            if len(enc["strings"]) != 2 or [len(lst) for lst in enc["strings"]] != [ny, N]:
-                raise RuntimeError(f"{who}: {nm} has {[len(lst) for lst in enc['strings']]} strings (two "
-                                   f"lists, y and z, of {ny} and {N})")
-            if frame.get("y_streams") == "rows":
-                for i, s_ in enumerate(enc["strings"][0]):
-                    if len(s_) < 8 or len(s_) % 4:
-                        raise RuntimeError(f"{who}: {nm} y row {i % (H // 16)} of image {i // (H // 16)} has {len(s_)} "
-                                           "bytes (rANS strings are whole 32-bit words, at least two)")
-        return box
 
     def _decoder_device(self):
         dev = self.mvCoder.entropy_bottleneck.quantiles.device
@@ -1794,9 +1764,10 @@ class VideoCompressor(nn.Module):
             raise RuntimeError("tdvc_b200.VideoCompressor runs on CUDA (sm_100a) only; there is no CPU fallback")
         return dev
 
-    def _decode_latents(self, box, plan, Wt, dev):
-        """Device half of decompress_latents on a checked container: {"mv" | "res": {"y_hat", "y_symbols", "y_indexes":
-        tensors of their own, "z_hat": the plan's dec.{cn}.z_hat Act}}, both coders finished."""
+    def _decode_latents(self, box, rows, plan, Wt, dev):
+        """Device half of decompress_latents on a checked container (rows: its y strings are row streams): {"mv" | "res":
+        {"y_hat", "y_symbols", "y_indexes": tensors of their own, "z_hat": the plan's dec.{cn}.z_hat Act}}, both coders
+        finished."""
         from tdvc_b200 import coding
         N = box["frame"]["N"]
         hz, wz = box["mv"]["shape"]
@@ -1816,8 +1787,7 @@ class VideoCompressor(nn.Module):
                 coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
                 params = plan.hyper_synthesis(Wt, cn, zh, b)
             # the motion chain is already decoding on the device while the host decodes the residual z strings
-            launch = coding.launch_decoding_rows if box["frame"].get("y_streams") == "rows" else coding.launch_decoding
-            h = launch(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream)
+            h = coding.launch_decoding(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream, rows=rows)
             pending.append((nm, zh, h))
         main.wait_stream(side)
         out = {}

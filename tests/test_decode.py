@@ -22,7 +22,8 @@ def oracle_model(oracle_model):
 # ------------------------------------------------------------------------------------------------------ CPU
 def test_decode_refuses_malformed_strings_on_the_host():
     """Strings that cannot be rANS output (not whole 32-bit words, shorter than the 8-byte final state), a string count that
-    does not match the batch and an unknown encoder cluster size are refused before anything reaches the device."""
+    does not match the batch (N strings, or N * h row strings) and an unknown encoder cluster size are refused before
+    anything reaches the device."""
     from tdvc_b200 import coding
     from tdvc_b200.model import Act
     t = torch.zeros(2, 4, 8, 256)
@@ -32,6 +33,12 @@ def test_decode_refuses_malformed_strings_on_the_host():
                              ([good, good], 4)):
         with pytest.raises(RuntimeError):
             coding.decode_latents({}, "mv", None, strings, params, cluster)
+    # row streams: N * h = 8 strings
+    for strings, cluster, msg in (([good] * 7 + [good[:6]], 16, "mv y row 3 of image 1 has 6 bytes"),
+                                  ([good] * 2, 16, "2 mv y row strings for 2 images of 4 rows"),
+                                  ([good] * 8, 4, "cluster size 4")):
+        with pytest.raises(RuntimeError, match=msg):
+            coding.decode_latents({}, "mv", None, strings, params, cluster, rows=True)
 
 
 def _coded():

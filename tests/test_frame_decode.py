@@ -31,8 +31,8 @@ def _coded(n=2, shape=(1, 2)):
 # ------------------------------------------------------------------------------------------------------ CPU
 def test_malformed_containers_are_refused_before_any_device_work(monkeypatch):
     """A version-1 container (no cluster sizes), a missing coder, a frame size that is not a multiple of 64, a hyper-latent
-    shape that does not fit the frame and string counts that do not match the batch raise RuntimeError before the weights
-    are packed or a string is decoded."""
+    shape that does not fit the frame, string counts that do not match the batch and y strings that are not whole 32-bit
+    words (or shorter than two) raise RuntimeError before the weights are packed or a string is decoded."""
     from tdvc_b200 import coding
     from tdvc_b200.model import VideoCompressor
     net = VideoCompressor().eval()
@@ -50,6 +50,10 @@ def test_malformed_containers_are_refused_before_any_device_work(monkeypatch):
     three_lists["mv"]["strings"].append([b"x", b"y"])
     one_string = _coded()
     one_string["res"]["strings"][1] = one_string["res"]["strings"][1][:1]
+    ragged = _coded()
+    ragged["res"]["strings"][0][1] = b"\0" * 10
+    short = _coded()
+    short["mv"]["strings"][0][0] = b"\0" * 4
     cases = {"version 1": (coding.pack_frame(_coded()), "version-1"),
              "missing coder": (coding.pack_frame(missing, frame=frame), "no res coder"),
              "frame size": (coding.pack_frame(_coded(shape=(1, 1)), frame=dict(frame, size=(64, 96))), "multiples of 64"),
@@ -57,7 +61,9 @@ def test_malformed_containers_are_refused_before_any_device_work(monkeypatch):
              "hyper shape": (coding.pack_frame(_coded(shape=(2, 1)), frame=frame), "hyper-latent shape"),
              "string lists": (coding.pack_frame(three_lists, frame=frame), "strings"),
              "string count": (coding.pack_frame(one_string, frame=frame), "strings"),
-             "batch": (coding.pack_frame(_coded(), frame=dict(frame, N=3)), "strings")}
+             "batch": (coding.pack_frame(_coded(), frame=dict(frame, N=3)), "strings"),
+             "y words": (coding.pack_frame(ragged, frame=frame), "res y string of image 1 has 10 bytes"),
+             "y too short": (coding.pack_frame(short, frame=frame), "mv y string of image 0 has 4 bytes")}
     for what, (blob, msg) in cases.items():
         with pytest.raises(RuntimeError, match=msg):
             net.decompress_latents(blob)

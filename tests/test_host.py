@@ -32,8 +32,9 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_struct_layouts_match_header():
-    """ctypes mirrors of the parameter structs must have the C sizes, and the chain the encoder and the decoder of y share
-    must sit at offset 0 of both (checked against a tiny C program)."""
+    """ctypes mirrors of the parameter structs must have the C sizes, and the chain the encoder and the decoders of y share
+    must sit at offset 0 of TdvcArParams and of TdvcArDecodeParams, which both decoders take (checked against a tiny C
+    program)."""
     import ctypes
     import subprocess
     import tempfile

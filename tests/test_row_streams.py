@@ -191,15 +191,19 @@ def test_row_streams_match_the_oracle_coder_and_end_where_they_started():
     assert digits == 8
 
 
-def test_row_decoder_is_declared_bound_and_compiles_without_spills():
-    """The entry points are in the header and bound in lib.py with a struct that starts with the chain; ptxas -v of the
-    decode instantiation of ar_code_kernel reports its register use."""
+def test_row_decoder_takes_the_decode_params_and_compiles_without_spills():
+    """The entry points are in the header and bound in lib.py; the row decoder takes the raster decoder's struct, which
+    starts with the chain (its layout: tests/test_host.py); ptxas -v of the decode instantiation of ar_code_kernel
+    reports its register use."""
+    import ctypes
     from tdvc_b200 import build
     from tdvc_b200 import lib as L
     hdr = open(os.path.join(build.ROOT, "include", "tdvc_b200.h")).read()
     for name in ("tdvc_ar_decode_rows_workspace_bytes", "tdvc_ar_decode_rows"):
         assert name + "(" in hdr and name in L.SIGNATURES
-    assert L.ArRowDecodeParams._fields_[0] == ("chain", L.ArChain)
+    assert "tdvc_ar_decode_rows(const TdvcArDecodeParams* p," in hdr
+    assert L.SIGNATURES["tdvc_ar_decode_rows"][0] is ctypes.POINTER(L.ArDecodeParams)
+    assert L.ArDecodeParams._fields_[0] == ("chain", L.ArChain)
     r = subprocess.run([build.NVCC] + build.FLAGS + ["-c", os.path.join(build.CSRC, "coding.cu"), "-o", os.devnull],
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
@@ -356,7 +360,7 @@ def test_gop_round_trips_with_row_streams(oracle_model):
 
 
 @pytest.mark.gpu
-def test_damaged_rows(oracle_model):
+def test_damaged_rows_through_the_shared_launcher(oracle_model):
     """A truncated row raises naming coder, image and row; one flipped byte inside row r raises at row r (the end-of-row
     rule); in a batch of 3 the other images decode (status -1); the good container then decodes exactly."""
     from tdvc_b200 import coding
@@ -386,7 +390,8 @@ def test_damaged_rows(oracle_model):
     lat = dec.decompress_latents(data)
     del lat
     params = plan.buf("dec.rs.params", n, hy, hw[1] // 16, 256)
-    h = coding.launch_decoding_rows(W, "rs", W["_tables"]["rs"], box["res"]["strings"][0], params, box["res"]["cluster"])
+    h = coding.launch_decoding(W, "rs", W["_tables"]["rs"], box["res"]["strings"][0], params, box["res"]["cluster"],
+                               rows=True)
     h["done"].synchronize()
     status = h["status"].tolist()
     assert status[0] >= 0 and status[1] == -1 and status[2] == -1, status

@@ -99,7 +99,7 @@ def main():
             assert torch.equal(dec["y_hat"], enc["y_hat"]) and torch.equal(dec["y_symbols"], enc["y_symbols"])
             if args.row_streams:
                 rows = coding.finish_coding(hold, rows=True)["strings"][0]
-                t_row, h = timed(lambda: coding.launch_decoding_rows(W, cn, tabs, rows, params, enc["cluster"]))
+                t_row, h = timed(lambda: coding.launch_decoding(W, cn, tabs, rows, params, enc["cluster"], rows=True))
                 dec = coding.finish_decoding(h)
                 assert torch.equal(dec["y_hat"], enc["y_hat"]) and torch.equal(dec["y_symbols"], enc["y_symbols"])
             if rep:
