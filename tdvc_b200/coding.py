@@ -356,21 +356,27 @@ def _pinned_like(t):
     return torch.empty(t.shape, dtype=t.dtype).pin_memory()
 
 
-def finish_decoding(h):
+def _image_name(images, i):
+    return f"image {i}" if images is None else images[i]
+
+
+def finish_decoding(h, images=None):
     """Waits for a launch_decoding and turns a failed image into RuntimeError (naming the coder, the image, with row streams
-    the row, and the latent position (h, w, c) where the stream broke).  Returns {"y_hat", "y_symbols", "y_indexes"}
-    (N, h, w, 128)."""
+    the row, and the latent position (h, w, c) where the stream broke).  images: what to call each image of the batch in
+    those messages (default "image i"; a batch of several containers names the container too).  Returns {"y_hat",
+    "y_symbols", "y_indexes"} (N, h, w, 128)."""
     h["done"].synchronize()
     wy = h["shape"][1]
     for i, st in enumerate(h["status"].tolist()):
+        img = _image_name(images, i)
         if st == AR_BAD_TABLES:
-            raise RuntimeError(f"ar_decode: the Gaussian CDF tables of the {h['cn']} coder are not valid rows (image {i})")
+            raise RuntimeError(f"ar_decode: the Gaussian CDF tables of the {h['cn']} coder are not valid rows ({img})")
         if st != AR_DECODED:
             pix, c = divmod(int(st), 128)
             if h["rows"]:
-                raise RuntimeError(f"ar_decode_rows: {h['cn']} y row {pix // wy} of image {i} is truncated or corrupt at "
+                raise RuntimeError(f"ar_decode_rows: {h['cn']} y row {pix // wy} of {img} is truncated or corrupt at "
                                    f"(h={pix // wy}, w={pix % wy}, c={c})")
-            raise RuntimeError(f"ar_decode: the {h['cn']} y string of image {i} is truncated or corrupt at latent position "
+            raise RuntimeError(f"ar_decode: the {h['cn']} y string of {img} is truncated or corrupt at latent position "
                                f"(h={pix // wy}, w={pix % wy}, c={c})")
     return {k: h[k] for k in ("y_hat", "y_symbols", "y_indexes")}
 
@@ -385,17 +391,19 @@ def eb_indexes(hz, wz, C=128):
     return np.repeat(np.arange(C, dtype=np.int32), hz * wz)
 
 
-def decode_z_symbols(cn, z_strings, tables, hz, wz, C=128):
+def decode_z_symbols(cn, z_strings, tables, hz, wz, C=128, images=None):
     """Host half of compressai `EntropyBottleneck.decompress` for coder `cn` ("mv" | "rs"): one z string per image ->
     int32 symbols (N, C, hz, wz), the NCHW order they were coded in.  A string that does not decode raises RuntimeError
-    naming the coder and the image (rANS cannot detect every corruption: a garbled string may decode to other symbols)."""
+    naming the coder and the image (rANS cannot detect every corruption: a garbled string may decode to other symbols);
+    images: the names of the images, as in finish_decoding."""
     idx = eb_indexes(hz, wz, C)
     out = np.empty((len(z_strings), C, hz, wz), dtype=np.int32)
     for i, s_ in enumerate(z_strings):
         try:
             out[i] = rans_decode(s_, idx, tables.eb).reshape(C, hz, wz)
         except RuntimeError as e:
-            raise RuntimeError(f"decompress_latents: the {cn} z string of image {i} is truncated or corrupt ({e})") from None
+            raise RuntimeError(f"decompress_latents: the {cn} z string of {_image_name(images, i)} is truncated or "
+                               f"corrupt ({e})") from None
     return out
 
 

@@ -137,12 +137,16 @@ def compress_gop(net, i_frame, p_frames, enable_amp=False, row_streams=False):
 
 def decompress_gop(net, i_frame, containers, size):
     """Decoder of `compress_gop`: the same I-frame (1,3,h,w), the containers in order and the frame size (h, w) ->
-    the cropped reconstructions, bit-identical to the encoder's."""
+    the cropped reconstructions, bit-identical to the encoder's.  The latents of all frames depend on the containers and
+    the weights alone, so they are entropy-decoded first, as one batch (`VideoCompressor.decompress_latents_many`); a
+    broken string raises naming its container before anything is synthesised.  Then each frame's synthesis runs on its
+    reference window, frame by frame (`decompress`'s second half)."""
+    latents = net.decompress_latents_many(containers)
     refs = RefBuffer(pad(i_frame, 64))
     recons = []
-    for data in containers:
+    for lat in latents:
         window, keys = refs.window()
-        recon = net.decompress(data, window, ref_keys=keys)
+        recon = net._synthesise(lat, window, ref_keys=keys, who="decompress_gop")
         refs.push(recon)
         recons.append(crop(recon, size))
     return recons
@@ -168,6 +172,76 @@ def validate(dataset, net, enable_amp=True, device=None, with_msssim=True, gops=
             from tdvc_b200.metrics import ms_ssim
             i_ms += float(ms_ssim(raw[0:1].to(device), i_frame, data_range=1.0))
     return combine_with_iframes(summarise(tot), n_i, i_bpp, i_psnr, i_ms)
+
+
+def coded_rates(data):
+    """Rates of one frame container (version 2 or 3) from its bytes, per padded pixel N * H * W as the reference
+    normalises bpp: (bpp_mv, bpp_res, bpp_container).  bpp_mv / bpp_res: 8 x the bytes of that coder's y and z strings;
+    bpp_container: 8 x every byte of the container, so that the header and the length fields count too."""
+    from tdvc_b200 import coding
+    box = coding.unpack_frame(data)
+    (H, W), N = box["frame"]["size"], box["frame"]["N"]
+    px = N * H * W
+    coder = lambda nm: 8.0 * sum(len(s) for lst in box[nm]["strings"] for s in lst) / px
+    return coder("mv"), coder("res"), 8.0 * len(data) / px
+
+
+def validate_codec(dataset, net, decoder=None, enable_amp=True, row_streams=False, with_msssim=True, gops=None):
+    """`validate` on real bitstreams: every GOP of a `tdvc_b200.data.GopDataset` (same contract and I-frame handling) is
+    coded in closed loop by `compress_gop` (row_streams: version-3 containers), rates are taken from the containers'
+    bytes (`coded_rates`) instead of the likelihoods, and PSNR / MS-SSIM / MSE from the frames a decoder rebuilds.
+    decoder: a second module; each GOP is then also decoded by `decompress_gop` on it, its reconstructions must equal the
+    encoder's (torch.equal, else RuntimeError naming GOP and P-frame) and the metrics are taken on them.  Without one, they
+    are taken on the encoder's closed-loop reconstructions, which a decoder rebuilds bit for bit.
+    Returns `summarise_codec` of the sums plus "stats": the sums themselves, an fp64 tensor of CODEC_STATS entries, so that
+    a rank's shard (`gops=shard_gops(...)`) is combined with `reduce_stats(stats)` and `summarise_codec(stats)`."""
+    from tdvc_b200.metrics import ms_ssim
+    device = next(net.parameters()).device
+    stats = torch.zeros(CODEC_STATS, device=device, dtype=torch.float64)
+    for g in (range(len(dataset)) if gops is None else gops):
+        p_frames, i_frame, bpp_i, psnr_i, _, raw = dataset[g]
+        p_frames, i_frame = p_frames.to(device), i_frame.to(device).unsqueeze(0)
+        T, _, h, w = p_frames.shape
+        containers, recons = compress_gop(net, i_frame, p_frames, enable_amp=enable_amp, row_streams=row_streams)
+        if decoder is not None:
+            got = decompress_gop(decoder, i_frame.to(next(decoder.parameters()).device), containers, (h, w))
+            got = [r.to(device) for r in got]
+            for t, (a, b) in enumerate(zip(got, recons)):
+                if not torch.equal(a, b):
+                    raise RuntimeError(f"validate_codec: GOP {g}, P-frame {t}: the decoder's reconstruction differs from "
+                                       "the encoder's")
+            recons = got
+        rates = torch.tensor([coded_rates(d) for d in containers], device=device, dtype=torch.float64)
+        res = {"bpp_mv": rates[:, 0], "bpp_res": rates[:, 1], "numel": 3 * h * w,
+               "sse": torch.zeros(T, device=device, dtype=torch.float64)}
+        for t in range(T):
+            sq_err_sum(recons[t], p_frames[t:t + 1], res["sse"], t)
+        if with_msssim:
+            res["msssim"] = torch.stack([ms_ssim(recons[t].float(), p_frames[t:t + 1], data_range=1.0) for t in range(T)])
+        i_ms = float(ms_ssim(raw[0:1].to(device), i_frame, data_range=1.0)) if with_msssim else 0.0
+        stats += torch.cat([gop_stats(res), rates[:, 2].sum().view(1),
+                            torch.tensor([1.0, float(bpp_i), float(psnr_i), i_ms], device=device, dtype=torch.float64)])
+    return dict(summarise_codec(stats), stats=stats)
+
+
+# validate_codec's sums: gop_stats' seven [sum bpp, sum bpp_mv, sum bpp_res, sum psnr, sum msssim, sum mse, P-frames],
+# then sum bpp_container, and of the I-frames [count, sum bpp, sum psnr, sum msssim] as their loader reports them
+CODEC_STATS = 12
+
+
+def summarise_codec(stats):
+    """validate_codec's averages from its sums (over GOPs, and over ranks once reduce_stats has added them): "bpp",
+    "bpp_container", "psnr" and "msssim" over the I- and P-frames as `validate` forms them (an I-frame counts with what its
+    loader reports, in bpp_container as in bpp), "bpp_mv", "bpp_res" and "mse" over the P-frames; "frames" (P-frames),
+    "iframes", and "p": the averages of the P-frames alone (`summarise` + "bpp_container")."""
+    s = [float(v) for v in stats.tolist()]
+    p = summarise(stats[:7])
+    p["bpp_container"] = s[7] / max(s[6], 1.0)
+    n_i = int(s[8])
+    bpp, _, _, psnr, msssim, _ = combine_with_iframes(p, n_i, s[9], s[10], s[11])
+    bpp_container = combine_with_iframes(dict(p, bpp=p["bpp_container"]), n_i, s[9], s[10], s[11])[0]
+    return {"bpp": bpp, "bpp_mv": p["bpp_mv"], "bpp_res": p["bpp_res"], "bpp_container": bpp_container, "psnr": psnr,
+            "msssim": msssim, "mse": p["mse"], "frames": p["frames"], "iframes": n_i, "p": p}
 
 
 def combine_with_iframes(p_summary, n_i, sum_i_bpp, sum_i_psnr, sum_i_msssim):

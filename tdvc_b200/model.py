@@ -1696,33 +1696,47 @@ class VideoCompressor(nn.Module):
 
     def decompress(self, data, refer_frames, ref_keys=None, taps=None):
         """Decoder of one P-frame: a version-2 container (`compress`) and the same refer_frames (N,4,3,H,W) the encoder
-        used -> recon (N,3,H,W) fp32, bit-identical to `compress`'s recon.  Both coders' y_hat come from the path of
-        `decompress_latents`; then extra_fea of refer_frames[:, -1], motion g_s, the prediction, residual g_s + prediction
-        and the in-loop filter run on the encoder's launches.  The precision mode is the container's; the per-GOP feature
-        caches serve as in `forward` (ref_keys likewise).  Exactness needs the encoder's kernels on sm_100a and its
-        `conv_impl`, which the container does not record: this module's own is used.
+        used -> recon (N,3,H,W) fp32, bit-identical to `compress`'s recon.  Two steps: both coders' latents as
+        `decompress_latents` decodes them (`_decode_latents`), then the synthesis (`_synthesise`): extra_fea of
+        refer_frames[:, -1], motion g_s, the prediction, residual g_s + prediction and the in-loop filter on the encoder's
+        launches.  The precision mode is the container's; the per-GOP feature caches serve as in `forward` (ref_keys
+        likewise).  Exactness needs the encoder's kernels on sm_100a and its `conv_impl`, which the container does not
+        record: this module's own is used.
         A malformed container, or refer_frames that do not match its frame, raise RuntimeError before any device work; a
         broken string raises as in `decompress_latents`.  taps: records "mv.x_hat", "prediction1", "prediction",
         "recon_feat"."""
         from tdvc_b200 import coding
         box, rows = coding.unpack_for_decoding(data, "decompress")
-        (H, Wd), N = box["frame"]["size"], box["frame"]["N"]
+        dev = self._check_refs(box["frame"], refer_frames, ref_keys, "decompress")
+        return self._synthesise(self._decode_latents([(box, rows)], dev)[0], refer_frames, ref_keys, taps)
+
+    def _check_refs(self, frame, refer_frames, ref_keys, who):
+        """refer_frames must be (N,4,3,H,W) of the container's frame on this module's CUDA device, ref_keys None or four
+        identities; else RuntimeError naming `who`.  -> the device."""
+        (H, Wd), N = frame["size"], frame["N"]
         if not isinstance(refer_frames, torch.Tensor) or tuple(refer_frames.shape) != (N, 4, 3, H, Wd):
             got = tuple(refer_frames.shape) if isinstance(refer_frames, torch.Tensor) else type(refer_frames).__name__
-            raise RuntimeError(f"decompress: refer_frames {got} do not match the container's frame (expected "
+            raise RuntimeError(f"{who}: refer_frames {got} do not match the container's frame (expected "
                                f"{(N, 4, 3, H, Wd)})")
         if ref_keys is not None and len(ref_keys) != 4:
             raise RuntimeError("ref_keys: expected four identities, one per reference slice")
         dev = self._decoder_device()
         if refer_frames.device != dev:
-            raise RuntimeError(f"decompress: refer_frames are on {refer_frames.device}, the module on {dev}")
+            raise RuntimeError(f"{who}: refer_frames are on {refer_frames.device}, the module on {dev}")
+        return dev
+
+    def _synthesise(self, lat, refer_frames, ref_keys=None, taps=None, who="decompress"):
+        """Synthesis half of `decompress`: one container's latents (an element of `decompress_latents_many`, whose y_hat
+        are wrapped as Acts, no copy) and its refer_frames -> recon (N,3,H,W), in the container's precision mode.
+        refer_frames are checked here too: the launches read them through raw pointers."""
+        dev = self._check_refs(lat["frame"], refer_frames, ref_keys, who)
+        (H, Wd), N = lat["frame"]["size"], lat["frame"]["N"]
         with torch.cuda.device(dev), torch.no_grad():
             refs = refer_frames.detach().float().contiguous()
             Wt = self._weights(dev)
             plan = self._plan(N, H, Wd, dev)
             plan.bind(Wt)
-            plan.impl, plan.precision = self.conv_impl, box["frame"]["precision"]
-            lat = self._decode_latents(box, rows, plan, Wt, dev)
+            plan.impl, plan.precision = self.conv_impl, lat["frame"]["precision"]
             y_hat = {cn: Act(t, t.data_ptr(), *t.shape, t.shape[3])
                      for cn, t in (("mv", lat["mv"]["y_hat"]), ("rs", lat["res"]["y_hat"]))}
             recon = plan.decompress(Wt, y_hat, refs, cache=self.cache_features, ref_keys=ref_keys, taps=taps)
@@ -1739,24 +1753,37 @@ class VideoCompressor(nn.Module):
         The result is bit-identical to the encoder's latents only with the same kernels on sm_100a and the same `conv_impl`
         as the encoder ran with: h_s feeds every predicted mean and scale, and the container does not record conv_impl.
         A malformed container raises RuntimeError before any device work; a broken z string raises naming the coder and
-        the image, a broken y string naming the latent position."""
+        the image, a broken y string naming the latent position.  `decompress_latents_many` decodes several at once."""
         from tdvc_b200 import coding
-        box, rows = coding.unpack_for_decoding(data, "decompress_latents")
-        (H, Wd), N = box["frame"]["size"], box["frame"]["N"]
-        dev = self._decoder_device()
-        with torch.cuda.device(dev), torch.no_grad():
-            Wt = self._weights(dev)
-            plan = self._plan(N, H, Wd, dev)
-            plan.bind(Wt)
-            # h_s is fp32-class in both precision modes (only rs.g_s* and lf.* take one-product weights), so the container's
-            # `precision` does not affect the latents and plan.precision is left as the last forward set it
-            plan.impl = self.conv_impl
-            lat = self._decode_latents(box, rows, plan, Wt, dev)
-            out = {"frame": dict(box["frame"])}
-            for nm in ("mv", "res"):
-                out[nm] = {k: v.clone() for k, v in lat[nm].items() if k != "z_hat"}
-                out[nm]["z_hat"] = lat[nm]["z_hat"].t.clone()
-        return out
+        return self._decode_latents([coding.unpack_for_decoding(data, "decompress_latents")], self._decoder_device())[0]
+
+    def decompress_latents_many(self, containers):
+        """`decompress_latents` of T containers (version 2 or 3, in any mix) of one frame size and batch N, entropy-decoded
+        as ONE batch of T * N images: their latents depend on the bytes and the weights alone, not on each other, so the z
+        steps and h_s run once per coder and y one launch per coder and per (encoder cluster, y layout) group, and the
+        decoder's clusters of all frames run side by side instead of one frame's 16 or 32 SMs at a time.  Returns one dict
+        per container, bit-identical to `decompress_latents` of that container (h_s gives each image the bits it gives it
+        alone: every convolution works on tiles of one image and picks its configuration from the layer's shape).
+        Every container is checked before any device work, and all must hold the (H, W, N) of the first; a RuntimeError
+        names the container index.  A broken z or y string raises naming the container, the coder and the image (for y
+        the position or row) after every launch has finished; nothing of the batch is returned then.  The y tensors of a
+        container are slices of its group's own tensors (no plan buffer), its z_hat a copy."""
+        from tdvc_b200 import coding
+        boxes = []
+        for k, data in enumerate(containers):
+            try:
+                boxes.append(coding.unpack_for_decoding(data, "decompress_latents_many"))
+            except RuntimeError as e:
+                raise RuntimeError(f"container {k}: {e}") from None
+        if not boxes:
+            return []
+        (H, Wd), N = boxes[0][0]["frame"]["size"], boxes[0][0]["frame"]["N"]
+        for k, (box, _) in enumerate(boxes):
+            (h, w), n = box["frame"]["size"], box["frame"]["N"]
+            if (h, w, n) != (H, Wd, N):
+                raise RuntimeError(f"decompress_latents_many: container {k} holds a {h}x{w} frame of N={n}, container 0 a "
+                                   f"{H}x{Wd} frame of N={N} (one batch needs one frame size and batch)")
+        return self._decode_latents(boxes, self._decoder_device(), named=True)
 
     def _decoder_device(self):
         dev = self.mvCoder.entropy_bottleneck.quantiles.device
@@ -1764,35 +1791,67 @@ class VideoCompressor(nn.Module):
             raise RuntimeError("tdvc_b200.VideoCompressor runs on CUDA (sm_100a) only; there is no CPU fallback")
         return dev
 
-    def _decode_latents(self, box, rows, plan, Wt, dev):
-        """Device half of decompress_latents on a checked container (rows: its y strings are row streams): {"mv" | "res":
-        {"y_hat", "y_symbols", "y_indexes": tensors of their own, "z_hat": the plan's dec.{cn}.z_hat Act}}, both coders
-        finished."""
+    def _decode_latents(self, boxes, dev, named=False):
+        """Device half of decompress_latents(_many) on checked containers [(box, rows: its y strings are row streams)] of
+        one (H, W, N), decoded as one batch of T * N images on the plan of that batch (only its dec.* buffers).  Per coder,
+        the batch holds the containers sorted by their (encoder cluster, y layout) group, in order inside a group, so
+        that a group's params are one slice of h_s's output: the z strings of all images on the host, z_hat and h_s once,
+        then one launch_decoding per group over its containers' strings.  The motion coder runs on the current stream, the
+        residual coder on the side stream.  named: error messages call an image "image j of container k".
+        -> per container {"frame", "mv" | "res": {"y_hat", "y_symbols", "y_indexes": slices of tensors of their own,
+        "z_hat": a copy}}, both coders finished."""
         from tdvc_b200 import coding
-        N = box["frame"]["N"]
-        hz, wz = box["mv"]["shape"]
-        main = torch.cuda.current_stream(dev)
-        side = plan._side_stream()
-        side.wait_stream(main)
-        pending = []
-        for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
-            tabs = self._coder_tables(Wt, cn, dev)
-            enc = box[nm]
-            z_sym = coding.decode_z_symbols(cn, enc["strings"][1], tabs, hz, wz)
-            # every buffer under dec.{cn}.*: the forward pass and launch_coding never read what the decoder writes
-            b = lambda nme, h, w, c=128, cn=cn, **kw: plan.buf(f"dec.{cn}.{nme}", N, h, w, c, **kw)
-            with torch.cuda.stream(stream):
-                sym_d = torch.from_numpy(z_sym).to(dev)
-                zh = b("z_hat", hz, wz)
-                coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
-                params = plan.hyper_synthesis(Wt, cn, zh, b)
-            # the motion chain is already decoding on the device while the host decodes the residual z strings
-            h = coding.launch_decoding(Wt, cn, tabs, enc["strings"][0], params, enc["cluster"], stream=stream, rows=rows)
-            pending.append((nm, zh, h))
-        main.wait_stream(side)
-        out = {}
-        for nm, zh, h in pending:
-            out[nm] = dict(coding.finish_decoding(h), z_hat=zh)
+        T = len(boxes)
+        (H, Wd), N = boxes[0][0]["frame"]["size"], boxes[0][0]["frame"]["N"]
+        hz, wz = H // 64, Wd // 64
+        out = [{"frame": dict(box["frame"])} for box, _ in boxes]
+        with torch.cuda.device(dev), torch.no_grad():
+            Wt = self._weights(dev)
+            plan = self._plan(T * N, H, Wd, dev)
+            plan.bind(Wt)
+            # h_s is fp32-class in both precision modes (only rs.g_s* and lf.* take one-product weights), so the container's
+            # `precision` does not affect the latents and plan.precision is left as the last forward set it
+            plan.impl = self.conv_impl
+            main = torch.cuda.current_stream(dev)
+            side = plan._side_stream()
+            side.wait_stream(main)
+            pending, z_hats = [], []
+            for cn, nm, stream in (("mv", "mv", main), ("rs", "res", side)):
+                tabs = self._coder_tables(Wt, cn, dev)
+                group = lambda k, nm=nm: (boxes[k][0][nm]["cluster"], boxes[k][1])
+                order = sorted(range(T), key=group)
+                names = [f"image {j} of container {k}" if named else f"image {j}" for k in order for j in range(N)]
+                z_sym = coding.decode_z_symbols(cn, [s_ for k in order for s_ in boxes[k][0][nm]["strings"][1]], tabs,
+                                                hz, wz, images=names)
+                # every buffer under dec.{cn}.*: the forward pass and launch_coding never read what the decoder writes
+                b = lambda nme, h, w, c=128, cn=cn, **kw: plan.buf(f"dec.{cn}.{nme}", T * N, h, w, c, **kw)
+                with torch.cuda.stream(stream):
+                    sym_d = torch.from_numpy(z_sym).to(dev)
+                    zh = b("z_hat", hz, wz)
+                    coding.dequantize_z(sym_d, Wt[f"{cn}.eb"][3], zh, stream)
+                    params = plan.hyper_synthesis(Wt, cn, zh, b)
+                z_hats.append((nm, zh, order))
+                # the motion chains are already decoding on the device while the host decodes the residual z strings
+                i0 = 0
+                for (cluster, rows), ks in itertools.groupby(order, key=group):
+                    ks = list(ks)
+                    n = len(ks) * N
+                    y_strings = [s_ for k in ks for s_ in boxes[k][0][nm]["strings"][0]]
+                    h = coding.launch_decoding(Wt, cn, tabs, y_strings, params.batch(i0, n), cluster, stream=stream,
+                                               rows=rows)
+                    if stream is not main:   # its outputs are handed to the caller's stream
+                        for k_ in ("y_hat", "y_symbols", "y_indexes"):
+                            h[k_].record_stream(main)
+                    pending.append((nm, ks, names[i0:i0 + n], h))
+                    i0 += n
+            main.wait_stream(side)
+            for nm, ks, images, h in pending:
+                got = coding.finish_decoding(h, images=images)
+                for i, k in enumerate(ks):
+                    out[k][nm] = {key: v[i * N:(i + 1) * N] for key, v in got.items()}
+            for nm, zh, order in z_hats:
+                for i, k in enumerate(order):
+                    out[k][nm]["z_hat"] = zh.t[i * N:(i + 1) * N].clone()
         return out
 
     def _forward_training(self, input_image, refer_frames, taps=None, noise=None):
